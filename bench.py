@@ -26,6 +26,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True     # a benchmark run leaves the source tree as it found it (no __pycache__ for tools/)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 
@@ -139,6 +140,19 @@ def cpu_reference_run(n_streams, steps, warmup, threads, make_frames):
     return n_streams * steps / timed, timed, n_streams * steps
 
 
+def dump_outputs(out_dir, prefix, poses, summaries, n_levels):
+    """Writes the tracker's results of one step as float64 .npy files: poses [S,7] (qw qx qy qz tx ty tz) and every field
+    of the per-stream, per-level solve summaries as summary_<field> [S, n_levels].  That is 272 bytes per stream at 3 levels."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"poses": np.asarray(poses, np.float64)}
+    rec = np.ctypeslib.as_array(summaries)
+    for f in rec.dtype.names:
+        if f != "reserved":
+            arrays["summary_" + f] = rec[f].astype(np.float64).reshape(len(poses), n_levels)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+
 def bind_to_gpu_numa_node(local_rank):
     """Run this rank (and allocate its pinned host buffers) on the NUMA node its GPU hangs off: with 8 ranks pushing
     ~55 GB/s each, uploads that cross the socket interconnect are the first thing to saturate.  Best effort."""
@@ -179,7 +193,14 @@ def main():
     ap.add_argument("--pairs", type=int, default=0, help="config3: total pairs (default 4096)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the tracker returned for the last "
+                    "one (poses and per-level summaries, float64) as DIR/<name>.npy; with more than one rank every name is "
+                    "prefixed rank<r>_. Inputs depend on the arguments only, so runs of two builds can be compared file by file")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "config2"):
+        ap.error("--dump-outputs is implemented for the default workload (--impl ours --workload config2) only")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 0)
 
     rank = int(os.environ.get("RANK", "0")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -288,6 +309,8 @@ def main():
     clocks = sampler.stop()
     ms = sharding.reduce_max(ms, dist, dev)                 # slowest rank defines the step
     value = world * S * K / (ms * 1e-3)
+    if args.dump_outputs:                                   # before the passes below reset the tracker
+        dump_outputs(args.dump_outputs, "rank%d_" % rank if world > 1 else "", *tracker.poses(), N_LEVELS)
 
     # ---- accounting pass (untimed): point-evaluations per solve launch from the per-step summaries ------------
     tracker.reset()

@@ -1,10 +1,10 @@
 #!/usr/bin/env python
-"""Generate the committed golden fixtures.  Run ONCE in the build container:
+"""Generate the committed golden fixtures.  Run once, given a checkout of the reference project:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
-Needs /root/reference (the bundled TUM frames, standalone/rgb-d) and cv2 (genuine
-OpenCV 4.13).  Nothing here runs on the GPU box; only its outputs travel:
+Needs the reference's bundled TUM frames (<reference checkout>/standalone/rgb-d) and cv2 (genuine
+OpenCV 4.13).  Nothing here runs on the GPU; only its outputs are committed:
 
   frames.npz        the reference's five bundled 640x480 RGB-D frames (data, re-encoded)
   cv2_stages.json   sha256 of every genuine-OpenCV preprocessing stage output per frame
@@ -30,7 +30,6 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 from oracle import oracle as O  # noqa: E402
 
-REF = "/root/reference/standalone/rgb-d/"
 K = (525.0, 525.0, 319.5, 239.5)  # standalone_edge_align.cpp:152
 ZSCALE = 5000.0                   # standalone_edge_align.cpp:160
 
@@ -127,12 +126,13 @@ def rotvec_pose(x6):
     return np.concatenate([q, x6[3:]])
 
 
-def main():
+def main(reference):
+    frames_dir = os.path.join(reference, "standalone", "rgb-d")
     cv2.ipp.setUseIPP(False)
     frames_bgr, frames_depth = [], []
     for i in range(1, 6):
-        frames_bgr.append(cv2.imread(REF + "rgb/%d.png" % i))
-        frames_depth.append(cv2.imread(REF + "depth/%d.png" % i, cv2.IMREAD_ANYDEPTH))
+        frames_bgr.append(cv2.imread(os.path.join(frames_dir, "rgb", "%d.png" % i)))
+        frames_depth.append(cv2.imread(os.path.join(frames_dir, "depth", "%d.png" % i), cv2.IMREAD_ANYDEPTH))
     bgr = np.stack(frames_bgr); depth = np.stack(frames_depth)
     np.savez_compressed(os.path.join(HERE, "frames.npz"), bgr=bgr, depth=depth, K=np.array(K), zscale=ZSCALE)
 
@@ -198,4 +198,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit("usage: make_golden.py <reference checkout>")
+    main(sys.argv[1])
