@@ -138,12 +138,11 @@ __global__ void __launch_bounds__(32) k_shard_lm(ShardState* st, const double* s
   local[lane] = lane < EA_SUMS ? sums[lane] : 0.0;
   for (int i = lane; i < int(sizeof(EaLmState) / 8); i += 32) reinterpret_cast<unsigned long long*>(&lm)[i] = reinterpret_cast<const unsigned long long*>(&st->lm)[i];
   __syncwarp();
-  double cand[7];
-  const int cmd = ea_lm_advance_warp(lm, local, sp, lane, cand);
+  const int cmd = ea_lm_advance_warp(lm, local, sp, lane);
   __syncwarp();
   for (int i = lane; i < int(sizeof(EaLmState) / 8); i += 32) reinterpret_cast<unsigned long long*>(&st->lm)[i] = reinterpret_cast<const unsigned long long*>(&lm)[i];
   if (lane == 0) {
-    if (cmd == EA_CMD_EVAL) { for (int i = 0; i < 7; ++i) st->cand[i] = cand[i]; }
+    if (cmd == EA_CMD_EVAL) { for (int i = 0; i < 7; ++i) st->cand[i] = lm.cand[i]; }
     else st->done = 1;
   }
 }
@@ -321,11 +320,10 @@ __global__ void __launch_bounds__(THREADS, 1) k_shard_solve(EaLevelDesc rd, EaLe
       if (s_late) err = 1;            // a CTA of this grid never delivered
       if (err) { if (lane == 0) { s_lm.term = EA_TERM_FAILURE_PEER; ctl->error = 1; } done = 1; }
       else {
-        double cand[7];
-        const int cmd = ea_lm_advance_warp(s_lm, wsum[0], sp, lane, cand);      // all 32 lanes: warp-cooperative LM step
+        const int cmd = ea_lm_advance_warp(s_lm, wsum[0], sp, lane);            // all 32 lanes: warp-cooperative LM step
         if (cmd == EA_CMD_EVAL) {
           EaPose Pn;
-          if (xyz) ea_pose_setup<true>(cand, rg, ng, Pn); else ea_pose_setup<false>(cand, rg, ng, Pn);
+          if (xyz) ea_pose_setup<true>(s_lm.cand, rg, ng, Pn); else ea_pose_setup<false>(s_lm.cand, rg, ng, Pn);
           if (lane == 0) ctl->P = Pn;
         } else done = 1;
       }
@@ -450,8 +448,7 @@ __global__ void __launch_bounds__(GV_THREADS, 1) k_views_solve(const ViewDev* __
         for (int i = lane; i < int(sizeof(EaLmState) / 8); i += 32) dst[i] = __ldcg(src + i);
       }
       __syncwarp();
-      double next[7];
-      const int cmd = ea_lm_advance_warp(s_lm, wsum[0], sp, lane, next);      // (the next candidate is also left in s_lm.cand)
+      const int cmd = ea_lm_advance_warp(s_lm, wsum[0], sp, lane);            // (the next candidate is left in s_lm.cand)
       __syncwarp();
       {
         const unsigned long long* src = reinterpret_cast<const unsigned long long*>(&s_lm);

@@ -126,14 +126,14 @@ __device__ __forceinline__ void ea_boss_next_impl(const EaSolveArgs& A, EaSolveS
 __device__ __noinline__ void ea_boss_next(const EaSolveArgs& A, EaSolveSmem& S, EaMsg& out, bool new_pair_needed) { ea_boss_next_impl<false>(A, S, out, new_pair_needed); }
 
 // Boss warp (all 32 lanes): consume the sums of one evaluation (S.sums) and write the next message into `out` (shared
-// memory).  The LM step itself is warp-cooperative (ea_lm_advance_warp); level / pair changes stay on lane 0.
-__device__ __noinline__ void ea_boss_step_warp(const EaSolveArgs& A, EaSolveSmem& S, const EaMsg& cur, EaMsg& out, const int lane) {
+// memory).  The LM step itself is warp-cooperative (ea_lm_advance_warp); level / pair changes stay on lane 0.  Inlined into
+// warp 0's branch of the kernel: as a call it received its arguments and the kernel's live values through the stack frame.
+__device__ __forceinline__ void ea_boss_step_warp(const EaSolveArgs& A, EaSolveSmem& S, const EaMsg& cur, EaMsg& out, const int lane) {
   const int acc0 = S.lm.accepted, rej0 = S.lm.rejected;
-  double cand[7];
 #ifdef EA_LM_PROFILE
   const long long t_in = clock64();
 #endif
-  const int cmd = ea_lm_advance_warp(S.lm, S.sums, A.sp, lane, cand);
+  const int cmd = ea_lm_advance_warp(S.lm, S.sums, A.sp, lane);
 #ifdef EA_LM_PROFILE
   __syncwarp();
   if (lane == 0) { S.lm.prof[6] += clock64() - t_in; S.lm.prof[7] += 1; }
@@ -151,8 +151,8 @@ __device__ __noinline__ void ea_boss_step_warp(const EaSolveArgs& A, EaSolveSmem
     // the same (pair, level) again at the new candidate: the fixed words are copied by lanes 0..4, every lane folds the pose
     // (no divergence), lane 0 stores it
     EaPose P;
-    if (cur.pts_mode == EA_POINTS_XYZ) ea_pose_setup<true>(cand, A.ref_geom[cur.level], A.now_geom[cur.level], P);
-    else ea_pose_setup<false>(cand, A.ref_geom[cur.level], A.now_geom[cur.level], P);
+    if (cur.pts_mode == EA_POINTS_XYZ) ea_pose_setup<true>(S.lm.cand, A.ref_geom[cur.level], A.now_geom[cur.level], P);
+    else ea_pose_setup<false>(S.lm.cand, A.ref_geom[cur.level], A.now_geom[cur.level], P);
     if (lane < EA_MSG_FIXED_WORDS) reinterpret_cast<unsigned long long*>(&out)[lane] = reinterpret_cast<const unsigned long long*>(&cur)[lane];
     if (lane == 5) { out.rev = S.lm.evals & 1; out.same = 1; out.nh = 0; out.pad = 0; }
     if (lane == 0) out.P = P;

@@ -307,9 +307,10 @@ static __device__ __forceinline__ int ea_lm_advance_impl(EaLmState& S, const dou
   return ea_lm_propose(S, sp);
 }
 
-// Out of line for the kernels whose hot loop needs the registers; inlined where calls are not possible (a kernel that uses
-// setmaxnreg cannot contain calls: ptxas C7600).
+// The serial state machine out of line: the slow paths of ea_lm_advance_warp call these, so that their register demand does not
+// apply to its fast track.
 static __device__ __noinline__ int ea_lm_advance(EaLmState& S, const double* sums, const ea_solve_params& sp) { return ea_lm_advance_impl(S, sums, sp); }
+static __device__ __noinline__ int ea_lm_propose_slow(EaLmState& S, const ea_solve_params& sp) { return ea_lm_propose(S, sp); }
 
 // ---- warp-cooperative advance: the common case on a fast track ------------------------------------------------------------
 // Between two evaluations of a pair nothing else runs on its CTA, so the latency of this step is dead time (the serial version
@@ -319,7 +320,7 @@ static __device__ __noinline__ int ea_lm_advance(EaLmState& S, const double* sum
 // the lanes, and the heavy pieces are arranged for instruction-level parallelism (in-place 6x6 LDL^T on the 21 unique entries,
 // six independent row chains for the model cost, series Plus).  Everything else (first evaluation of a level, rejected or
 // invalid steps, any termination, the dogleg strategy) takes the serial state machine on lane 0, whose arithmetic for the
-// shared parts is identical operation for operation.  out_cand: the next candidate in registers (all lanes) on EA_CMD_EVAL.
+// shared parts is identical operation for operation.  On EA_CMD_EVAL the next candidate is in S.cand.
 __device__ __forceinline__ bool ea_ldlt_solve6_packed(double (&U)[21], const double (&bs)[6], double (&y)[6]) {
   // U: upper triangle, row-major (ea_tri), damping already on the diagonal.  In place: U[tri(j,j)] <- d_j, U[tri(j,i)] <- L[i][j].
   double dinv[6];
@@ -341,7 +342,7 @@ __device__ __forceinline__ bool ea_ldlt_solve6_packed(double (&U)[21], const dou
       U[ea_tri(j, i)] = t * dinv[j];
     }
   }
-  if (!ok) return false;
+  // (no early exit on a failed pivot: y is then meaningless but unused, and a branch here made ptxas spill y at the merge)
 #pragma unroll
   for (int i = 0; i < 6; ++i) {
     double t = bs[i];
@@ -363,7 +364,7 @@ __device__ __forceinline__ bool ea_ldlt_solve6_packed(double (&U)[21], const dou
 }
 
 static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S, const double* __restrict__ sums, const ea_solve_params& __restrict__ sp,
-                                                      const int lane, double (&out_cand)[7]) {
+                                                      const int lane) {
   // (S, sums and the parameters never alias: without the qualifiers every store into S -- and there is one per state field --
   // orders the loads behind it, which serialises six clamp chains and most of the section boundaries)
   const unsigned full = 0xffffffffu;
@@ -373,13 +374,13 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
   // the serial state machine serves: the dogleg strategy, failed evaluations, rejected steps, near-tolerance decisions
   bool fast = (sp.trust_region_strategy == 0) && !(sums[27] > 0.0);
   const int phase = S.phase;
-  double xc[7], rel = 0.0, radius = 0.0;
+  double rel = 0.0, radius = 0.0;
   const double cand_cost = sums[28];
   int iter = 0;
   if (fast && phase == 1) {
     double sn = 0.0, xn = 0.0;
 #pragma unroll
-    for (int i = 0; i < 7; ++i) { const double xo = S.x[i]; xc[i] = S.cand[i]; const double d = xo - xc[i]; sn += d * d; xn += xo * xo; }
+    for (int i = 0; i < 7; ++i) { const double xo = S.x[i]; const double d = xo - S.cand[i]; sn += d * d; xn += xo * xo; }
     const double pt2 = sp.parameter_tolerance * sp.parameter_tolerance;
     if (sn <= 2.0 * pt2 * (xn + pt2)) fast = false;                    // near the parameter tolerance: the exact test decides
     const double cost_change = S.cost - cand_cost;
@@ -395,25 +396,16 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
   }
   if (!fast) {
     int cmd = 0;
-    if (lane == 0) cmd = ea_lm_advance_impl(S, sums, sp);
+    if (lane == 0) cmd = ea_lm_advance(S, sums, sp);
     cmd = __shfl_sync(full, cmd, 0);
     __syncwarp();
-    if (cmd == EA_CMD_EVAL) {
-#pragma unroll
-      for (int i = 0; i < 7; ++i) out_cand[i] = S.cand[i];
-    }
     return cmd;
   }
   EA_LM_LAP(0);
-  double sc[6];
   if (phase == 0) {
     // ---- IterationZero: the state at x0, Jacobi scaling from the first Jacobian (one sqrt + one division per lane) ----
-#pragma unroll
-    for (int i = 0; i < 7; ++i) xc[i] = S.x[i];
     double mine = 1.0;
     if (lane < 6 && sp.jacobi_scaling) mine = 1.0 / (1.0 + sqrt(sums[ea_tri(lane, lane)]));
-#pragma unroll
-    for (int j = 0; j < 6; ++j) sc[j] = __shfl_sync(full, mine, j);
     radius = sp.initial_trust_region_radius;
     iter = 0;
     __syncwarp();
@@ -428,19 +420,19 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
     const double t = 2.0 * rel - 1.0;
     radius = fmin(sp.max_trust_region_radius, S.radius / fmax(1.0 / 3.0, 1.0 - t * t * t));
     iter = S.iter;
-#pragma unroll
-    for (int j = 0; j < 6; ++j) sc[j] = S.scale[j];
     __syncwarp();                                  // every lane has read the old state
     if (lane < 7) S.x[lane] = S.cand[lane];
     if (lane < 21) S.H[lane] = sums[lane]; else if (lane < 27) S.b[lane - 21] = sums[lane];
     if (lane == 27) { S.cost = cand_cost; S.radius = radius; S.decrease_factor = 2.0; S.accepted++; S.evals++; S.invalid_run = 0; }
   }
+  // From here on the iterate and the scaling are read from the state where they are used (S.x, S.scale): held in registers
+  // across the factorisation they pushed the fast track past the register budget of the solve kernels and into local memory.
+  __syncwarp();
   // gradient tolerance (same shortcut as ea_gradient_converged: the translation block of Plus is a plain addition)
   {
     const double gt = fmax(fabs(sums[24]), fmax(fabs(sums[25]), fabs(sums[26])));
-    const double xt = fmax(fabs(xc[4]), fmax(fabs(xc[5]), fabs(xc[6])));
+    const double xt = fmax(fabs(S.x[4]), fmax(fabs(S.x[5]), fabs(S.x[6])));
     if (!(gt > 2.0 * sp.gradient_tolerance + 4.5e-16 * xt)) {
-      __syncwarp();
       int conv = 0;
       if (lane == 0) { conv = ea_gradient_converged(S, sp.gradient_tolerance) ? 1 : 0; if (conv) S.term = EA_TERM_CONVERGENCE_GRADIENT; }
       if (__shfl_sync(full, conv, 0)) { if (lane == 0) { S.iter = iter; S.reuse_diag = 0; } __syncwarp(); return EA_CMD_DONE; }
@@ -455,32 +447,31 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
   const double inv_radius = 1.0 / radius;
 #pragma unroll
   for (int a = 0; a < 6; ++a) {
-    bs[a] = sc[a] * sums[21 + a];
+    bs[a] = S.scale[a] * sums[21 + a];
 #pragma unroll
-    for (int c = a; c < 6; ++c) U[ea_tri(a, c)] = sc[a] * sums[ea_tri(a, c)] * sc[c];
+    for (int c = a; c < 6; ++c) U[ea_tri(a, c)] = S.scale[a] * sums[ea_tri(a, c)] * S.scale[c];
   }
   const double dg_lo = sp.min_lm_diagonal, dg_hi = sp.max_lm_diagonal;
-  double dgv[6];
 #pragma unroll
-  for (int j = 0; j < 6; ++j) {
-    dgv[j] = fmin(fmax(U[ea_tri(j, j)], dg_lo), dg_hi);
-    U[ea_tri(j, j)] += dgv[j] * inv_radius;
-  }
-#pragma unroll
-  for (int j = 0; j < 6; ++j) if (lane == j) S.diag[j] = dgv[j];
+  for (int j = 0; j < 6; ++j) U[ea_tri(j, j)] += fmin(fmax(U[ea_tri(j, j)], dg_lo), dg_hi) * inv_radius;
+  // lane j stores diag[j], recomputed from shared memory with the same operations (picking element `lane` of a register
+  // array would put the array in local memory)
+  if (lane < 6) S.diag[lane] = fmin(fmax(S.scale[lane] * sums[ea_tri(lane, lane)] * S.scale[lane], dg_lo), dg_hi);
   EA_LM_LAP(2);
   bool ok = ea_ldlt_solve6_packed(U, bs, y);
 #pragma unroll
-  for (int a = 0; a < 6; ++a) delta[a] = -y[a] * sc[a];
+  for (int a = 0; a < 6; ++a) delta[a] = -y[a] * S.scale[a];
   EA_LM_LAP(3);
-  // model_cost_change = -(delta^T b + 1/2 delta^T H delta): the serial code's order, as six independent row chains
+  // model_cost_change = -(delta^T b + 1/2 delta^T H delta): the serial code's order, as six independent row chains.  The sums
+  // are read from their copies in the state (S.H, S.b, as the serial code does): reading `sums` again let the compiler keep
+  // the 27 values loaded for U in registers across the factorisation.
   double lin = 0.0, quad = 0.0;
 #pragma unroll
   for (int a = 0; a < 6; ++a) {
-    lin = fma(delta[a], sums[21 + a], lin);
+    lin = fma(delta[a], S.b[a], lin);
     double row = 0.0;
 #pragma unroll
-    for (int c = 0; c < 6; ++c) row = fma(sums[a <= c ? ea_tri(a, c) : ea_tri(c, a)], delta[c], row);
+    for (int c = 0; c < 6; ++c) row = fma(S.H[a <= c ? ea_tri(a, c) : ea_tri(c, a)], delta[c], row);
     quad = fma(delta[a], row, quad);
   }
   const double model = -(lin + 0.5 * quad);
@@ -489,21 +480,18 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
   if (!ok) {     // HandleInvalidStep: rare; the serial loop recomputes this step, finds it invalid and carries on from there
     __syncwarp();
     int cmd = 0;
-    if (lane == 0) { S.iter = iter; S.reuse_diag = 0; cmd = ea_lm_propose(S, sp); }
+    if (lane == 0) { S.iter = iter; S.reuse_diag = 0; cmd = ea_lm_propose_slow(S, sp); }
     cmd = __shfl_sync(full, cmd, 0);
     __syncwarp();
-    if (cmd == EA_CMD_EVAL) {
-#pragma unroll
-      for (int i = 0; i < 7; ++i) out_cand[i] = S.cand[i];
-    }
     return cmd;
   }
-  ea_pose_plus(xc, delta, out_cand);
+  double cand[7];
+  ea_pose_plus(S.x, delta, cand);
   __syncwarp();
   if (lane == 28) { S.model_cost_change = model; S.iter = iter + 1; S.reuse_diag = 1; }
   if (lane == 29) {
 #pragma unroll
-    for (int i = 0; i < 7; ++i) S.cand[i] = out_cand[i];
+    for (int i = 0; i < 7; ++i) S.cand[i] = cand[i];
   }
   __syncwarp();
   EA_LM_LAP(5);
