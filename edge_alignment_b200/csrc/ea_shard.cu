@@ -702,6 +702,11 @@ int ea_shard_solve(ea_shard* s, ea_frameset* ref, int ref_slot, ea_frameset* now
   rc = ea_frameset_get_num_points(ref, ref_slot, level, &n_pts);
   if (rc) return rc;
   const int n_res = (n_pts + sp->point_stride - 1) / sp->point_stride;
+  if (n_res == 0) {   // as ea_solve_batch: nothing to align, pose untouched, no launch (every rank sees the same count)
+    for (int i = 0; i < 8; ++i) s->prof[i] = 0.0;
+    if (summary) { *summary = ea_summary{}; summary->termination = EA_TERM_SKIPPED_NO_POINTS; }
+    return EA_OK;
+  }
   // this rank's contiguous slice of the ordered residual list
   const int j0 = int((long long)n_res * s->rank / s->world), j1 = int((long long)n_res * (s->rank + 1) / s->world);
   if (s->in_kernel) return shard_solve_persistent(s, ref, ref_slot, now, now_slot, level, pose7, sp, summary, n_res, j0, j1);
@@ -855,6 +860,10 @@ int ea_solve_views(ea_context* c, int n_views, const ea_view* views, int level, 
     nb[i] = nres[i] > 0 ? std::max(1, std::min(c->sm_count, (nres[i] + 2047) / 2048)) : 0;
     total += nres[i]; nb_total += nb[i];
   }
+  if (total == 0) {   // as ea_solve_batch: nothing to align, pose untouched, no launch
+    if (summary) { *summary = ea_summary{}; summary->termination = EA_TERM_SKIPPED_NO_POINTS; }
+    return EA_OK;
+  }
   // One persistent cooperative kernel for the whole solve (k_views_solve).  View descriptors, control block and CTA totals live
   // in the context's scratch (allocated on first use, grown on demand): no allocation on the path of a solve.
   const int grid = std::max(1, std::min(c->sm_count, (total + 1023) / 1024));
@@ -901,7 +910,7 @@ int ea_solve_views(ea_context* c, int n_views, const ea_view* views, int level, 
     summary->termination = h.done ? h.lm.term : EA_TERM_NO_CONVERGENCE;
     summary->iterations = h.lm.iter; summary->accepted = h.lm.accepted; summary->rejected = h.lm.rejected;
     summary->n_residuals = total; summary->evaluations = h.lm.evals;
-    summary->initial_cost = h.lm.initial_cost; summary->final_cost = h.lm.cost;
+    summary->initial_cost = h.lm.initial_cost; summary->final_cost = h.lm.cost; summary->truncated = 0; summary->reserved = 0;
   }
   return EA_OK;
 }
