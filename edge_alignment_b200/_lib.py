@@ -11,6 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 SO_PATH = os.path.join(HERE, "libea_b200.so")
 
 EA_MAX_LEVELS = 4
+EA_MAX_VIEWS_PER_PROBLEM = 16
 EA_OK = 0
 LOSS_TRIVIAL, LOSS_CAUCHY, LOSS_HUBER = 0, 1, 2
 STRATEGY_LM, STRATEGY_DOGLEG = 0, 1
@@ -99,6 +100,7 @@ PROTOTYPES = {
     "ea_solve_batch_device": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(SolveParams), _vp]),
     "ea_eval_views": (_i, [_vp, _i, C.POINTER(View), _i, _f64p, C.POINTER(SolveParams), _pi, _f64p, _f64p, _f64p, _f64p, _pi]),
     "ea_solve_views": (_i, [_vp, _i, C.POINTER(View), _i, _f64p, C.POINTER(SolveParams), C.POINTER(Summary)]),
+    "ea_solve_views_batch": (_i, [_vp, _i, _i32p, C.POINTER(View), _f64p, C.POINTER(SolveParams), C.POINTER(Summary)]),
     "ea_tracker_create": (_i, [_vp, C.POINTER(FrameParams), C.POINTER(SolveParams), _i, _i, C.POINTER(_vp)]),
     "ea_tracker_destroy": (_i, [_vp]),
     "ea_tracker_reset": (_i, [_vp]),

@@ -165,6 +165,22 @@ class Context:
         _check(L.lib().ea_solve_views(self._h, len(views), arr, level, _ptr(pose, C.c_double), C.byref(sp), C.byref(s)))
         return pose, s.asdict()
 
+    def solve_views_batch(self, problems, poses7=None, sp=None):
+        """Many multi-camera problems, each solved coarse to fine in one persistent launch (ea_solve_views_batch).
+        problems: list of lists of the view dicts eval_views / solve_views take.  Returns (poses [n, 7], [[summary per level]
+        per problem])."""
+        sp = sp or solve_params()
+        n = len(problems)
+        flat = [v for pr in problems for v in pr]
+        offsets = np.zeros(n + 1, np.int32)
+        offsets[1:] = np.cumsum([len(pr) for pr in problems])
+        arr = self._views(flat) if flat else (L.View * 1)()
+        poses = np.tile(IDENTITY, (n, 1)) if poses7 is None else np.array(poses7, np.float64).reshape(n, 7).copy()
+        nl = flat[0]["ref"].params.n_levels if flat else 1
+        S = (L.Summary * max(n * nl, 1))()
+        _check(L.lib().ea_solve_views_batch(self._h, n, _ptr(offsets, C.c_int32), arr, _ptr(poses, C.c_double), C.byref(sp), S))
+        return poses, [[S[i * nl + l].asdict() for l in range(nl)] for i in range(n)]
+
     def solve_batch_device(self, n, ref, d_ref_slots, now, d_now_slots, d_poses, sp, d_pose_index=0, d_summaries=0):
         """All pointer arguments are raw device addresses (ints); asynchronous on the context stream."""
         _check(L.lib().ea_solve_batch_device(self._h, n, ref._h, d_ref_slots, now._h, d_now_slots, d_poses,

@@ -191,6 +191,14 @@ struct EaEventPair {
   EaEventPair() = default; EaEventPair(const EaEventPair&) = delete; EaEventPair& operator=(const EaEventPair&) = delete;
 };
 int ea_ensure_tmp(ea_context* c, size_t bytes);
+// A view's rig transform and distortion in the form the general per-point evaluation takes (identity / zero when unused).
+inline void ea_view_xf(const ea_view& v, EaViewXf& X) {
+  memset(&X, 0, sizeof X);
+  X.use_rig = v.use_rig != 0; X.use_dist = v.use_distortion != 0;
+  for (int i = 0; i < 12; ++i) { X.T21[i] = v.cam_T_first[i]; X.T12[i] = v.first_T_cam[i]; }
+  if (!X.use_rig) { for (int i = 0; i < 12; ++i) X.T21[i] = X.T12[i] = (i % 5 == 0) ? 1.0 : 0.0; }
+  for (int i = 0; i < 5; ++i) X.dist[i] = X.use_dist ? v.dist[i] : 0.0;
+}
 extern "C" int ea_check_solve_params(const ea_solve_params* sp);   // shared argument validation of every solve entry point
 int ea_solve_batch_device_ordered(ea_context* c, int n, ea_frameset* ref, const int32_t* d_ref_slots, ea_frameset* now,
                                    const int32_t* d_now_slots, double* d_poses7, const int32_t* d_pose_index,

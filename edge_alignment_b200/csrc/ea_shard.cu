@@ -762,14 +762,6 @@ int ea_shard_solve(ea_shard* s, ea_frameset* ref, int ref_slot, ea_frameset* now
 // ---- multi-camera problems: every view adds its residual blocks to the same 6-DoF problem ----------------------------
 // (standalone_edge_align.cpp:791-803 / 3204-3219: one AddResidualBlock loop per camera with EAResidue /
 //  EAResidueSecondCam / EAResidueEx / EAResidueSecondCamEx, all on the same b_quat_a, b_t_a)
-static int view_xf(const ea_view& v, EaViewXf& X) {
-  std::memset(&X, 0, sizeof X);
-  X.use_rig = v.use_rig != 0; X.use_dist = v.use_distortion != 0;
-  for (int i = 0; i < 12; ++i) { X.T21[i] = v.cam_T_first[i]; X.T12[i] = v.first_T_cam[i]; }
-  if (!X.use_rig) { for (int i = 0; i < 12; ++i) X.T21[i] = X.T12[i] = (i % 5 == 0) ? 1.0 : 0.0; }
-  for (int i = 0; i < 5; ++i) X.dist[i] = X.use_dist ? v.dist[i] : 0.0;
-  return EA_OK;
-}
 static int check_view(const ea_view& v, int level) {
   if (!v.ref || !v.now) return ea_fail(EA_ERR_INVALID_ARG, "view with a null frameset");
   if (v.ref->ctx->device != v.now->ctx->device) return ea_fail(EA_ERR_INVALID_ARG, "view framesets on different devices");
@@ -806,7 +798,7 @@ int ea_eval_views(ea_context* c, int n_views, const ea_view* views, int level, c
     const ea_view& v = views[i];
     const EaLevelDesc& rd = v.ref->h_desc[size_t(v.ref_slot) * EA_MAX_LEVELS + level];
     const EaLevelDesc& nd = v.now->h_desc[size_t(v.now_slot) * EA_MAX_LEVELS + level];
-    EaViewXf X; view_xf(v, X);
+    EaViewXf X; ea_view_xf(v, X);
     const double ids = v.ref->inv_depth_unit;
     if (nres[i] > 0) {
       const int blocks = (nres[i] + 255) / 256;
@@ -887,7 +879,7 @@ int ea_solve_views(ea_context* c, int n_views, const ea_view* views, int level, 
     D.rd = v.ref->h_desc[size_t(v.ref_slot) * EA_MAX_LEVELS + level];
     D.nd = v.now->h_desc[size_t(v.now_slot) * EA_MAX_LEVELS + level];
     D.rg = v.ref->geom[level]; D.ng = v.now->geom[level];
-    view_xf(v, D.X);
+    ea_view_xf(v, D.X);
     D.inv_depth_scale = v.ref->inv_depth_unit;
     D.n_res = nres[i]; D.xyz = D.rd.pts_mode == EA_POINTS_XYZ ? 1 : 0;
   }

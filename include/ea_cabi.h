@@ -255,6 +255,16 @@ int ea_eval_views(ea_context* ctx, int n_views, const ea_view* views, int level,
                   double* sums28, int* failed);
 int ea_solve_views(ea_context* ctx, int n_views, const ea_view* views, int level, double* pose7,
                    const ea_solve_params* sp, ea_summary* summary);
+/* n independent multi-camera problems, each solved coarse-to-fine (sp->coarsest_level .. sp->finest_level, as
+ * ea_solve_batch).  Problem i is views[view_offsets[i] .. view_offsets[i+1]) (1..EA_MAX_VIEWS_PER_PROBLEM views); at level l its
+ * residual blocks are exactly those ea_solve_views(..., level = l) would use.  The pose found at level l starts level l-1.
+ * poses7 [n][7] in/out (HOST); summaries [n][L] (HOST, may be NULL), L = n_levels shared by every frameset of the call.
+ * One persistent launch: one CTA per problem, largest problem first; cluster_size is ignored.  Point counts are read on the
+ * device.  A truncated reference list is solved with the cut list: results are written, then EA_ERR_CAPACITY names the first
+ * (problem, view, level).  Synchronous. */
+#define EA_MAX_VIEWS_PER_PROBLEM 16
+int ea_solve_views_batch(ea_context* ctx, int n_problems, const int32_t* view_offsets /*[n+1]*/, const ea_view* views,
+                         double* poses7, const ea_solve_params* sp, ea_summary* summaries);
 
 /* ---- tracker: the caller of the path (src/ea.cpp:87-131 consumer loop, re-stated) ------ */
 /* n_streams independent cameras; every step each stream gets one new frame which is aligned

@@ -128,3 +128,18 @@ def make_sequences(n_streams, n_frames, seed=0, width=640, height=480, K=TUM_K, 
         bgr[:, s] = b; depth[:, s] = d
         traj.append((Rw, tw))
     return bgr, depth, traj
+
+
+def stereo_rig(Rw, tw, baseline=0.12, yaw_deg=2.0):
+    """A second camera rigidly mounted beside the one that follows (Rw, tw): `baseline` metres along its x axis, turned by
+    `yaw_deg` about its y axis.  Returns the second camera's camera-to-world poses (R [n,3,3], t [n,3]) and T21, the 4x4
+    transform from first-camera to second-camera coordinates (ea_view.cam_T_first; X_2 = R21 X_1 + t21)."""
+    a = np.radians(yaw_deg)
+    R12 = np.array([[np.cos(a), 0, np.sin(a)], [0, 1, 0], [-np.sin(a), 0, np.cos(a)]])   # second camera's axes in the first's
+    t12 = np.array([baseline, 0.0, 0.0])
+    Rw2 = np.einsum("nij,jk->nik", np.asarray(Rw), R12)
+    tw2 = np.asarray(tw) + np.einsum("nij,j->ni", np.asarray(Rw), t12)
+    T21 = np.eye(4)
+    T21[:3, :3] = R12.T
+    T21[:3, 3] = -R12.T @ t12
+    return Rw2, tw2, T21
