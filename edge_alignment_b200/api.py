@@ -231,6 +231,26 @@ class FrameSet:
         slots = np.ascontiguousarray(slots, np.int32)
         _check(L.lib().ea_frameset_preprocess_device(self._h, len(slots), _ptr(slots, C.c_int32), d_bgr, d_depth or None, roles))
 
+    def preprocess_gray_host(self, slots, gray, depth=None, roles=L.ROLE_BOTH, ref_mask=None, now_mask=None):
+        """8-bit gray frames [n][h][w]: the same results as preprocess_host on (g, g, g), from a third of the bytes.
+        ref_mask: reference points only where > 0 (get_aX_mask); now_mask: now-frame edges only where > 1."""
+        slots = np.ascontiguousarray(slots, np.int32)
+        gray = np.ascontiguousarray(gray, np.uint8)
+        depth = None if depth is None else np.ascontiguousarray(depth, np.float32 if self.params.depth_type == L.DEPTH_F32 else np.uint16)
+        ref_mask = None if ref_mask is None else np.ascontiguousarray(ref_mask, np.uint8)
+        now_mask = None if now_mask is None else np.ascontiguousarray(now_mask, np.uint8)
+        assert gray.size == len(slots) * self.params.width * self.params.height
+        _check(L.lib().ea_frameset_preprocess_gray_host(self._h, len(slots), _ptr(slots, C.c_int32), gray.ctypes.data,
+                                                        None if depth is None else depth.ctypes.data,
+                                                        None if ref_mask is None else ref_mask.ctypes.data,
+                                                        None if now_mask is None else now_mask.ctypes.data, roles))
+        self.ctx.sync()   # numpy buffers may be pageable and short-lived
+
+    def preprocess_gray_device(self, slots, d_gray, d_depth=0, roles=L.ROLE_BOTH):
+        """d_gray / d_depth: device addresses (ints) of [n][h][w] u8 gray frames and their depth."""
+        slots = np.ascontiguousarray(slots, np.int32)
+        _check(L.lib().ea_frameset_preprocess_gray_device(self._h, len(slots), _ptr(slots, C.c_int32), d_gray, d_depth or None, roles))
+
     def set_points(self, slot, pts4, level=0, mode=L.POINTS_PIXEL):
         pts4 = np.ascontiguousarray(pts4, np.float32).reshape(-1, 4)
         _check(L.lib().ea_frameset_set_points(self._h, slot, level, _ptr(pts4, C.c_float), len(pts4), mode))
@@ -273,10 +293,17 @@ class FrameSet:
 class Tracker:
     """n_streams frame-to-keyframe trackers stepped in lock-step (the caller of the path, src/ea.cpp:87-131)."""
 
-    def __init__(self, ctx, fparams, sparams, n_streams, keyframe_interval=10):
+    def __init__(self, ctx, fparams, sparams, n_streams, keyframe_interval=10, image_format=L.IMAGE_BGR8):
         self.ctx = ctx; self.n_streams = n_streams; self.n_levels = fparams.n_levels
         self._h = C.c_void_p()
         _check(L.lib().ea_tracker_create(ctx._h, C.byref(fparams), C.byref(sparams), n_streams, keyframe_interval, C.byref(self._h)))
+        if image_format != L.IMAGE_BGR8:
+            self.set_image_format(image_format)
+
+    def set_image_format(self, image_format):
+        """IMAGE_BGR8 ([n_streams][h][w][3]) or IMAGE_GRAY8 ([n_streams][h][w]) for step_host / step_device; only before the
+        first step (after creation or reset)."""
+        _check(L.lib().ea_tracker_set_image_format(self._h, image_format))
 
     def close(self):
         if self._h:
@@ -287,7 +314,8 @@ class Tracker:
         _check(L.lib().ea_tracker_reset(self._h))
 
     def step_host(self, bgr_ptr, depth_ptr, fetch=True):
-        """bgr_ptr/depth_ptr: host addresses (ints) of [n_streams][h][w][3] u8 / [n_streams][h][w] u16."""
+        """bgr_ptr/depth_ptr: host addresses (ints) of [n_streams][h][w][3] u8 (IMAGE_BGR8) or [n_streams][h][w] u8
+        (IMAGE_GRAY8) / [n_streams][h][w] u16."""
         if fetch:
             poses = np.empty((self.n_streams, 7)); S = (L.Summary * (self.n_streams * self.n_levels))()
             _check(L.lib().ea_tracker_step_host(self._h, bgr_ptr, depth_ptr or None, _ptr(poses, C.c_double), S))
@@ -317,6 +345,7 @@ class Tracker:
         return n.value / (ms.value * 1e-3), ms.value, n.value
 
     def step_device(self, d_bgr, d_depth=0):
+        """Device addresses of the frames, laid out as for step_host."""
         _check(L.lib().ea_tracker_step_device(self._h, d_bgr, d_depth or None))
 
     def poses(self, want_summaries=True):

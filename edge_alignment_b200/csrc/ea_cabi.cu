@@ -280,13 +280,13 @@ static int check_slots(ea_frameset* fs, int n, const int32_t* slots) {
 
 }  // extern "C"
 int ea_preprocess_impl(ea_frameset* fs, int n, const int32_t* d_slots, const uint8_t* d_bgr, const void* d_depth, int roles,
-                       const uint8_t* d_mask, const uint8_t* d_now_mask, cudaStream_t stream) {
+                       const uint8_t* d_mask, const uint8_t* d_now_mask, cudaStream_t stream, int in_channels) {
   ea_context* c = fs->ctx;
   if (!stream) stream = c->stream;
   EaPrepArgs A;
   std::memset(&A, 0, sizeof A);
   for (int l = 0; l < fs->p.n_levels; ++l) A.lv[l] = fs->lv[l];
-  A.n_levels = fs->p.n_levels; A.slots = d_slots; A.in_bgr = d_bgr; A.in_depth = d_depth; A.in_mask = d_mask; A.in_now_mask = d_now_mask;
+  A.n_levels = fs->p.n_levels; A.slots = d_slots; A.in_bgr = d_bgr; A.in_channels = in_channels; A.in_depth = d_depth; A.in_mask = d_mask; A.in_now_mask = d_now_mask;
   A.n_pts = fs->d_npts; A.dt_minmax = fs->d_minmax; A.dt_affine = fs->d_affine; A.overflow = fs->d_overflow;
   A.n = n; A.roles = roles; A.grad_threshold = fs->p.grad_threshold; A.use_median = fs->p.use_median;
   A.dt_normalize = fs->p.dt_normalize;
@@ -405,6 +405,60 @@ int ea_frameset_preprocess_host(ea_frameset* fs, int n, const int32_t* slots, co
   CU(cudaMemcpyAsync(fs->stage_bgr, bgr, px * 3 * n, cudaMemcpyHostToDevice, c->stream));
   if (depth) CU(cudaMemcpyAsync(fs->stage_depth, depth, px * fs->depth_elem * n, cudaMemcpyHostToDevice, c->stream));
   return ea_frameset_preprocess_device(fs, n, slots, fs->stage_bgr, depth ? fs->stage_depth : nullptr, roles);
+}
+
+// ---- 8-bit gray input: the same pipeline as on BGR (g, g, g), from a third of the bytes -----------------------------------
+static int check_gray_args(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* gray, const void* depth,
+                           const uint8_t* ref_mask, const uint8_t* now_mask, int roles) {
+  int rc = check_slots(fs, n, slots);
+  if (rc) return rc;
+  if (!gray) return ea_fail(EA_ERR_INVALID_ARG, "gray is null");
+  if (roles < EA_ROLE_REF || roles > EA_ROLE_BOTH) return ea_fail(EA_ERR_INVALID_ARG, "roles must be EA_ROLE_REF, EA_ROLE_NOW or EA_ROLE_BOTH");
+  if ((roles & EA_ROLE_REF) && !depth) return ea_fail(EA_ERR_INVALID_ARG, "EA_ROLE_REF needs depth");
+  if (ref_mask && !(roles & EA_ROLE_REF)) return ea_fail(EA_ERR_INVALID_ARG, "ref_mask only applies to the reference role");
+  if (now_mask && !(roles & EA_ROLE_NOW)) return ea_fail(EA_ERR_INVALID_ARG, "now_mask only applies to the now role");
+  return EA_OK;
+}
+
+int ea_frameset_preprocess_gray_device(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* d_gray, const void* d_depth, int roles) {
+  int rc = check_gray_args(fs, n, slots, d_gray, d_depth, nullptr, nullptr, roles);
+  if (rc) return rc;
+  ea_context* c = fs->ctx;
+  CU(cudaSetDevice(c->device));
+  EaAsyncBuf d_slots(c->stream);
+  CU(d_slots.alloc(size_t(n) * sizeof(int32_t)));
+  CU(cudaMemcpyAsync(d_slots.p, slots, size_t(n) * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+  rc = ea_preprocess_impl(fs, n, d_slots.as<int32_t>(), d_gray, d_depth, roles, nullptr, nullptr, nullptr, 1);
+  if (rc == EA_OK && (roles & EA_ROLE_REF)) rc = reset_points_mode(fs, n, slots);
+  return rc;
+}
+
+int ea_frameset_preprocess_gray_host(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* gray, const void* depth,
+                                     const uint8_t* ref_mask, const uint8_t* now_mask, int roles) {
+  int rc = check_gray_args(fs, n, slots, gray, depth, ref_mask, now_mask, roles);
+  if (rc) return rc;
+  ea_context* c = fs->ctx;
+  CU(cudaSetDevice(c->device));
+  const size_t px = size_t(fs->p.width) * fs->p.height;
+  const bool ref = (roles & EA_ROLE_REF) != 0;
+  // the staging area is sized for BGR frames; a gray frame set takes the first third of it
+  if (!fs->stage_bgr) CU(cudaMalloc((void**)&fs->stage_bgr, px * 3 * fs->n_slots));
+  if (ref && !fs->stage_depth) CU(cudaMalloc((void**)&fs->stage_depth, px * fs->depth_elem * fs->n_slots));
+  EaAsyncBuf d_masks(c->stream), d_slots(c->stream);
+  const int n_masks = (ref_mask ? 1 : 0) + (now_mask ? 1 : 0);
+  if (n_masks) CU(d_masks.alloc(px * n * n_masks));
+  CU(d_slots.alloc(size_t(n) * sizeof(int32_t)));
+  uint8_t* d_ref_mask = ref_mask ? d_masks.as<uint8_t>() : nullptr;
+  uint8_t* d_now_mask = now_mask ? d_masks.as<uint8_t>() + (ref_mask ? px * n : 0) : nullptr;
+  CU(cudaMemcpyAsync(fs->stage_bgr, gray, px * n, cudaMemcpyHostToDevice, c->stream));
+  if (ref) CU(cudaMemcpyAsync(fs->stage_depth, depth, px * fs->depth_elem * n, cudaMemcpyHostToDevice, c->stream));
+  if (ref_mask) CU(cudaMemcpyAsync(d_ref_mask, ref_mask, px * n, cudaMemcpyHostToDevice, c->stream));
+  if (now_mask) CU(cudaMemcpyAsync(d_now_mask, now_mask, px * n, cudaMemcpyHostToDevice, c->stream));
+  CU(cudaMemcpyAsync(d_slots.p, slots, size_t(n) * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+  rc = ea_preprocess_impl(fs, n, d_slots.as<int32_t>(), fs->stage_bgr, ref ? fs->stage_depth : nullptr, roles, d_ref_mask, d_now_mask,
+                          nullptr, 1);
+  if (rc == EA_OK && ref) rc = reset_points_mode(fs, n, slots);
+  return rc;
 }
 
 static int check_slot_level(ea_frameset* fs, int slot, int level) {

@@ -14,24 +14,27 @@ __device__ __forceinline__ int reflect101c(int i, int n) {
 __device__ __forceinline__ int clampi(int i, int n) { return i < 0 ? 0 : (i >= n ? n - 1 : i); }
 
 // cv::blur(3x3) (REFLECT_101, rounded /9) + cv::cvtColor(RGB2GRAY) on BGR data -> 8UC1   (utils.cpp:88-91)
+// CN = 1: gray input; RGB2GRAY of three equal channels is the identity, so the blurred value is the output
+template <int CN>
 __global__ void __launch_bounds__(256) k_box_gray(const uint8_t* __restrict__ bgr, size_t frame_stride_px, const int32_t* __restrict__ src_slots,
                                                   uint8_t* __restrict__ gray, size_t scratch_stride_px, int w, int h) {
   const int f = blockIdx.y;
-  const uint8_t* img = bgr + (src_slots ? size_t(src_slots[f]) : size_t(f)) * frame_stride_px * 3;
+  const uint8_t* img = bgr + (src_slots ? size_t(src_slots[f]) : size_t(f)) * frame_stride_px * CN;
   uint8_t* out = gray + size_t(f) * scratch_stride_px;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < w * h; i += gridDim.x * blockDim.x) {
     const int x = i % w, y = i / w;
-    int ch[3];
+    int ch[CN];
 #pragma unroll
-    for (int c = 0; c < 3; ++c) {
+    for (int c = 0; c < CN; ++c) {
       int acc = 0;
       for (int dy = -1; dy <= 1; ++dy) {
         const int yy = reflect101c(y + dy, h);
-        for (int dx = -1; dx <= 1; ++dx) acc += img[(size_t(yy) * w + reflect101c(x + dx, w)) * 3 + c];
+        for (int dx = -1; dx <= 1; ++dx) acc += img[(size_t(yy) * w + reflect101c(x + dx, w)) * CN + c];
       }
       ch[c] = __double2int_rn(double(acc) * (1.0 / 9.0));
     }
-    out[i] = uint8_t((ch[0] * 9798 + ch[1] * 19235 + ch[2] * 3735 + 16384) >> 15);
+    if constexpr (CN == 3) out[i] = uint8_t((ch[0] * 9798 + ch[1] * 19235 + ch[2] * 3735 + 16384) >> 15);
+    else out[i] = uint8_t(ch[0]);
   }
 }
 
@@ -209,7 +212,7 @@ __global__ void k_edt_affine(const unsigned* fminmax, const int32_t* dst_slots, 
 
 }  // namespace
 
-// Edge planes of level l by Canny.  src = BGR of that level.  scratch: gray u8 | mag i32 | dxy short2 | map u8, each
+// Edge planes of level l by Canny.  src = BGR (or gray, A.in_channels == 1) of that level.  scratch: gray u8 | mag i32 | dxy short2 | map u8, each
 // [n][stride] with stride = level-0 pixels.
 cudaError_t ea_launch_canny_level(const EaPrepArgs& A, int l, const uint8_t* bgr, const void* depth, size_t frame_stride_px,
                                   bool slot_indexed, const EaCannyCfg& cfg, const EaScratch& S, cudaStream_t stream, int* launches) {
@@ -225,10 +228,13 @@ cudaError_t ea_launch_canny_level(const EaPrepArgs& A, int l, const uint8_t* bgr
   }
   const int low = int(floor(t1)), high = int(floor(t2));
   if (cfg.on_color) {
-    k_canny_grad<3><<<grid, 256, 0, stream>>>(bgr, frame_stride_px, A.slots, slot_indexed, S.mag, S.dxy, S.stride, L.w, L.h, cfg.l2);
+    // on gray input the channel of largest gradient (first on ties) of (g, g, g) is g itself
+    if (A.in_channels == 1) k_canny_grad<1><<<grid, 256, 0, stream>>>(bgr, frame_stride_px, A.slots, slot_indexed, S.mag, S.dxy, S.stride, L.w, L.h, cfg.l2);
+    else k_canny_grad<3><<<grid, 256, 0, stream>>>(bgr, frame_stride_px, A.slots, slot_indexed, S.mag, S.dxy, S.stride, L.w, L.h, cfg.l2);
     ++*launches;
   } else {
-    k_box_gray<<<grid, 256, 0, stream>>>(bgr, frame_stride_px, slot_indexed ? A.slots : nullptr, S.gray, S.stride, L.w, L.h);
+    if (A.in_channels == 1) k_box_gray<1><<<grid, 256, 0, stream>>>(bgr, frame_stride_px, slot_indexed ? A.slots : nullptr, S.gray, S.stride, L.w, L.h);
+    else k_box_gray<3><<<grid, 256, 0, stream>>>(bgr, frame_stride_px, slot_indexed ? A.slots : nullptr, S.gray, S.stride, L.w, L.h);
     k_canny_grad<1><<<grid, 256, 0, stream>>>(S.gray, S.stride, nullptr, false, S.mag, S.dxy, S.stride, L.w, L.h, cfg.l2);
     *launches += 2;
   }

@@ -51,7 +51,7 @@ cudaError_t ea_launch_eval_sums(const EaLevelDesc& rd, const EaLevelDesc& nd, co
 
 // ---- preprocessing (ea_preprocess.cu) ---------------------------------------------------------------
 struct EaPrepLevel {            // device pointers of one pyramid level, slot-major pools
-  uint8_t* bgr;                 // [slots][h][w][3]   (level 0: null, the caller's input is read directly)
+  uint8_t* bgr;                 // [slots][h][w][3], or [slots][h][w] for gray input (level 0: null, the caller's input is read directly)
   void* depth;                  // [slots][h][w] u16 or f32 (level 0: null)
   uint32_t* edge_bits;          // [slots][h][words]  raw Laplacian>threshold mask, 1 bit / pixel
   uint32_t* ref_bits;           // [slots][h][words]  edge & depth>0
@@ -69,7 +69,8 @@ struct EaPrepArgs {
   EaPrepLevel lv[EA_MAX_LEVELS];
   int n_levels;
   const int32_t* slots;         // [n] device: destination slot of frame i
-  const uint8_t* in_bgr;        // [n][h0][w0][3]
+  const uint8_t* in_bgr;        // [n][h0][w0][in_channels]
+  int in_channels;              // 3: BGR; 1: gray, preprocessed exactly as BGR (g, g, g) would be
   const void* in_depth;         // [n][h0][w0] u16 raw units or f32 metres (depth_type), or null
   const uint8_t* in_mask;       // [n][h0][w0] or null: reference points only where mask > 0 (get_aX_mask, utils.cpp:283-369)
   const uint8_t* in_now_mask;   // [n][h0][w0] or null: now-frame edges only where mask > 1 (get_distance_transform2_masked, utils.cpp:124-128)
@@ -153,7 +154,7 @@ struct ea_frameset {
   unsigned* d_minmax = nullptr;
   float2* d_affine = nullptr;             // [n_slots][EA_MAX_LEVELS]
   int* d_overflow = nullptr;
-  uint8_t* stage_bgr = nullptr;           // [n_slots][h][w][3]  (host-upload staging)
+  uint8_t* stage_bgr = nullptr;           // [n_slots][h][w][3]  (host-upload staging; gray frames use its first third)
   void* stage_depth = nullptr;
   size_t depth_elem = 2;                  // bytes per depth sample (2: u16, 4: f32)
   double inv_depth_unit = 1.0 / 5000.0;   // metres per stored depth unit
@@ -205,4 +206,5 @@ int ea_solve_batch_device_ordered(ea_context* c, int n, ea_frameset* ref, const 
                                    const int32_t* d_order, const ea_solve_params* sp, ea_summary* d_summaries, bool tail_helpers = true);
 cudaError_t ea_launch_order_by_work(const ea_summary* d_summaries, int n, int n_levels, int32_t* d_order, cudaStream_t stream);
 int ea_preprocess_impl(ea_frameset* fs, int n, const int32_t* d_slots, const uint8_t* d_bgr, const void* d_depth, int roles,
-                       const uint8_t* d_mask = nullptr, const uint8_t* d_now_mask = nullptr, cudaStream_t stream = nullptr);
+                       const uint8_t* d_mask = nullptr, const uint8_t* d_now_mask = nullptr, cudaStream_t stream = nullptr,
+                       int in_channels = 3);

@@ -19,8 +19,9 @@ __device__ __forceinline__ int reflect101(int i, int n) {
   return i;
 }
 
-// ---- pyramid: cv::resize(0.5) INTER_LINEAR on BGR (== 2x2 mean, +2 >> 2), INTER_NEAREST on depth ---------
-template <typename D>
+// ---- pyramid: cv::resize(0.5) INTER_LINEAR on BGR or gray (== 2x2 mean, +2 >> 2, per channel), INTER_NEAREST on depth
+// CN: channels of the image (3: BGR, 1: gray)
+template <typename D, int CN>
 __global__ void __launch_bounds__(256) k_pyr_down(const uint8_t* __restrict__ src_bgr, const D* __restrict__ src_depth,
                                                   size_t src_frame_stride_px, const int32_t* __restrict__ src_slots,
                                                   uint8_t* __restrict__ dst_bgr, D* __restrict__ dst_depth,
@@ -31,19 +32,19 @@ __global__ void __launch_bounds__(256) k_pyr_down(const uint8_t* __restrict__ sr
   const size_t dbase = size_t(dst_slots[f]) * size_t(dw) * dh;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < dw * dh; i += gridDim.x * blockDim.x) {
     const int x = i % dw, y = i / dw;
-    const uint8_t* p = src_bgr + (sbase + size_t(2 * y) * sw + 2 * x) * 3;
-    const uint8_t* q = p + size_t(sw) * 3;
-    uint8_t* d = dst_bgr + (dbase + i) * 3;
+    const uint8_t* p = src_bgr + (sbase + size_t(2 * y) * sw + 2 * x) * CN;
+    const uint8_t* q = p + size_t(sw) * CN;
+    uint8_t* d = dst_bgr + (dbase + i) * CN;
 #pragma unroll
-    for (int c = 0; c < 3; ++c) d[c] = uint8_t((p[c] + p[3 + c] + q[c] + q[3 + c] + 2) >> 2);
+    for (int c = 0; c < CN; ++c) d[c] = uint8_t((p[c] + p[CN + c] + q[c] + q[CN + c] + 2) >> 2);
     if (src_depth) dst_depth[dbase + i] = src_depth[sbase + size_t(2 * y) * sw + 2 * x];
   }
 }
 
-// Same arithmetic, four output pixels per thread: 2 x 24 source bytes as 8-byte loads, 12 result bytes as 4-byte stores
-// (the byte-per-load version above moves 3.3 TB/s; frames whose rows allow it take this one).  Needs dw % 4 == 0 and
+// Same arithmetic, four output pixels per thread: 2 x 8 CN source bytes as 8-byte loads, 4 CN result bytes as 4-byte stores
+// (the byte-per-load version above moves 3.3 TB/s on BGR; frames whose rows allow it take this one).  Needs dw % 4 == 0 and
 // 8-byte aligned frame bases.
-template <typename D>
+template <typename D, int CN>
 __global__ void __launch_bounds__(256) k_pyr_down4(const uint8_t* __restrict__ src_bgr, const D* __restrict__ src_depth,
                                                    size_t src_frame_stride_px, const int32_t* __restrict__ src_slots,
                                                    uint8_t* __restrict__ dst_bgr, D* __restrict__ dst_depth,
@@ -54,19 +55,20 @@ __global__ void __launch_bounds__(256) k_pyr_down4(const uint8_t* __restrict__ s
   const size_t dbase = size_t(dst_slots[f]) * size_t(dw) * dh;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < qw * dh; i += gridDim.x * blockDim.x) {
     const int xq = i % qw, y = i / qw;
-    const uint2* p = reinterpret_cast<const uint2*>(src_bgr + (sbase + size_t(2 * y) * sw + size_t(8 * xq)) * 3);
-    const uint2* q = reinterpret_cast<const uint2*>(src_bgr + (sbase + size_t(2 * y + 1) * sw + size_t(8 * xq)) * 3);
-    union { uint2 v[3]; unsigned char b[24]; } a, c;
+    const uint2* p = reinterpret_cast<const uint2*>(src_bgr + (sbase + size_t(2 * y) * sw + size_t(8 * xq)) * CN);
+    const uint2* q = reinterpret_cast<const uint2*>(src_bgr + (sbase + size_t(2 * y + 1) * sw + size_t(8 * xq)) * CN);
+    union { uint2 v[CN]; unsigned char b[8 * CN]; } a, c;
 #pragma unroll
-    for (int k = 0; k < 3; ++k) { a.v[k] = __ldg(p + k); c.v[k] = __ldg(q + k); }
-    union { unsigned w[3]; unsigned char b[12]; } o;
+    for (int k = 0; k < CN; ++k) { a.v[k] = __ldg(p + k); c.v[k] = __ldg(q + k); }
+    union { unsigned w[CN]; unsigned char b[4 * CN]; } o;
 #pragma unroll
     for (int px = 0; px < 4; ++px)
 #pragma unroll
-      for (int ch = 0; ch < 3; ++ch)
-        o.b[3 * px + ch] = (unsigned char)((a.b[6 * px + ch] + a.b[6 * px + 3 + ch] + c.b[6 * px + ch] + c.b[6 * px + 3 + ch] + 2) >> 2);
-    unsigned* d = reinterpret_cast<unsigned*>(dst_bgr + (dbase + size_t(y) * dw + size_t(4 * xq)) * 3);
-    d[0] = o.w[0]; d[1] = o.w[1]; d[2] = o.w[2];
+      for (int ch = 0; ch < CN; ++ch)
+        o.b[CN * px + ch] = (unsigned char)((a.b[2 * CN * px + ch] + a.b[2 * CN * px + CN + ch] + c.b[2 * CN * px + ch] + c.b[2 * CN * px + CN + ch] + 2) >> 2);
+    unsigned* d = reinterpret_cast<unsigned*>(dst_bgr + (dbase + size_t(y) * dw + size_t(4 * xq)) * CN);
+#pragma unroll
+    for (int k = 0; k < CN; ++k) d[k] = o.w[k];
     if (src_depth) {
 #pragma unroll
       for (int px = 0; px < 4; ++px) dst_depth[dbase + size_t(y) * dw + 4 * xq + px] = src_depth[sbase + size_t(2 * y) * sw + 2 * (4 * xq + px)];
@@ -75,41 +77,43 @@ __global__ void __launch_bounds__(256) k_pyr_down4(const uint8_t* __restrict__ s
 }
 
 // ---- fused GaussianBlur3 -> RGB2GRAY -> Laplacian3 -> |.| saturate -> threshold -> bit mask ----------------
-// Block = 32x8 pixels; one ballot word per warp row.
+// Block = 32x8 pixels; one ballot word per warp row.  CN = 1: gray input, blurred straight into the gray tile (RGB2GRAY of
+// three equal channels is the identity: 9798 + 19235 + 3735 == 1 << 15).
 #define ET_W 32
 #define ET_H 8
-template <typename D>
+template <typename D, int CN>
 __global__ void __launch_bounds__(256) k_edge_mask(const uint8_t* __restrict__ bgr, const D* __restrict__ depth,
                                                    size_t frame_stride_px, const int32_t* __restrict__ src_slots,
                                                    const int32_t* __restrict__ dst_slots, uint32_t* __restrict__ edge_bits,
                                                    uint32_t* __restrict__ ref_bits, int w, int h, int words, int thresh, int zero_to_one) {
-  __shared__ uint8_t tile[ET_H + 4][(ET_W + 4) * 3 + 4];
+  __shared__ uint8_t tile[ET_H + 4][(ET_W + 4) * CN + 4];
   __shared__ uint8_t gray[ET_H + 2][ET_W + 2 + 2];
   const int f = blockIdx.z;
   const size_t sbase = (src_slots ? size_t(src_slots[f]) : size_t(f)) * frame_stride_px;
   const int x0 = blockIdx.x * ET_W, y0 = blockIdx.y * ET_H;
   const int tid = threadIdx.y * ET_W + threadIdx.x;
-  // stage the BGR tile with a 2-pixel halo; outside the image map through REFLECT_101 (the composition of the
+  // stage the tile with a 2-pixel halo; outside the image map through REFLECT_101 (the composition of the
   // blur's and the Laplacian's border handling reduces to this because both kernels are symmetric)
-  for (int i = tid; i < (ET_H + 4) * (ET_W + 4) * 3; i += 256) {
-    const int row = i / ((ET_W + 4) * 3), b = i % ((ET_W + 4) * 3);
-    const int px = b / 3, c = b % 3;
+  for (int i = tid; i < (ET_H + 4) * (ET_W + 4) * CN; i += 256) {
+    const int row = i / ((ET_W + 4) * CN), b = i % ((ET_W + 4) * CN);
+    const int px = b / CN, c = b % CN;
     const int gx = reflect101(x0 - 2 + px, w), gy = reflect101(y0 - 2 + row, h);
-    tile[row][b] = bgr[(sbase + size_t(gy) * w + gx) * 3 + c];
+    tile[row][b] = bgr[(sbase + size_t(gy) * w + gx) * CN + c];
   }
   __syncthreads();
   for (int i = tid; i < (ET_H + 2) * (ET_W + 2); i += 256) {
     const int gyr = i / (ET_W + 2), gxr = i % (ET_W + 2);  // gray position == tile position (gxr+1, gyr+1)
-    int ch[3];
+    int ch[CN];
 #pragma unroll
-    for (int c = 0; c < 3; ++c) {
-      const uint8_t* r0 = &tile[gyr][gxr * 3 + c];
-      const uint8_t* r1 = &tile[gyr + 1][gxr * 3 + c];
-      const uint8_t* r2 = &tile[gyr + 2][gxr * 3 + c];
-      const int s = (r0[0] + 2 * r0[3] + r0[6]) + 2 * (r1[0] + 2 * r1[3] + r1[6]) + (r2[0] + 2 * r2[3] + r2[6]);
+    for (int c = 0; c < CN; ++c) {
+      const uint8_t* r0 = &tile[gyr][gxr * CN + c];
+      const uint8_t* r1 = &tile[gyr + 1][gxr * CN + c];
+      const uint8_t* r2 = &tile[gyr + 2][gxr * CN + c];
+      const int s = (r0[0] + 2 * r0[CN] + r0[2 * CN]) + 2 * (r1[0] + 2 * r1[CN] + r1[2 * CN]) + (r2[0] + 2 * r2[CN] + r2[2 * CN]);
       ch[c] = (s + 8) >> 4;                       // GaussianBlur 3x3 sigma 0: [1 2 1]/4 separable, one rounding
     }
-    gray[gyr][gxr] = uint8_t((ch[0] * 9798 + ch[1] * 19235 + ch[2] * 3735 + 16384) >> 15);  // RGB2GRAY on BGR data
+    if constexpr (CN == 3) gray[gyr][gxr] = uint8_t((ch[0] * 9798 + ch[1] * 19235 + ch[2] * 3735 + 16384) >> 15);  // RGB2GRAY on BGR data
+    else gray[gyr][gxr] = uint8_t(ch[0]);
   }
   __syncthreads();
   const int lx = threadIdx.x, ly = threadIdx.y, x = x0 + lx, y = y0 + ly;
@@ -147,6 +151,46 @@ __device__ __forceinline__ unsigned e2_gray(unsigned v_bg, unsigned v_r) {
   const unsigned b_r = (v_r + 8u) >> 4;
   const unsigned B = b_bg & 0xFFFFu, G = b_bg >> 16;
   return (B * 9798u + G * 19235u + b_r * 3735u + 16384u) >> 15;
+}
+
+// Phase 3 of the fused edge kernels: Laplacian (ksize 3) + convertScaleAbs + threshold over the gray tile (column g <-> image
+// column x0 - 1 + g, row r <-> image row y0 - 1 + r), one ballot word per warp row; REF: also the reference-point plane.
+// min(|v|, 255) > thresh  <=>  |v| > thresh for thresh < 255 (never true above); columns beyond the image read gray
+// column 0 (harmless) and vote "no edge"; the row loop stops at the image's last row.
+template <typename D, int TW, bool REF>
+__device__ __forceinline__ void e2_laplacian_bits(const uint8_t (*gray)[TW + 4], const D* __restrict__ depth, size_t sbase, int dst_slot,
+                                                  uint32_t* __restrict__ edge_bits, uint32_t* __restrict__ ref_bits, int x0, int y0,
+                                                  int w, int h, int words, int thresh, int zero_to_one) {
+  const int t = threadIdx.x;
+  const int x = x0 + t, lane = t & 31, wq = t >> 5;
+  const bool col_ok = x < w;
+  const int gl = col_ok ? reflect101(x - 1, w) - x0 + 1 : 0, gc = col_ok ? t + 1 : 0, gr = col_ok ? reflect101(x + 1, w) - x0 + 1 : 0;
+  const int thr = (col_ok && thresh < 255) ? thresh : 0x7fffffff;
+  const int rows = min(E2_TH, h - y0);
+  int s0 = gray[0][gl] + gray[0][gr];
+  int s1 = gray[1][gl] + gray[1][gr], c1 = gray[1][gc];
+  const bool writer = lane == 0 && (x0 >> 5) + wq < words;
+  const size_t o0 = (size_t(dst_slot) * h + y0) * words + (x0 >> 5) + wq;
+  uint32_t* eo = edge_bits + o0;
+  uint32_t* ro = REF ? ref_bits + o0 : nullptr;
+  const D* dep = REF ? depth + sbase + size_t(y0) * w + (col_ok ? x : 0) : nullptr;
+#pragma unroll 4
+  for (int r = 0; r < rows; ++r) {
+    const int s2 = gray[r + 2][gl] + gray[r + 2][gr], c2 = gray[r + 2][gc];
+    const int v = 2 * (s0 + s2) - 8 * c1;
+    const bool edge = abs(v) > thr;
+    const unsigned eb = __ballot_sync(0xffffffffu, edge);
+    if (REF) {
+      bool valid = false;
+      if (edge) valid = zero_to_one || dep[0] > D(0);
+      const unsigned rb = __ballot_sync(0xffffffffu, valid);
+      if (writer) *ro = rb;
+      ro += words; dep += w;
+    }
+    if (writer) *eo = eb;
+    eo += words;
+    s0 = s1; s1 = s2; c1 = c2;
+  }
 }
 
 // TW = tile width = threads per CTA (128; 64 for levels whose width is a multiple of 64 but not of 128, where a 128-wide
@@ -267,38 +311,102 @@ __global__ void __launch_bounds__(TW) k_edge_mask2(const uint8_t* __restrict__ b
     }
   }
   __syncthreads();
-  // ---- phase 3: Laplacian (ksize 3) + convertScaleAbs + threshold, one ballot word per warp row ----
-  // min(|v|, 255) > thresh  <=>  |v| > thresh for thresh < 255 (never true above); columns beyond the image read gray
-  // column 0 (harmless) and vote "no edge"; the row loop stops at the image's last row.
-  const int x = x0 + t, lane = t & 31, wq = t >> 5;
-  const bool col_ok = x < w;
-  const int gl = col_ok ? reflect101(x - 1, w) - x0 + 1 : 0, gc = col_ok ? t + 1 : 0, gr = col_ok ? reflect101(x + 1, w) - x0 + 1 : 0;
-  const int thr = (col_ok && thresh < 255) ? thresh : 0x7fffffff;
-  const int rows = min(E2_TH, h - y0);
-  int s0 = gray[0][gl] + gray[0][gr];
-  int s1 = gray[1][gl] + gray[1][gr], c1 = gray[1][gc];
-  const bool writer = lane == 0 && (x0 >> 5) + wq < words;
-  const size_t o0 = (size_t(dst_slots[f]) * h + y0) * words + (x0 >> 5) + wq;
-  uint32_t* eo = edge_bits + o0;
-  uint32_t* ro = REF ? ref_bits + o0 : nullptr;
-  const D* dep = REF ? depth + sbase + size_t(y0) * w + (col_ok ? x : 0) : nullptr;
-#pragma unroll 4
-  for (int r = 0; r < rows; ++r) {
-    const int s2 = gray[r + 2][gl] + gray[r + 2][gr], c2 = gray[r + 2][gc];
-    const int v = 2 * (s0 + s2) - 8 * c1;
-    const bool edge = abs(v) > thr;
-    const unsigned eb = __ballot_sync(0xffffffffu, edge);
-    if (REF) {
-      bool valid = false;
-      if (edge) valid = zero_to_one || dep[0] > D(0);
-      const unsigned rb = __ballot_sync(0xffffffffu, valid);
-      if (writer) *ro = rb;
-      ro += words; dep += w;
+  // ---- phase 3 ----
+  e2_laplacian_bits<D, TW, REF>(gray, depth, sbase, dst_slots[f], edge_bits, ref_bits, x0, y0, w, h, words, thresh, zero_to_one);
+}
+
+// ---- k_edge_mask2 on 8-bit gray input: the same edges as k_edge_mask2 on BGR (g, g, g), from a third of the bytes ----------
+// RGB2GRAY of three equal blurred channels is the identity (9798 + 19235 + 3735 == 1 << 15, rounding constant half of it), so
+// the blur goes straight into the gray tile.  The byte tile is staged REFLECT_101-padded (columns outside the image hold their
+// mirror image), which makes every gray column -- the two halo columns too -- a contiguous 3-tap window: each thread blurs two
+// adjacent columns in 16-bit lanes over one half of the tile's rows.  Phase 3 is k_edge_mask2's.  Needs w % 4 == 0 and a
+// 4-byte aligned image (32-bit row loads, 4 pixels each).
+template <typename D, int TW, bool REF>
+__global__ void __launch_bounds__(TW) k_edge_mask2_gray(const uint8_t* __restrict__ src, const D* __restrict__ depth,
+                                                          size_t frame_stride_px, const int32_t* __restrict__ src_slots,
+                                                          const int32_t* __restrict__ dst_slots, uint32_t* __restrict__ edge_bits,
+                                                          uint32_t* __restrict__ ref_bits, int w, int h, int words, int thresh, int zero_to_one,
+                                                          uint8_t* __restrict__ pyr, D* __restrict__ pyr_depth) {
+  constexpr int PW = TW + 8;          // tile bytes per row: image columns x0-4 .. x0+TW+3
+  constexpr int GW = TW + 4;          // gray tile: columns x0-1 .. x0+TW (+2 pad)
+  constexpr int NG = PW / 4;          // 4-pixel words per tile row
+  constexpr int RS = TW / NG;         // tile rows staged per pass
+  constexpr int NP = (TW + 2) / 2;    // gray column pairs, halo columns included
+  constexpr int H2 = (E2_TH + 2) / 2; // gray rows per half
+  __shared__ __align__(16) uint8_t tile[E2_PH][PW];
+  __shared__ __align__(16) uint8_t gray[E2_TH + 2][GW];
+  const int f = blockIdx.z;
+  const size_t sbase = (src_slots ? size_t(src_slots[f]) : size_t(f)) * frame_stride_px;
+  const int x0 = blockIdx.x * TW, y0 = blockIdx.y * E2_TH;
+  const int t = threadIdx.x;
+  const uint8_t* img = src + sbase;
+  // ---- phase 1: one 32-bit load = 4 pixels; groups outside the image are gathered through REFLECT_101 byte by byte ----
+  {
+    const int g = t % NG, rr = t / NG;
+    const int col = x0 - 4 + 4 * g;                       // first image column of the group (multiple of 4)
+    const bool inside = col >= 0 && col + 3 < w;
+    const int m0 = reflect101(col, w), m1 = reflect101(col + 1, w), m2 = reflect101(col + 2, w), m3 = reflect101(col + 3, w);
+    if (rr < RS) {
+#pragma unroll 2
+      for (int r = rr; r < E2_PH; r += RS) {
+        // rows y0-2 .. h+1 are all that the tile's outputs can reach (h >= 4: one reflection maps them inside); the rest stay unstaged
+        const int y = y0 - 2 + r;
+        if (y > h + 1) break;
+        int ry = abs(y);
+        ry = ry >= h ? 2 * h - 2 - ry : ry;
+        const uint8_t* row = img + size_t(unsigned(ry) * unsigned(w));
+        unsigned v;
+        if (inside) v = __ldg(reinterpret_cast<const unsigned*>(row + col));
+        else v = unsigned(row[m0]) | unsigned(row[m1]) << 8 | unsigned(row[m2]) << 16 | unsigned(row[m3]) << 24;
+        *reinterpret_cast<unsigned*>(&tile[r][4 * g]) = v;
+      }
     }
-    if (writer) *eo = eb;
-    eo += words;
-    s0 = s1; s1 = s2; c1 = c2;
   }
+  __syncthreads();
+  // ---- next pyramid level from the staged tile (pyr != null): (a+b+c+d+2) >> 2 in 16-bit lanes, four output pixels per 32-bit
+  //      store; INTER_NEAREST on depth (key frames) ----
+  if (pyr) {
+    const int dw = w >> 1, dh = h >> 1;
+    const size_t dbase = size_t(dst_slots[f]) * size_t(dw) * dh;
+    for (int i = t; i < (TW / 8) * (E2_TH / 2); i += TW) {
+      const int yl = i / (TW / 8), xq = i % (TW / 8);
+      const int oy = (y0 >> 1) + yl, ox = (x0 >> 1) + 4 * xq;
+      if (oy >= dh || ox + 3 >= dw) continue;
+      const unsigned* a = reinterpret_cast<const unsigned*>(&tile[2 * yl + 2][8 * xq + 4]);
+      const unsigned* b = reinterpret_cast<const unsigned*>(&tile[2 * yl + 3][8 * xq + 4]);
+      // {p0 + p1, p2 + p3} of a 4-pixel word in 16-bit lanes
+      auto pairs = [](unsigned v) { return __byte_perm(v, 0, 0x4240) + __byte_perm(v, 0, 0x4341); };
+      const unsigned m01 = ((pairs(a[0]) + pairs(b[0]) + 0x00020002u) >> 2) & 0x00FF00FFu;
+      const unsigned m23 = ((pairs(a[1]) + pairs(b[1]) + 0x00020002u) >> 2) & 0x00FF00FFu;
+      *reinterpret_cast<unsigned*>(pyr + dbase + size_t(oy) * dw + ox) = __byte_perm(m01, m23, 0x6420);
+      if (REF && pyr_depth) {
+        const D* sd = depth + sbase + size_t(2 * oy) * w + 2 * ox;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) pyr_depth[dbase + size_t(oy) * dw + ox + j] = sd[2 * j];
+      }
+    }
+  }
+  // ---- phase 2: rolling 3x3 blur of gray columns (g, g+1) <-> image columns x0-1+g, x0+g; item = (pair, half of the rows) ----
+  for (int it = t; it < 2 * NP; it += TW) {
+    const int g = 2 * (it % NP), r0 = (it / NP) * H2;
+    const int wi = g >> 2;
+    const bool aligned = (g & 2) != 0;                  // tile bytes g+2 .. g+5 (left, centre, centre, right) are word wi + 1
+    unsigned h0 = 0, h1 = 0;
+#pragma unroll 4
+    for (int r = 0; r < H2 + 2; ++r) {
+      const unsigned* row = reinterpret_cast<const unsigned*>(&tile[r0 + r][0]);
+      const unsigned v = aligned ? row[wi + 1] : __byte_perm(row[wi], row[wi + 1], 0x5432);
+      const unsigned hs = __byte_perm(v, 0, 0x4140) + (__byte_perm(v, 0, 0x4241) << 1) + __byte_perm(v, 0, 0x4342);
+      if (r >= 2) {
+        const unsigned s = ((h0 + hs + (h1 << 1) + 0x00080008u) >> 4) & 0x00FF00FFu;
+        *reinterpret_cast<uint16_t*>(&gray[r0 + r - 2][g]) = uint16_t(__byte_perm(s, 0, 0x0020));
+      }
+      h0 = h1; h1 = hs;
+    }
+  }
+  __syncthreads();
+  // ---- phase 3 ----
+  e2_laplacian_bits<D, TW, REF>(gray, depth, sbase, dst_slots[f], edge_bits, ref_bits, x0, y0, w, h, words, thresh, zero_to_one);
 }
 
 // ---- masks: keep set bits only where mask > thr (level l samples mask(x<<l, y<<l)) ----------------------------
@@ -871,18 +979,36 @@ __global__ void __launch_bounds__(256) k_unpack_mask(const uint32_t* __restrict_
 
 }  // namespace
 
-// can level l's Laplacian edge kernel (k_edge_mask2) also emit level l + 1's BGR / depth from its staged tile?
+// the gray edge kernel loads whole 32-bit words of level l's image: a caller's device pointer that is not 4-byte aligned takes the
+// byte path (k_edge_mask) instead
+static bool gray_words_ok(const EaPrepArgs& A, int l) {
+  return A.in_channels != 1 || (reinterpret_cast<uintptr_t>(l == 0 ? A.in_bgr : A.lv[l].bgr) & 3) == 0;
+}
+// can level l's Laplacian edge kernel (k_edge_mask2 / k_edge_mask2_gray) also emit level l + 1's image / depth from its staged
+// tile?  (Both store whole 32-bit words of level l + 1: 4 BGR pixels in 3 words, or 4 gray pixels in one; next level's width a
+// multiple of 4 and a 4-byte aligned pool keep every such word aligned in either layout.)
 static bool edge_kernel_fuses_pyramid(const EaPrepArgs& A, int l) {
   if (l + 1 >= A.n_levels || A.edge_detector != EA_EDGE_LAPLACIAN) return false;
   const EaPrepLevel& L = A.lv[l];
   const EaPrepLevel& N = A.lv[l + 1];
   static const int env_fuse = getenv("EA_PYR_FUSE") ? atoi(getenv("EA_PYR_FUSE")) : 1;
-  return env_fuse && (L.w & 3) == 0 && L.w >= 8 && L.h >= 4 && (N.w & 3) == 0 && (reinterpret_cast<uintptr_t>(N.bgr) & 3) == 0;
+  return env_fuse && (L.w & 3) == 0 && L.w >= 8 && L.h >= 4 && gray_words_ok(A, l) && (N.w & 3) == 0 && (reinterpret_cast<uintptr_t>(N.bgr) & 3) == 0;
+}
+
+// the fused edge kernel of one level for CN-channel input (k_edge_mask2 on BGR, k_edge_mask2_gray on gray)
+template <typename D, int TW, bool REF>
+static void launch_edge_mask2(const EaPrepArgs& A, const EaPrepLevel& L, const uint8_t* b, const D* d, size_t pxl, const int32_t* ss,
+                              uint8_t* nb, D* nd, cudaStream_t stream) {
+  dim3 grid(unsigned((L.w + TW - 1) / TW), unsigned((L.h + E2_TH - 1) / E2_TH), unsigned(A.n));
+  uint32_t* rb = REF ? L.ref_bits : nullptr;
+  if (A.in_channels == 1) k_edge_mask2_gray<D, TW, REF><<<grid, TW, 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
+  else k_edge_mask2<D, TW, REF><<<grid, TW, 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
 }
 
 template <typename D>
 static cudaError_t launch_edges_and_points(const EaPrepArgs& A, cudaStream_t stream, int& nl) {
   const bool want_ref = (A.roles & EA_ROLE_REF) != 0;
+  const bool gray = A.in_channels == 1;
   const size_t px0 = size_t(A.lv[0].w) * A.lv[0].h;
   const D* in_depth = static_cast<const D*>(A.in_depth);
   for (int l = 0; l < A.n_levels; ++l) {
@@ -893,13 +1019,17 @@ static cudaError_t launch_edges_and_points(const EaPrepArgs& A, cudaStream_t str
       const uint8_t* sb = (l == 1) ? A.in_bgr : S.bgr;
       const D* sd = want_ref ? ((l == 1) ? in_depth : static_cast<const D*>(S.depth)) : nullptr;
       const size_t sstride = (l == 1) ? px0 : size_t(S.w) * S.h;
+      const int32_t* sslots = (l == 1) ? nullptr : A.slots;
+      D* dd = static_cast<D*>(L.depth);
       const bool vec4 = ((L.w & 3) == 0) && ((reinterpret_cast<uintptr_t>(sb) & 7) == 0) && ((reinterpret_cast<uintptr_t>(L.bgr) & 3) == 0);
       if (vec4) {
         dim3 grid(unsigned((pxl / 4 + 255) / 256), unsigned(A.n));
-        k_pyr_down4<D><<<grid, 256, 0, stream>>>(sb, sd, sstride, (l == 1) ? nullptr : A.slots, L.bgr, static_cast<D*>(L.depth), A.slots, S.w, S.h);
+        if (gray) k_pyr_down4<D, 1><<<grid, 256, 0, stream>>>(sb, sd, sstride, sslots, L.bgr, dd, A.slots, S.w, S.h);
+        else k_pyr_down4<D, 3><<<grid, 256, 0, stream>>>(sb, sd, sstride, sslots, L.bgr, dd, A.slots, S.w, S.h);
       } else {
         dim3 grid(unsigned((pxl + 255) / 256), unsigned(A.n));
-        k_pyr_down<D><<<grid, 256, 0, stream>>>(sb, sd, sstride, (l == 1) ? nullptr : A.slots, L.bgr, static_cast<D*>(L.depth), A.slots, S.w, S.h);
+        if (gray) k_pyr_down<D, 1><<<grid, 256, 0, stream>>>(sb, sd, sstride, sslots, L.bgr, dd, A.slots, S.w, S.h);
+        else k_pyr_down<D, 3><<<grid, 256, 0, stream>>>(sb, sd, sstride, sslots, L.bgr, dd, A.slots, S.w, S.h);
       }
       ++nl;
     }
@@ -911,22 +1041,22 @@ static cudaError_t launch_edges_and_points(const EaPrepArgs& A, cudaStream_t str
       cudaError_t ce = ea_launch_canny_level(A, l, b, d, pxl, l != 0, A.canny, A.scratch, stream, &k);
       nl += k - 1;
       if (ce != cudaSuccess) return ce;
-    } else if ((L.w & 3) == 0 && L.w >= 8 && L.h >= 4) {
+    } else if ((L.w & 3) == 0 && L.w >= 8 && L.h >= 4 && gray_words_ok(A, l)) {
       const bool fuse = edge_kernel_fuses_pyramid(A, l);
       uint8_t* nb = fuse ? A.lv[l + 1].bgr : nullptr;
       D* nd = (fuse && want_ref) ? static_cast<D*>(A.lv[l + 1].depth) : nullptr;
       if ((L.w % 128) != 0 && (L.w % 128) <= 64) {   // the last 128-wide tile would be at most half full: 64-wide tiles
-        dim3 grid(unsigned((L.w + 63) / 64), unsigned((L.h + E2_TH - 1) / E2_TH), unsigned(A.n));
-        if (want_ref) k_edge_mask2<D, 64, true><<<grid, 64, 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, L.ref_bits, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
-        else k_edge_mask2<D, 64, false><<<grid, 64, 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, nullptr, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
+        if (want_ref) launch_edge_mask2<D, 64, true>(A, L, b, d, pxl, ss, nb, nd, stream);
+        else launch_edge_mask2<D, 64, false>(A, L, b, d, pxl, ss, nb, nd, stream);
       } else {
-        dim3 grid(unsigned((L.w + E2_TW - 1) / E2_TW), unsigned((L.h + E2_TH - 1) / E2_TH), unsigned(A.n));
-        if (want_ref) k_edge_mask2<D, E2_TW, true><<<grid, E2_TW, 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, L.ref_bits, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
-        else k_edge_mask2<D, E2_TW, false><<<grid, E2_TW, 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, nullptr, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
+        if (want_ref) launch_edge_mask2<D, E2_TW, true>(A, L, b, d, pxl, ss, nb, nd, stream);
+        else launch_edge_mask2<D, E2_TW, false>(A, L, b, d, pxl, ss, nb, nd, stream);
       }
     } else {   // generic byte path (any width)
       dim3 grid(unsigned((L.w + ET_W - 1) / ET_W), unsigned((L.h + ET_H - 1) / ET_H), unsigned(A.n));
-      k_edge_mask<D><<<grid, dim3(ET_W, ET_H), 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, want_ref ? L.ref_bits : nullptr, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one);
+      uint32_t* rb = want_ref ? L.ref_bits : nullptr;
+      if (gray) k_edge_mask<D, 1><<<grid, dim3(ET_W, ET_H), 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one);
+      else k_edge_mask<D, 3><<<grid, dim3(ET_W, ET_H), 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one);
     }
     ++nl;
     if (want_ref && A.in_mask) {
@@ -992,7 +1122,7 @@ static EaPrepArgs prep_slice(const EaPrepArgs& A, int f0, int n) {
   EaPrepArgs S = A;
   const size_t px0 = size_t(A.lv[0].w) * A.lv[0].h;
   S.n = n; S.slots = A.slots + f0;
-  S.in_bgr = A.in_bgr + size_t(f0) * px0 * 3;
+  S.in_bgr = A.in_bgr + size_t(f0) * px0 * A.in_channels;
   if (A.in_depth) S.in_depth = static_cast<const char*>(A.in_depth) + size_t(f0) * px0 * (A.depth_type == 1 ? 4 : 2);
   if (A.in_mask) S.in_mask = A.in_mask + size_t(f0) * px0;
   if (A.in_now_mask) S.in_now_mask = A.in_now_mask + size_t(f0) * px0;

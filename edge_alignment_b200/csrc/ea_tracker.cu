@@ -33,6 +33,7 @@ struct ea_tracker {
   cudaStream_t prep_stream = nullptr;
   cudaEvent_t ev_prep[2] = {nullptr, nullptr}, ev_solved[2] = {nullptr, nullptr};
   int inputs_ready = 0;            // ea_tracker_set_inputs_ready: device inputs are complete at call time (not stream-ordered)
+  int channels = 3;                // image bytes per pixel: 3 (EA_IMAGE_BGR8) or 1 (EA_IMAGE_GRAY8)
   double* d_poses = nullptr;       // warm-start table [n_streams][7]
   double* d_result = nullptr;      // poses of the latest step [n_streams][7]
   double* d_identity = nullptr;    // [n_streams][7]
@@ -41,7 +42,7 @@ struct ea_tracker {
   bool have_order = false;
   // host-input pipeline: frame t+1 is uploaded on a copy stream while frame t is being aligned
   cudaStream_t copy_stream = nullptr;
-  uint8_t* stage_bgr[2] = {nullptr, nullptr};
+  uint8_t* stage_bgr[2] = {nullptr, nullptr};   // [n_streams][h][w][channels]
   void* stage_depth[2] = {nullptr, nullptr};
   cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_consumed[2] = {nullptr, nullptr}, ev_result[2] = {nullptr, nullptr};
   double* h_poses[2] = {nullptr, nullptr};          // pinned result ring
@@ -156,7 +157,7 @@ static int tracker_step(ea_tracker* t, const uint8_t* d_bgr, const void* d_depth
     CU(cudaStreamWaitEvent(ps, t->ev_prep[fb], 0));
   }
   if (t->frame >= 3) CU(cudaStreamWaitEvent(ps, t->ev_solved[fb], 0));   // last reader of this slot set: the solve of frame - 2
-  int rc = ea_preprocess_impl(t->fs, t->n_streams, t->d_slots[cur], d_bgr, d_depth, roles, nullptr, nullptr, ps);
+  int rc = ea_preprocess_impl(t->fs, t->n_streams, t->d_slots[cur], d_bgr, d_depth, roles, nullptr, nullptr, ps, t->channels);
   if (rc) return rc;
   CU(cudaEventRecord(t->ev_prep[fb], ps));
   if (consumed) CU(cudaEventRecord(consumed, ps));              // the input buffers may be overwritten from here on
@@ -195,6 +196,20 @@ int ea_tracker_step_device(ea_tracker* t, const uint8_t* d_bgr, const void* d_de
   return tracker_step(t, d_bgr, d_depth, nullptr, nullptr);
 }
 
+int ea_tracker_set_image_format(ea_tracker* t, int image_format) {
+  if (!t) return ea_fail(EA_ERR_INVALID_ARG, "null tracker");
+  if (image_format != EA_IMAGE_BGR8 && image_format != EA_IMAGE_GRAY8) return ea_fail(EA_ERR_INVALID_ARG, "unknown image format %d", image_format);
+  if (t->frame != 0) return ea_fail(EA_ERR_STATE, "the image format can only change before the first step (after create or reset)");
+  const int channels = image_format == EA_IMAGE_GRAY8 ? 1 : 3;
+  if (channels != t->channels) {   // the host-path staging buffers are sized for the format; the next step_host allocates them anew
+    CU(cudaSetDevice(t->ctx->device));
+    CU(cudaStreamSynchronize(t->copy_stream));
+    for (int b = 0; b < 2; ++b) { CU(cudaFree(t->stage_bgr[b])); t->stage_bgr[b] = nullptr; }
+    t->channels = channels;
+  }
+  return EA_OK;
+}
+
 int ea_tracker_set_inputs_ready(ea_tracker* t, int ready) {
   if (!t) return ea_fail(EA_ERR_INVALID_ARG, "null tracker");
   t->inputs_ready = ready ? 1 : 0;
@@ -231,11 +246,12 @@ int ea_tracker_step_host(ea_tracker* t, const uint8_t* bgr, const void* depth, d
   const int frame = t->frame, b = frame & 1;
   const bool becomes_key = (frame % t->interval) == 0;
   if (becomes_key && !depth) return ea_fail(EA_ERR_INVALID_ARG, "frame %d becomes a key frame and needs depth", frame);
-  if (!t->stage_bgr[b]) CU(cudaMalloc((void**)&t->stage_bgr[b], px * 3 * n));
+  const size_t frame_bytes = px * t->channels * n;
+  if (!t->stage_bgr[b]) CU(cudaMalloc((void**)&t->stage_bgr[b], frame_bytes));
   if (becomes_key && !t->stage_depth[b]) CU(cudaMalloc((void**)&t->stage_depth[b], px * fs->depth_elem * n));
   // upload on the copy stream once the kernels that read this staging buffer two frames ago are done
   if (frame >= 2) CU(cudaStreamWaitEvent(t->copy_stream, t->ev_consumed[b], 0));
-  CU(cudaMemcpyAsync(t->stage_bgr[b], bgr, px * 3 * n, cudaMemcpyHostToDevice, t->copy_stream));
+  CU(cudaMemcpyAsync(t->stage_bgr[b], bgr, frame_bytes, cudaMemcpyHostToDevice, t->copy_stream));
   if (becomes_key) CU(cudaMemcpyAsync(t->stage_depth[b], depth, px * fs->depth_elem * n, cudaMemcpyHostToDevice, t->copy_stream));
   CU(cudaEventRecord(t->ev_copied[b], t->copy_stream));
   int rc = tracker_step(t, t->stage_bgr[b], becomes_key ? t->stage_depth[b] : nullptr, t->ev_copied[b], t->ev_consumed[b]);

@@ -11,8 +11,9 @@
  *
  * Conventions
  *   - every function returns ea_status (0 == EA_OK); ea_last_error() gives the text
- *   - images: BGR u8 interleaved row-major (cv::imread order, standalone_edge_align.cpp:118),
- *     depth u16 row-major (raw units; metres = raw / depth_scale, utils.cpp:235)
+ *   - images: BGR u8 interleaved row-major (cv::imread order, standalone_edge_align.cpp:118), or 8-bit gray
+ *     row-major through the *_gray_* entry points / ea_tracker_set_image_format; depth u16 row-major (raw units;
+ *     metres = raw / depth_scale, utils.cpp:235)
  *   - pose: 7 doubles {qw,qx,qy,qz,tx,ty,tz} = b_T_a, Eigen/Ceres (w,x,y,z) order
  *     (standalone/PoseManipUtils.cpp:16-27)
  *   - there is NO CPU fallback: every compute entry point needs a CUDA device
@@ -199,6 +200,22 @@ int ea_frameset_preprocess_now_masked(ea_frameset* fs, int n, const int32_t* slo
 int ea_frameset_preprocess_device(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* d_bgr,
                                   const void* d_depth, int roles);
 
+/* 8-bit gray input (grayscale / IR cameras, the Y plane of YUV frames): a third of the bytes of BGR.  A gray frame g is
+ * preprocessed exactly as the BGR entry points preprocess (g, g, g) -- every level, every edge detector, DT kind, mask and
+ * depth type -- so points, distance transforms and solves are bit-identical: OpenCV's 8-bit RGB2GRAY weights sum to 2^15
+ * (9798 + 19235 + 3735) with half of that as rounding constant, so three equal channels convert back to the same value, the
+ * 2x2 pyramid mean is per channel, and CANNY_COLOR's channel of largest gradient is that value itself.
+ * HOST buffers: gray [n][h][w] u8; depth as ea_frameset_preprocess_host (may be NULL unless roles include EA_ROLE_REF);
+ * ref_mask [n][h][w] u8 or NULL: reference points only where ref_mask > 0 (get_aX_mask, needs EA_ROLE_REF); now_mask
+ * [n][h][w] u8 or NULL: now-frame edges only where now_mask > 1 (get_distance_transform2_masked, needs EA_ROLE_NOW).
+ * roles: EA_ROLE_REF, EA_ROLE_NOW or EA_ROLE_BOTH.  Asynchronous on the context stream. */
+typedef enum ea_image_format { EA_IMAGE_BGR8 = 0, EA_IMAGE_GRAY8 = 1 } ea_image_format;
+int ea_frameset_preprocess_gray_host(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* gray, const void* depth,
+                                     const uint8_t* ref_mask, const uint8_t* now_mask, int roles);
+/* same, inputs already resident in device memory (d_gray 4-byte aligned for the word-wide kernels; any address works) */
+int ea_frameset_preprocess_gray_device(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* d_gray,
+                                       const void* d_depth, int roles);
+
 /* Bypass hooks (parity on oracle-made inputs; CAD point sets as in edge_align_test5..8). */
 int ea_frameset_set_points(ea_frameset* fs, int slot, int level, const float* pts4, int n, int mode);
 int ea_frameset_set_dt(ea_frameset* fs, int slot, int level, const float* dt /* [h_l][w_l] */);
@@ -274,7 +291,7 @@ int ea_tracker_create(ea_context* ctx, const ea_frame_params* fp, const ea_solve
                       int keyframe_interval, ea_tracker** out);
 int ea_tracker_destroy(ea_tracker* tr);
 int ea_tracker_reset(ea_tracker* tr);
-/* HOST inputs [n_streams][h][w][3] / [n_streams][h][w]; poses7 out [n_streams][7] = keyframe_T_frame
+/* HOST inputs [n_streams][h][w][3] (or [n_streams][h][w], EA_IMAGE_GRAY8) / [n_streams][h][w]; poses7 out [n_streams][7] = keyframe_T_frame
  * (HOST, may be NULL => fetch later with ea_tracker_get_poses); asynchronous unless poses7 given. */
 int ea_tracker_step_host(ea_tracker* tr, const uint8_t* bgr, const void* depth, double* poses7,
                          ea_summary* summaries);
@@ -284,6 +301,11 @@ int ea_tracker_step_host(ea_tracker* tr, const uint8_t* bgr, const void* depth, 
  * frame must stay valid until its results have been waited for. */
 int ea_tracker_wait(ea_tracker* tr, int frame, double* poses7, ea_summary* summaries);
 int ea_tracker_step_device(ea_tracker* tr, const uint8_t* d_bgr, const void* d_depth);
+/* ea_image_format of the image argument of ea_tracker_step_host / _device: EA_IMAGE_BGR8 (default, [n_streams][h][w][3]) or
+ * EA_IMAGE_GRAY8 ([n_streams][h][w] u8; the host path then uploads w*h bytes per stream and frame instead of 3*w*h).  Results
+ * are those of BGR frames (g, g, g).  Only before the first step (after ea_tracker_create or ea_tracker_reset), else
+ * EA_ERR_STATE. */
+int ea_tracker_set_image_format(ea_tracker* tr, int image_format);
 /* By default the device buffers passed to ea_tracker_step_device are ordered by the context stream (work enqueued there
  * before the call produces them).  ready != 0 declares instead that they are COMPLETE in memory when the call is made; the
  * tracker then preprocesses frame t+1 on its own stream while frame t is still being aligned (its kernels take over the

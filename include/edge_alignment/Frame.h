@@ -44,16 +44,19 @@ class Frame {
   ea_frameset* handle() const { return fs_; }
   ea_context* context() const { return ctx_; }
 
-  // rgb: 8UC3 (BGR as cv::imread gives it); depth: 16UC1 raw units or 32FC1 metres (SolveEA.cpp:27,68), converted to the
-  // frameset's own depth_type when they differ; depth may be null for a now-only frame.  The "Z==0 -> 1.0" rule of
-  // SolveEA.cpp:69 is a frameset parameter (zero_depth_to_one) applied on the device.
+  // rgb: 8UC3 (BGR as cv::imread gives it) or 8UC1 (gray / IR; preprocessed exactly as the BGR image (g, g, g)); any other
+  // type throws.  depth: 16UC1 raw units or 32FC1 metres (SolveEA.cpp:27,68), converted to the frameset's own depth_type
+  // when they differ; depth may be null for a now-only frame.  The "Z==0 -> 1.0" rule of SolveEA.cpp:69 is a frameset
+  // parameter (zero_depth_to_one) applied on the device.
   template <class MatT>
   void set(const MatT& rgb, const MatT* depth, int roles) {
     if (!fs_) throw std::runtime_error("Frame::set before init");
     if (rgb.rows != params_.height || rgb.cols != params_.width) throw std::runtime_error("Frame::set: image size differs from ea_frame_params");
-    const size_t W = size_t(params_.width), H = size_t(params_.height);
-    bgr_.resize(W * H * 3);
-    for (size_t y = 0; y < H; ++y) std::copy(rgb.data + y * size_t(rgb.step), rgb.data + y * size_t(rgb.step) + W * 3, bgr_.begin() + y * W * 3);
+    const int type = rgb.type();
+    if (type != ea::U8C3 && type != ea::U8C1) throw std::runtime_error("Frame::set: the image must be 8UC3 (BGR) or 8UC1 (gray)");
+    const size_t W = size_t(params_.width), H = size_t(params_.height), C = (type == ea::U8C3) ? 3 : 1;
+    bgr_.resize(W * H * C);
+    for (size_t y = 0; y < H; ++y) std::copy(rgb.data + y * size_t(rgb.step), rgb.data + y * size_t(rgb.step) + W * C, bgr_.begin() + y * W * C);
     const void* dptr = nullptr;
     if (depth && depth->data) {
       const bool want_f32 = params_.depth_type == EA_DEPTH_F32, have_f32 = depth->type() == ea::F32C1;
@@ -75,7 +78,8 @@ class Frame {
       dptr = depth_.data();
     }
     const int32_t slot = 0;
-    ea::check(ea_frameset_preprocess_host(fs_, 1, &slot, bgr_.data(), dptr, roles), "ea_frameset_preprocess_host");
+    if (C == 3) ea::check(ea_frameset_preprocess_host(fs_, 1, &slot, bgr_.data(), dptr, roles), "ea_frameset_preprocess_host");
+    else ea::check(ea_frameset_preprocess_gray_host(fs_, 1, &slot, bgr_.data(), dptr, nullptr, nullptr, roles), "ea_frameset_preprocess_gray_host");
     ea::check(ea_sync(ctx_), "ea_sync");
   }
 
@@ -100,6 +104,6 @@ class Frame {
   ea_context* ctx_ = nullptr;
   ea_frameset* fs_ = nullptr;
   ea_frame_params params_{};
-  std::vector<uint8_t> bgr_;
+  std::vector<uint8_t> bgr_;            // the image as uploaded: BGR or gray rows without padding
   std::vector<unsigned char> depth_;
 };
