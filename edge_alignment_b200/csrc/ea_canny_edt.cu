@@ -66,15 +66,21 @@ __global__ void __launch_bounds__(256) k_canny_grad(const uint8_t* __restrict__ 
   }
 }
 
-// non-maximum suppression with the fixed-point tan(22.5 deg) test -> map: 1 = no edge, 0 = candidate, 2 = strong
-__global__ void __launch_bounds__(256) k_canny_nms(const int* __restrict__ mag, const short2* __restrict__ dxy, uint8_t* __restrict__ map,
+// non-maximum suppression with the fixed-point tan(22.5 deg) test -> map: 1 = no edge, 0 = candidate, 2 = strong.  Each candidate or
+// strong pixel also gets its union-find key for the hysteresis (hy_key) in lab, which is the dxy plane: the thread that reads pixel i's
+// gradient is the one that overwrites it, after the read (the stored value depends on it).
+__device__ __forceinline__ int hy_key(int i, bool strong, int n) { return strong ? i : n + i; }
+__device__ __forceinline__ int hy_node(int key, int n) { return key >= n ? key - n : key; }
+
+__global__ void __launch_bounds__(256) k_canny_nms(const int* __restrict__ mag, short2* dxy, uint8_t* __restrict__ map,
                                                    size_t scratch_stride_px, int w, int h, int low, int high) {
-  const int f = blockIdx.y;
+  const int f = blockIdx.y, n = w * h;
   const int* M = mag + size_t(f) * scratch_stride_px;
-  const short2* G = dxy + size_t(f) * scratch_stride_px;
+  short2* G = dxy + size_t(f) * scratch_stride_px;
+  int* lab = reinterpret_cast<int*>(G);
   uint8_t* P = map + size_t(f) * scratch_stride_px;
   auto at = [&](int x, int y) { return (x < 0 || x >= w || y < 0 || y >= h) ? 0 : M[size_t(y) * w + x]; };
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < w * h; i += gridDim.x * blockDim.x) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const int x = i % w, y = i / w;
     const int m = M[i];
     bool is_max = false;
@@ -90,52 +96,85 @@ __global__ void __launch_bounds__(256) k_canny_nms(const int* __restrict__ mag, 
       }
     }
     P[i] = is_max ? (m > high ? 2 : 0) : 1;
+    if (is_max) lab[i] = hy_key(i, m > high, n);
   }
 }
 
-// hysteresis: one CTA per frame promotes candidates that touch a strong pixel until nothing changes (the fixed point
-// is the 8-connected closure of the strong pixels, independent of visiting order), then packs the bit planes.
-template <typename D>
-__global__ void __launch_bounds__(1024) k_canny_hysteresis(uint8_t* __restrict__ map, size_t scratch_stride_px, const D* __restrict__ depth,
-                                                           size_t depth_stride_px, const int32_t* __restrict__ depth_slots, bool depth_slot_indexed,
-                                                           const int32_t* __restrict__ dst_slots, uint32_t* __restrict__ edge_bits,
-                                                           uint32_t* __restrict__ ref_bits, int w, int h, int words, int zero_to_one) {
-  const int f = blockIdx.x;
-  uint8_t* P = map + size_t(f) * scratch_stride_px;
-  const int n = w * h, per = (n + blockDim.x - 1) / blockDim.x;
-  const int b = threadIdx.x * per, e = min(b + per, n);
-  for (int it = 0; it < 4096; ++it) {
-    int changed = 0;
-    const bool fwd = (it & 1) == 0;
-    for (int k = 0; k < e - b; ++k) {
-      const int i = fwd ? b + k : e - 1 - k;
-      if (P[i] != 0) continue;
-      const int x = i % w, y = i / w;
-      bool hit = false;
-      for (int dy = -1; dy <= 1 && !hit; ++dy) {
-        const int yy = y + dy;
-        if (yy < 0 || yy >= h) continue;
-        for (int dx = -1; dx <= 1; ++dx) {
-          const int xx = x + dx;
-          if (xx >= 0 && xx < w && P[size_t(yy) * w + xx] == 2) { hit = true; break; }
-        }
-      }
-      if (hit) { P[i] = 2; changed = 1; }
-    }
-    if (!__syncthreads_or(changed)) break;
+// ---- hysteresis: the edges are the candidate and strong pixels 8-connected to a strong one.  Union-find over those pixels: a node's
+// entry in lab is the key of its parent, a root's is its own key.  Keys order strong pixels before candidates (hy_key), and a union
+// always hangs the root with the larger key under the other, so a tree's root has its smallest key: the component holds a strong
+// pixel iff its root key is < n.  Every entry only ever decreases (atomicMin) to the key of an ancestor, so concurrent unions and
+// path halving keep every tree a tree of its component (the lock-free union of Playne & Hawick, 2018).  Work per pixel does not
+// depend on how far along a chain the nearest strong pixel is.
+__device__ __forceinline__ int hy_find(int* lab, int i, int n) {
+  int k = __ldcg(lab + i);
+  while (hy_node(k, n) != i) {
+    const int p = hy_node(k, n), kp = __ldcg(lab + p);
+    if (hy_node(kp, n) == p) return kp;
+    atomicMin(lab + i, kp);                                     // path halving: i skips its parent
+    i = hy_node(kp, n);
+    k = __ldcg(lab + i);
   }
-  __syncthreads();
+  return k;
+}
+__device__ __forceinline__ void hy_unite(int* lab, int a, int b, int n) {
+  int ka = hy_find(lab, a, n), kb = hy_find(lab, b, n);
+  while (ka != kb) {
+    if (ka > kb) { const int t = ka; ka = kb; kb = t; }
+    const int old = atomicMin(lab + hy_node(kb, n), ka);
+    if (old == kb) return;                                      // kb was still a root: now under ka
+    kb = hy_find(lab, hy_node(old, n), n);                      // kb was linked meanwhile: unite with its new root
+  }
+}
+
+__global__ void __launch_bounds__(256) k_canny_union(const uint8_t* __restrict__ map, short2* dxy, size_t scratch_stride_px, int w, int h) {
+  const int f = blockIdx.y, n = w * h;
+  const uint8_t* P = map + size_t(f) * scratch_stride_px;
+  int* lab = reinterpret_cast<int*>(dxy + size_t(f) * scratch_stride_px);
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    if (P[i] == 1) continue;
+    const int x = i % w, y = i / w;
+    // the neighbours before i in raster order (left, up-left, up, up-right); a pair of them that touch each other is united
+    // by its own later pixel, so up alone, or left / up-left plus up-right, suffice
+    const bool l = x > 0 && P[i - 1] != 1, ul = x > 0 && y > 0 && P[i - w - 1] != 1, u = y > 0 && P[i - w] != 1,
+               ur = x + 1 < w && y > 0 && P[i - w + 1] != 1;
+    if (u) { hy_unite(lab, i, i - w, n); continue; }
+    if (l) hy_unite(lab, i, i - 1, n);
+    else if (ul) hy_unite(lab, i, i - w - 1, n);
+    if (ur) hy_unite(lab, i, i - w + 1, n);
+  }
+}
+
+// edge = candidate or strong pixel whose root key is a strong pixel's; packs the edge plane and the reference plane (edge with depth,
+// or every edge with zero_to_one), one warp per 32-pixel word
+template <typename D>
+__global__ void __launch_bounds__(256) k_canny_pack(const uint8_t* __restrict__ map, const short2* dxy, size_t scratch_stride_px,
+                                                    const D* __restrict__ depth, size_t depth_stride_px, const int32_t* __restrict__ depth_slots,
+                                                    bool depth_slot_indexed, const int32_t* __restrict__ dst_slots, uint32_t* __restrict__ edge_bits,
+                                                    uint32_t* __restrict__ ref_bits, int w, int h, int words, int zero_to_one) {
+  const int f = blockIdx.y, n = w * h;
+  const uint8_t* P = map + size_t(f) * scratch_stride_px;
+  const int* lab = reinterpret_cast<const int*>(dxy + size_t(f) * scratch_stride_px);
   const D* dep = depth ? depth + ((depth_slot_indexed && depth_slots) ? size_t(depth_slots[f]) : size_t(f)) * depth_stride_px : nullptr;
   const size_t obase = size_t(dst_slots[f]) * h * words;
-  for (int wi = threadIdx.x; wi < h * words; wi += blockDim.x) {
-    const int y = wi / words, x0 = (wi % words) * 32;
-    unsigned eb = 0, rb = 0;
-    for (int k = 0; k < 32 && x0 + k < w; ++k) {
-      const size_t i = size_t(y) * w + x0 + k;
-      if (P[i] == 2) { eb |= 1u << k; if (dep && (zero_to_one || dep[i] > D(0))) rb |= 1u << k; }
+  const int total = h * words * 32;                           // a multiple of 32: every warp's pixels fall in one word
+  for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < total; t += gridDim.x * blockDim.x) {
+    const int y = t / (words * 32), x = t % (words * 32);
+    bool edge = false, ref = false;
+    if (x < w) {
+      const int i = y * w + x;
+      if (P[i] != 1) {
+        int j = i, k = lab[i];
+        while (hy_node(k, n) != j) { j = hy_node(k, n); k = lab[j]; }
+        edge = k < n;
+        ref = edge && dep && (zero_to_one || dep[i] > D(0));
+      }
     }
-    edge_bits[obase + wi] = eb;
-    if (ref_bits) ref_bits[obase + wi] = rb;
+    const unsigned eb = __ballot_sync(0xffffffffu, edge), rb = __ballot_sync(0xffffffffu, ref);
+    if ((threadIdx.x & 31) == 0) {
+      edge_bits[obase + (t >> 5)] = eb;
+      if (ref_bits) ref_bits[obase + (t >> 5)] = rb;
+    }
   }
 }
 
@@ -218,6 +257,7 @@ cudaError_t ea_launch_canny_level(const EaPrepArgs& A, int l, const uint8_t* bgr
                                   bool slot_indexed, const EaCannyCfg& cfg, const EaScratch& S, cudaStream_t stream, int* launches) {
   const EaPrepLevel& L = A.lv[l];
   const int npx = L.w * L.h;
+  if (npx > (1 << 30)) return cudaErrorInvalidValue;              // the hysteresis' union-find keys go up to 2 w h
   dim3 grid(unsigned(std::min((npx + 255) / 256, 4096)), unsigned(A.n));
   double t1 = cfg.low, t2 = cfg.high;
   if (t1 > t2) { const double t = t1; t1 = t2; t2 = t; }
@@ -239,14 +279,18 @@ cudaError_t ea_launch_canny_level(const EaPrepArgs& A, int l, const uint8_t* bgr
     *launches += 2;
   }
   k_canny_nms<<<grid, 256, 0, stream>>>(S.mag, S.dxy, S.map, S.stride, L.w, L.h, low, high);
+  k_canny_union<<<grid, 256, 0, stream>>>(S.map, S.dxy, S.stride, L.w, L.h);
+  const int npack = L.h * L.words * 32;
+  const dim3 pgrid(unsigned(std::min((npack + 255) / 256, 4096)), unsigned(A.n));
   const bool want_ref = (A.roles & EA_ROLE_REF) != 0;
   if (A.depth_type == 1)
-    k_canny_hysteresis<float><<<A.n, 1024, 0, stream>>>(S.map, S.stride, want_ref ? static_cast<const float*>(depth) : nullptr, frame_stride_px, A.slots, slot_indexed, A.slots,
-                                                        L.edge_bits, want_ref ? L.ref_bits : nullptr, L.w, L.h, L.words, A.zero_to_one);
+    k_canny_pack<float><<<pgrid, 256, 0, stream>>>(S.map, S.dxy, S.stride, want_ref ? static_cast<const float*>(depth) : nullptr, frame_stride_px, A.slots,
+                                                   slot_indexed, A.slots, L.edge_bits, want_ref ? L.ref_bits : nullptr, L.w, L.h, L.words, A.zero_to_one);
   else
-    k_canny_hysteresis<uint16_t><<<A.n, 1024, 0, stream>>>(S.map, S.stride, want_ref ? static_cast<const uint16_t*>(depth) : nullptr, frame_stride_px, A.slots, slot_indexed, A.slots,
-                                                           L.edge_bits, want_ref ? L.ref_bits : nullptr, L.w, L.h, L.words, A.zero_to_one);
-  *launches += 2;
+    k_canny_pack<uint16_t><<<pgrid, 256, 0, stream>>>(S.map, S.dxy, S.stride, want_ref ? static_cast<const uint16_t*>(depth) : nullptr, frame_stride_px,
+                                                      A.slots, slot_indexed, A.slots, L.edge_bits, want_ref ? L.ref_bits : nullptr, L.w, L.h, L.words,
+                                                      A.zero_to_one);
+  *launches += 3;
   return cudaGetLastError();
 }
 

@@ -62,7 +62,7 @@ struct EaPrepLevel {            // device pointers of one pyramid level, slot-ma
   int w, h, words, cap;
 };
 struct EaCannyCfg { double low, high; int l2, on_color; };
-struct EaScratch {              // Canny / exact-EDT work buffers, [n_slots][stride] each (stride = level-0 pixels)
+struct EaScratch {              // Canny / exact-EDT work buffers, [n_slots][stride] each (stride = level-0 pixels); after NMS, dxy holds the hysteresis' union-find keys
   uint8_t* gray; int* mag; short2* dxy; uint8_t* map; size_t stride;
 };
 struct EaPrepArgs {
