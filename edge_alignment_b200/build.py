@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libea_b200.so")
-SOURCES = ["ea_cabi.cu", "ea_solve.cu", "ea_preprocess.cu", "ea_canny_edt.cu", "ea_tracker.cu", "ea_shard.cu", "ea_views_batch.cu"]
+SOURCES = ["ea_cabi.cu", "ea_solve.cu", "ea_preprocess.cu", "ea_canny_edt.cu", "ea_tracker.cu", "ea_shard.cu", "ea_views.cu", "ea_views_batch.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-Wall,-Wno-unused-function", "--expt-relaxed-constexpr",
               "-I", os.path.join(ROOT, "include"), "-I", CSRC]

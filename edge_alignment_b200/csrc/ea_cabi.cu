@@ -32,6 +32,23 @@ int ea_ensure_tmp(ea_context* c, size_t bytes) {
   c->tmp_cap = bytes;
   return EA_OK;
 }
+
+int ea_ensure_views(ea_context* c, size_t bytes) {
+  if (c->views_cap >= bytes) return EA_OK;
+  CU(cudaStreamSynchronize(c->stream));
+  if (c->d_views) { cudaFree(c->d_views); c->d_views = nullptr; c->views_cap = 0; }
+  CU(cudaMalloc(&c->d_views, bytes));
+  c->views_cap = bytes;
+  return EA_OK;
+}
+
+void ea_fold_sums28(const double* partials, int n_blocks, double* sums28) {
+  double t[EA_SUMS] = {0};
+  for (int b = 0; b < n_blocks; ++b) for (int k = 0; k < EA_SUMS; ++k) t[k] += partials[size_t(b) * EA_SUMS + k];
+  sums28[0] = t[28];                                   // cost
+  for (int k = 0; k < 6; ++k) sums28[1 + k] = t[21 + k];  // J^T r
+  for (int k = 0; k < 21; ++k) sums28[7 + k] = t[k];      // upper-tri J^T J
+}
 extern "C" {
 
 int ea_abi_version(void) { return EA_ABI_VERSION; }
@@ -661,11 +678,7 @@ int ea_eval(ea_context* c, ea_frameset* ref, int ref_slot, ea_frameset* now, int
       std::vector<double> h(size_t(nb) * EA_SUMS);
       CU(cudaMemcpyAsync(h.data(), c->d_sums, h.size() * 8, cudaMemcpyDeviceToHost, c->stream));
       CU(cudaStreamSynchronize(c->stream));
-      double t[EA_SUMS] = {0};
-      for (int b = 0; b < nb; ++b) for (int k = 0; k < EA_SUMS; ++k) t[k] += h[size_t(b) * EA_SUMS + k];
-      sums28[0] = t[28];                                   // cost
-      for (int k = 0; k < 6; ++k) sums28[1 + k] = t[21 + k];  // J^T r
-      for (int k = 0; k < 21; ++k) sums28[7 + k] = t[k];      // upper-tri J^T J
+      ea_fold_sums28(h.data(), nb, sums28);
     }
   }
   CU(cudaStreamSynchronize(c->stream));

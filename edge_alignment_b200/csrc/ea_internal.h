@@ -125,7 +125,7 @@ struct ea_context {
   size_t idx_cap = 0;
   void* d_tmp = nullptr;
   size_t tmp_cap = 0;
-  void* d_views = nullptr; size_t views_cap = 0;   // ea_solve_views: view descriptors, control block and CTA totals of the persistent kernel
+  void* d_views = nullptr; size_t views_cap = 0;   // ea_solve_views / ea_solve_views_batch: view descriptors and the persistent kernel's scratch
   EaPrepPipe prep_pipe;           // auxiliary streams of the preprocessing pipeline (created on first use)
   // optional profiling: event pairs around preprocessing pipelines [0] and solve launches [1]
   bool profile = false;
@@ -192,6 +192,9 @@ struct EaEventPair {
   EaEventPair() = default; EaEventPair(const EaEventPair&) = delete; EaEventPair& operator=(const EaEventPair&) = delete;
 };
 int ea_ensure_tmp(ea_context* c, size_t bytes);
+int ea_ensure_views(ea_context* c, size_t bytes);   // grows c->d_views (after the stream's work on it has finished)
+// The C ABI's sums28 ({cost, J^T r [6], upper-tri J^T J [21]}) from n_blocks rows of EA_SUMS partial sums, added in row order.
+void ea_fold_sums28(const double* partials, int n_blocks, double* sums28);
 // A view's rig transform and distortion in the form the general per-point evaluation takes (identity / zero when unused).
 inline void ea_view_xf(const ea_view& v, EaViewXf& X) {
   memset(&X, 0, sizeof X);

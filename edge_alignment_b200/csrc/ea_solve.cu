@@ -112,7 +112,7 @@ __device__ __forceinline__ void ea_boss_next_impl(const EaSolveArgs& A, EaSolveS
       continue;
     }
     EaLmState& L = S.lm;
-    L.phase = 0; L.iter = 0; L.accepted = 0; L.rejected = 0; L.invalid_run = 0; L.evals = 0; L.term = EA_TERM_NONE;
+    ea_lm_restart(L);
 #pragma unroll 1
     for (int i = 0; i < 7; ++i) L.cand[i] = L.x[i];
     if (rd.pts_mode == EA_POINTS_XYZ) ea_pose_setup<true>(L.cand, A.ref_geom[level], A.now_geom[level], out.P);
@@ -160,28 +160,11 @@ __device__ __forceinline__ void ea_boss_step_warp(const EaSolveArgs& A, EaSolveS
     return;
   }
   if (lane == 0) {
-    if (A.summaries) {
-      const EaLmState& L = S.lm;
-      ea_summary z;
-      z.termination = L.term; z.iterations = L.iter; z.accepted = L.accepted; z.rejected = L.rejected;
-      z.n_residuals = cur.n_res; z.evaluations = L.evals; z.initial_cost = L.initial_cost; z.final_cost = L.cost;
-      z.truncated = S.truncated; z.reserved = 0;
-      A.summaries[size_t(S.pair) * A.n_levels + cur.level] = z;
-    }
+    if (A.summaries) A.summaries[size_t(S.pair) * A.n_levels + cur.level] = ea_lm_summary(S.lm, cur.n_res, S.truncated);
     S.level = cur.level - 1;
     ea_boss_next(A, S, out, false);
   }
   __syncwarp();
-}
-
-
-__device__ __forceinline__ unsigned long long ea_ld_acquire(const unsigned long long* p) {
-  unsigned long long v;
-  asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void ea_st_release(unsigned long long* p, unsigned long long v) {
-  asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
 }
 
 // One worker's share of an evaluation: chunks [cb, ce) of M, walked in M's direction; per-chunk partials into S.part / S.cpart.
@@ -616,18 +599,7 @@ __global__ void __launch_bounds__(1024) ea_k_order_by_work(const ea_summary* __r
     key[i] = k;
   }
   __syncthreads();
-  for (int size = 2; size <= m; size <<= 1)
-    for (int stride = size >> 1; stride > 0; stride >>= 1) {
-      for (int i = threadIdx.x; i < m; i += blockDim.x) {
-        const int j = i ^ stride;
-        if (j > i) {
-          const bool desc = (i & size) == 0;
-          const unsigned long long a = key[i], b = key[j];
-          if (desc ? (a < b) : (a > b)) { key[i] = b; key[j] = a; }
-        }
-      }
-      __syncthreads();
-    }
+  ea_cta_sort_desc(key, m);
   for (int i = threadIdx.x; i < n; i += blockDim.x) order[i] = int32_t(0xFFFFF - int(key[i] & 0xFFFFF));
 }
 

@@ -708,3 +708,151 @@ __device__ __forceinline__ double ea_cta_total(const double (*part)[EA_NSUM], co
   return s;
 }
 
+// =====================================================================================================================
+// Pieces shared by the schedulers around the LM step (ea_solve.cu, ea_shard.cu, ea_views.cu, ea_views_batch.cu).
+
+// Start of a (pair, level): the state machine back to its first evaluation.  The caller sets cand (and x).
+__device__ __forceinline__ void ea_lm_restart(EaLmState& L) {
+  L.phase = 0; L.iter = 0; L.accepted = 0; L.rejected = 0; L.invalid_run = 0; L.evals = 0; L.term = EA_TERM_NONE;
+}
+
+// (The counts are taken by reference so that they are read after the state's fields, as the solve kernels always read them:
+// taken by value, they move ea_k_solve_batch's register allocation.)
+__host__ __device__ __forceinline__ ea_summary ea_lm_summary(const EaLmState& L, const int& n_residuals, const int& truncated) {
+  ea_summary z;
+  z.termination = L.term; z.iterations = L.iter; z.accepted = L.accepted; z.rejected = L.rejected;
+  z.n_residuals = n_residuals; z.evaluations = L.evals; z.initial_cost = L.initial_cost; z.final_cost = L.cost;
+  z.truncated = truncated; z.reserved = 0;
+  return z;
+}
+
+__device__ __forceinline__ unsigned long long ea_ld_acquire(const unsigned long long* p) {
+  unsigned long long v;
+  asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void ea_st_release(unsigned long long* p, unsigned long long v) {
+  asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+
+// A warp copies an LM state between global and shared memory, 8-byte words; global memory is read from L2 and written past
+// L1 (the state may have been written by another CTA of the grid, and may be read by one).
+static_assert(sizeof(EaLmState) % 8 == 0, "EaLmState is copied as 8-byte words");
+__device__ __forceinline__ void ea_lm_load_warp(EaLmState& dst, const EaLmState& src /*global*/, const int lane) {
+  const unsigned long long* s = reinterpret_cast<const unsigned long long*>(&src);
+  unsigned long long* d = reinterpret_cast<unsigned long long*>(&dst);
+  for (int i = lane; i < int(sizeof(EaLmState) / 8); i += 32) d[i] = __ldcg(s + i);
+}
+__device__ __forceinline__ void ea_lm_store_warp(EaLmState& dst /*global*/, const EaLmState& src, const int lane) {
+  const unsigned long long* s = reinterpret_cast<const unsigned long long*>(&src);
+  unsigned long long* d = reinterpret_cast<unsigned long long*>(&dst);
+  for (int i = lane; i < int(sizeof(EaLmState) / 8); i += 32) __stcg(d + i, s[i]);
+}
+
+// ---- persistent cooperative solve of one (pair, level) by a whole grid (k_shard_solve, k_views_solve) ----------------
+// Evaluation e runs when `go` reaches e; every CTA stores its totals and takes a ticket; one CTA adds the totals in a fixed
+// order (ea_grid_total), advances the LM state, sets `done` and releases e + 1.  Every wait is bounded (EA_GRID_SPIN_LIMIT
+// polls): a lost CTA or peer rank ends the solve with an error instead of hanging the GPU.
+#define EA_GRID_SPIN_LIMIT (1ll << 22)   // ~3 s of polling
+struct EaGridCtl {                                  // device memory
+  EaLmState lm;
+  EaPose P;                                         // candidate pose folded with the intrinsics, for the evaluation in flight
+  unsigned long long go;                            // evaluation epoch released to the grid
+  unsigned long long ticket;                        // CTAs that have delivered their totals (monotonic over the solve)
+  int done, error;
+  long long prof[6];                                // cycles: {evaluation (CTA 0), grid reduce, all-reduce, LM} of the CTA that did them, evaluations
+};
+
+// First evaluation's control block: LM state at the initial pose, its folded pose, evaluation 1 released (ea_shard.cu).
+__global__ void k_shard_ctl_init(EaGridCtl* ctl, const double* pose7, EaLevelGeom rg, EaLevelGeom ng, int xyz);
+
+// Thread 0 waits for the release of evaluation e; every thread returns 0 (evaluate), 1 (the solve is done) or 2 (the release
+// never came).  s_stop: shared.
+__device__ __forceinline__ int ea_grid_wait(EaGridCtl* ctl, const unsigned long long e, int& s_stop) {
+  if (threadIdx.x == 0) {
+    long long spins = 0;
+    int stop = 0;
+    while (ea_ld_acquire(&ctl->go) < e) {
+      if (++spins > EA_GRID_SPIN_LIMIT) { stop = 2; break; }
+      __nanosleep(20);
+    }
+    if (!stop) stop = *reinterpret_cast<volatile int*>(&ctl->done);
+    s_stop = stop;
+  }
+  __syncthreads();
+  return s_stop;
+}
+
+// Grid reduce by one CTA of the per-CTA totals partials[grid][32], fixed order: warp w adds CTAs w, w + W, ...; then the warps
+// in order.  Every thread calls it; lane k of warp 0 returns slot k.  wsum: shared scratch.
+template <int WARPS>
+__device__ __forceinline__ double ea_grid_total(const double* partials, double (*wsum)[32], const int warp, const int lane) {
+  double s = 0.0;
+  for (unsigned b = warp; b < gridDim.x; b += WARPS) s += __ldcg(&partials[size_t(b) * 32 + lane]);
+  wsum[warp][lane] = s;
+  __syncthreads();
+  double tot = 0.0;
+  if (warp == 0) {
+#pragma unroll
+    for (int w2 = 0; w2 < WARPS; ++w2) tot += wsum[w2][lane];
+  }
+  return tot;
+}
+
+// One view of a multi-camera problem (ea_views.cu, ea_views_batch.cu).
+// Residuals [j0, j1) of one view at the folded pose P, in tiles of THREADS x ITERS: residual tile + it * THREADS + tid belongs
+// to this thread.  At every tile end the lanes' fp32 slots are folded into the fp64 per-lane slot (acc64: warp slot `lane`) and
+// the thread's fp32 cost into cost64.  ITERS, the flush cadence, decides the rounding of the sums: each caller keeps its own.
+template <int ITERS, int THREADS>
+__device__ __forceinline__ void ea_eval_view(const bool xyz, const void* const& pts, const float* const& dt, const float2& affine,
+                                             const EaLevelGeom& ng, const double& inv_depth_scale, const EaPoseG& P, const ea_solve_params& sp, const int j0,
+                                             const int j1, const int tid, const int lane, double& acc64, double& cost64) {
+  const int stride = sp.point_stride, loss_type = sp.loss_type;
+  const float loss_a = float(sp.loss_scale);
+  float acc[EA_NSUM];
+#pragma unroll
+  for (int k = 0; k < EA_NSUM; ++k) acc[k] = 0.0f;
+  for (int tile = j0; tile < j1; tile += THREADS * ITERS) {
+    float cost = 0.0f;
+    const int it_end = min(ITERS, (j1 - tile + THREADS - 1) / THREADS);     // iterations with at least one residual (uniform)
+    for (int it = 0; it < it_end; ++it) {
+      const int j = tile + it * THREADS + tid;
+      if (j < j1) {
+        float f, w, rho0, J[6];
+        bool fail;
+        if (xyz) {
+          const float4 p = EaPtStream<true>::as_float4(EaPtStream<true>::load(pts, size_t(j) * stride));
+          fail = ea_point_eval_general<true>(p, ng, inv_depth_scale, P, dt, affine, loss_type, loss_a, f, w, rho0, J);
+        } else {
+          const float4 p = EaPtStream<false>::as_float4(EaPtStream<false>::load(pts, size_t(j) * stride));
+          fail = ea_point_eval_general<false>(p, ng, inv_depth_scale, P, dt, affine, loss_type, loss_a, f, w, rho0, J);
+        }
+        ea_accumulate(acc, J, f * w);
+        acc[27] += fail ? 1.0f : 0.0f;
+        cost = fmaf(0.5f, rho0, cost);
+      }
+    }
+    acc64 += double(ea_warp_transpose_reduce(acc, lane));
+#pragma unroll
+    for (int k = 0; k < EA_NSUM; ++k) acc[k] = 0.0f;
+    cost64 += double(cost);
+  }
+}
+
+// Bitonic sort of key[0, m) into descending order by every thread of the CTA (m a power of two, the keys stored and visible
+// to the CTA); ends with __syncthreads().
+__device__ __forceinline__ void ea_cta_sort_desc(unsigned long long* key, const int m) {
+  for (int size = 2; size <= m; size <<= 1)
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int i = threadIdx.x; i < m; i += blockDim.x) {
+        const int j = i ^ stride;
+        if (j > i) {
+          const bool desc = (i & size) == 0;
+          const unsigned long long a = key[i], b = key[j];
+          if (desc ? (a < b) : (a > b)) { key[i] = b; key[j] = a; }
+        }
+      }
+      __syncthreads();
+    }
+}
+

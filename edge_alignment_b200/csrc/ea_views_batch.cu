@@ -10,8 +10,8 @@
 //   queue     one persistent CTA per problem: a CTA takes the next problem from an atomic ticket and runs its whole pyramid
 //   boss      warp 0 runs the warp-cooperative LM step (ea_lm_advance_warp) on the state in shared memory, folds the candidate
 //             pose once per view (ea_pose_setup_general, one lane per view) and handles the level / problem transitions
-//   evaluate  all warps walk the problem's views in order; a view's residuals are cut into tiles of THREADS x 16: per lane 16
-//             points in fp32, the transposing warp butterfly, fp64 per-warp slots, CTA totals in fixed warp order
+//   evaluate  all warps walk the problem's views in order (ea_eval_view); a view's residuals are cut into tiles of THREADS x 16:
+//             per lane 16 points in fp32, the transposing warp butterfly, fp64 per-warp slots, CTA totals in fixed warp order
 //
 // The sums of a problem depend only on its views and VB_THREADS: not on the CTA that ran it, the batch or the order.
 #include <algorithm>
@@ -131,46 +131,13 @@ __device__ __noinline__ void vb_boss_next(const VbArgs& A, VbSmem& S, const int 
       continue;
     }
     if (lane == 0) {
-      EaLmState& L = S.lm;
-      L.phase = 0; L.iter = 0; L.accepted = 0; L.rejected = 0; L.invalid_run = 0; L.evals = 0; L.term = EA_TERM_NONE;
+      ea_lm_restart(S.lm);
       S.n_res = total; S.truncated = trunc; S.cmd = EA_CMD_EVAL;
     }
     if (lane < 7) S.lm.cand[lane] = S.lm.x[lane];
     __syncwarp();
     vb_fold(S, lane);
     return;
-  }
-}
-
-// One view's residuals [0, n) in tiles of THREADS x VB_TILE_ITERS.  Residual tile + it * THREADS + tid belongs to this thread;
-// its lanes' fp32 slots are folded into the fp64 per-lane slot (acc64: warp slot `lane`) and cost (cost64) at every tile end.
-template <bool XYZ, int THREADS>
-__device__ __forceinline__ void vb_eval_view(const VbLive& Lv, const EaPoseG& P, const ea_solve_params& sp, const int tid, const int lane,
-                                             double& acc64, double& cost64) {
-  const int n = Lv.n_res, stride = sp.point_stride, loss_type = sp.loss_type;
-  const float loss_a = float(sp.loss_scale);
-  const float2 affine = Lv.affine;
-  float acc[EA_NSUM];
-#pragma unroll
-  for (int k = 0; k < EA_NSUM; ++k) acc[k] = 0.0f;
-  for (int tile = 0; tile < n; tile += THREADS * VB_TILE_ITERS) {
-    float cost = 0.0f;
-    const int it_end = min(VB_TILE_ITERS, (n - tile + THREADS - 1) / THREADS);     // iterations with at least one residual (uniform)
-    for (int it = 0; it < it_end; ++it) {
-      const int j = tile + it * THREADS + tid;
-      if (j < n) {
-        const float4 p = EaPtStream<XYZ>::as_float4(EaPtStream<XYZ>::load(Lv.pts, size_t(j) * stride));
-        float f, w, rho0, J[6];
-        const bool fail = ea_point_eval_general<XYZ>(p, Lv.ng, Lv.inv_depth_scale, P, Lv.dt, affine, loss_type, loss_a, f, w, rho0, J);
-        ea_accumulate(acc, J, f * w);
-        acc[27] += fail ? 1.0f : 0.0f;
-        cost = fmaf(0.5f, rho0, cost);
-      }
-    }
-    acc64 += double(ea_warp_transpose_reduce(acc, lane));
-#pragma unroll
-    for (int k = 0; k < EA_NSUM; ++k) acc[k] = 0.0f;
-    cost64 += double(cost);
   }
 }
 
@@ -189,9 +156,10 @@ __global__ void __launch_bounds__(THREADS, VB_MIN_CTAS) k_views_batch(const __gr
     double acc64 = 0.0, cost64 = 0.0;
     const int nv = S.nv;
     for (int v = 0; v < nv; ++v) {
-      if (S.live[v].n_res == 0) continue;
-      if (S.live[v].xyz) vb_eval_view<true, THREADS>(S.live[v], S.P[v], A.sp, tid, lane, acc64, cost64);
-      else vb_eval_view<false, THREADS>(S.live[v], S.P[v], A.sp, tid, lane, acc64, cost64);
+      const VbLive& Lv = S.live[v];
+      if (Lv.n_res == 0) continue;
+      if (Lv.xyz) ea_eval_view<VB_TILE_ITERS, THREADS>(true, Lv.pts, Lv.dt, Lv.affine, Lv.ng, Lv.inv_depth_scale, S.P[v], A.sp, 0, Lv.n_res, tid, lane, acc64, cost64);
+      else ea_eval_view<VB_TILE_ITERS, THREADS>(false, Lv.pts, Lv.dt, Lv.affine, Lv.ng, Lv.inv_depth_scale, S.P[v], A.sp, 0, Lv.n_res, tid, lane, acc64, cost64);
     }
     cost64 = ea_warp_sum(cost64);
     S.part[warp][lane] = acc64;
@@ -208,12 +176,7 @@ __global__ void __launch_bounds__(THREADS, VB_MIN_CTAS) k_views_batch(const __gr
         vb_fold(S, lane);
       } else {
         if (lane == 0) {
-          const EaLmState& L = S.lm;
-          ea_summary z;
-          z.termination = L.term; z.iterations = L.iter; z.accepted = L.accepted; z.rejected = L.rejected;
-          z.n_residuals = S.n_res; z.evaluations = L.evals; z.initial_cost = L.initial_cost; z.final_cost = L.cost;
-          z.truncated = S.truncated; z.reserved = 0;
-          A.summaries[size_t(S.problem) * A.n_levels + level] = z;
+          A.summaries[size_t(S.problem) * A.n_levels + level] = ea_lm_summary(S.lm, S.n_res, S.truncated);
           S.level = level - 1;
         }
         __syncwarp();
@@ -246,18 +209,7 @@ __global__ void __launch_bounds__(1024) k_vb_order(const VbView* __restrict__ vi
     key[i] = k;
   }
   __syncthreads();
-  for (int size = 2; size <= m; size <<= 1)
-    for (int str = size >> 1; str > 0; str >>= 1) {
-      for (int i = threadIdx.x; i < m; i += blockDim.x) {
-        const int j = i ^ str;
-        if (j > i) {
-          const bool desc = (i & size) == 0;
-          const unsigned long long a = key[i], b = key[j];
-          if (desc ? (a < b) : (a > b)) { key[i] = b; key[j] = a; }
-        }
-      }
-      __syncthreads();
-    }
+  ea_cta_sort_desc(key, m);
   for (int i = threadIdx.x; i < n; i += blockDim.x) order[i] = int32_t(0xFFFFFFFFu - unsigned(key[i] & 0xFFFFFFFFull));
 }
 
@@ -316,12 +268,8 @@ extern "C" int ea_solve_views_batch(ea_context* c, int n, const int32_t* view_of
   const size_t off_work = off_sum + vb_align(size_t(n) * L * sizeof(ea_summary));
   const size_t off_keys = off_work + 256;
   const size_t need = off_keys + (m > VB_SORT_SMEM ? size_t(m) * sizeof(unsigned long long) : 0);
-  if (c->views_cap < need) {
-    CU(cudaStreamSynchronize(st));
-    if (c->d_views) { cudaFree(c->d_views); c->d_views = nullptr; c->views_cap = 0; }
-    CU(cudaMalloc(&c->d_views, need));
-    c->views_cap = need;
-  }
+  rc = ea_ensure_views(c, need);
+  if (rc) return rc;
   char* base = static_cast<char*>(c->d_views);
   VbArgs A;
   std::memset(&A, 0, sizeof A);

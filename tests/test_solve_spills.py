@@ -3,7 +3,7 @@
 The warp-cooperative LM step (ea_lm_advance_warp) runs in the 128-register budget of the solve kernels while the other 15
 warps of the CTA wait at a barrier. Spilled to local memory, its loads miss the L1 that the evaluation sweep has just
 filled with distance transform, and the step becomes several times slower than its fp64 dependency chains. This test compiles
-the two translation units that contain it with the project's flags plus `-Xptxas -v` and checks ptxas' spill report. The
+the translation units that contain it with the project's flags plus `-Xptxas -v` and checks ptxas' spill report. The
 serial state machine (ea_lm_advance, ea_lm_propose_slow) only runs on rare paths and may spill.
 
 The limits are ptxas' figures for CUDA 12.9. The fast track's spill loads in ea_solve.cu are its pointer arguments, which
@@ -30,6 +30,11 @@ LIMITS = {
     "ea_shard.cu": {
         "ea_lm_advance_warp": (0, 0),
         "k_shard_solveILi512E": (52, 148),
+    },
+    "ea_views.cu": {
+        "ea_lm_advance_warp": (0, 0),
+        "k_views_solve": (0, 0),
+        "k_view_eval_sums": (0, 0),
     },
 }
 
