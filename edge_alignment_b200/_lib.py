@@ -22,6 +22,7 @@ DT_CHAMFER3, DT_EXACT = 0, 1
 DEPTH_U16, DEPTH_F32 = 0, 1
 POINTS_PIXEL, POINTS_XYZ = 0, 1
 IMAGE_BGR8, IMAGE_GRAY8 = 0, 1
+KEY_FIRST, KEY_INTERVAL, KEY_TRANSLATION, KEY_ROTATION, KEY_COST, KEY_LOST = 1, 2, 4, 8, 16, 32
 TERMINATION = {0: "NONE", 1: "CONVERGENCE_GRADIENT", 2: "CONVERGENCE_FUNCTION", 3: "CONVERGENCE_PARAMETER",
                4: "CONVERGENCE_MIN_RADIUS", 5: "NO_CONVERGENCE", 6: "FAILURE_EVAL_X0", 7: "FAILURE_INVALID_STEPS",
                8: "SKIPPED_NO_POINTS", 9: "FAILURE_PEER"}
@@ -61,6 +62,15 @@ class View(C.Structure):
     _fields_ = [("ref", C.c_void_p), ("ref_slot", C.c_int32), ("now", C.c_void_p), ("now_slot", C.c_int32),
                 ("use_distortion", C.c_int32), ("use_rig", C.c_int32), ("dist", C.c_double * 5),
                 ("cam_T_first", C.c_double * 12), ("first_T_cam", C.c_double * 12)]
+
+
+class KeyframePolicy(C.Structure):
+    _fields_ = [("max_interval", C.c_int32), ("reserved", C.c_int32), ("max_translation", C.c_double),
+                ("max_rotation", C.c_double), ("max_cost_per_residual", C.c_double)]
+
+
+class TrackInfo(C.Structure):
+    _fields_ = [("key_frame", C.c_int32), ("key_reasons", C.c_int32)]
 
 
 # every symbol include/ea_cabi.h declares: name -> (restype, argtypes)
@@ -115,6 +125,9 @@ PROTOTYPES = {
     "ea_tracker_probe_gather": (_i, [_vp, _i, _i, C.POINTER(C.c_float), C.POINTER(C.c_double)]),
     "ea_tracker_get_poses": (_i, [_vp, _f64p, C.POINTER(Summary)]),
     "ea_tracker_frame_index": (_i, [_vp, _pi]),
+    "ea_tracker_set_keyframe_policy": (_i, [_vp, C.POINTER(KeyframePolicy)]),
+    "ea_tracker_get_trajectory": (_i, [_vp, _f64p, C.POINTER(TrackInfo)]),
+    "ea_tracker_wait_trajectory": (_i, [_vp, _i, _f64p, C.POINTER(TrackInfo)]),
     "ea_shard_unique_id": (_i, [_u8p]),
     "ea_shard_create": (_i, [_vp, _u8p, _i, _i, C.POINTER(_vp)]),
     "ea_shard_destroy": (_i, [_vp]),

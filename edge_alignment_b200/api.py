@@ -354,6 +354,32 @@ class Tracker:
         _check(L.lib().ea_tracker_get_poses(self._h, _ptr(poses, C.c_double), S))
         return poses, S
 
+    def set_keyframe_policy(self, max_interval=0, max_translation=0.0, max_rotation=0.0, max_cost_per_residual=0.0):
+        """Per-stream key frames chosen on the device (ea_tracker_set_keyframe_policy); 0 turns a criterion off.
+        set_keyframe_policy(None): the fixed keyframe_interval again.  Only before the first step (after creation or reset)."""
+        if max_interval is None:
+            _check(L.lib().ea_tracker_set_keyframe_policy(self._h, None))
+            return
+        p = L.KeyframePolicy(max_interval=max_interval, max_translation=max_translation, max_rotation=max_rotation,
+                             max_cost_per_residual=max_cost_per_residual)
+        _check(L.lib().ea_tracker_set_keyframe_policy(self._h, C.byref(p)))
+
+    @staticmethod
+    def _track(world, info):
+        return (world, np.array([i.key_frame for i in info], np.int32), np.array([i.key_reasons for i in info], np.int32))
+
+    def trajectory(self):
+        """Latest step in policy mode: (world_T_frame [n_streams, 7], key_frame [n_streams], key_reasons [n_streams])."""
+        world = np.empty((self.n_streams, 7)); info = (L.TrackInfo * self.n_streams)()
+        _check(L.lib().ea_tracker_get_trajectory(self._h, _ptr(world, C.c_double), info))
+        return self._track(world, info)
+
+    def wait_trajectory(self, frame):
+        """trajectory() of a frame submitted with step_host(..., fetch=False)."""
+        world = np.empty((self.n_streams, 7)); info = (L.TrackInfo * self.n_streams)()
+        _check(L.lib().ea_tracker_wait_trajectory(self._h, frame, _ptr(world, C.c_double), info))
+        return self._track(world, info)
+
 
 class Shard:
     """One huge pair solved by all ranks together (BASELINE configs[4]): every rank holds the full distance transform and a

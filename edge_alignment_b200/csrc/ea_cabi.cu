@@ -297,7 +297,8 @@ static int check_slots(ea_frameset* fs, int n, const int32_t* slots) {
 
 }  // extern "C"
 int ea_preprocess_impl(ea_frameset* fs, int n, const int32_t* d_slots, const uint8_t* d_bgr, const void* d_depth, int roles,
-                       const uint8_t* d_mask, const uint8_t* d_now_mask, cudaStream_t stream, int in_channels) {
+                       const uint8_t* d_mask, const uint8_t* d_now_mask, cudaStream_t stream, int in_channels, int compact,
+                       const ea_track_info* compact_gate) {
   ea_context* c = fs->ctx;
   if (!stream) stream = c->stream;
   EaPrepArgs A;
@@ -311,6 +312,7 @@ int ea_preprocess_impl(ea_frameset* fs, int n, const int32_t* d_slots, const uin
   A.canny.low = fs->p.canny_low; A.canny.high = fs->p.canny_high; A.canny.l2 = fs->p.canny_l2;
   A.canny.on_color = (fs->p.edge_detector == EA_EDGE_CANNY_COLOR);
   A.scratch = fs->scratch;
+  A.compact = compact; A.compact_gate = compact_gate;
   A.depth_type = fs->p.depth_type; A.zero_to_one = fs->p.zero_depth_to_one;
   A.depth_one = fs->p.depth_type == EA_DEPTH_F32 ? 1.0f : float(fs->p.depth_scale);
   if (A.edge_detector != EA_EDGE_LAPLACIAN) A.use_median = 0;   // the Canny pipelines of the reference have no median step

@@ -85,7 +85,12 @@ struct EaPrepArgs {
   float depth_one;              // the stored value meaning Z = 1 (depth_scale for u16, 1.0 for f32)
   EaCannyCfg canny;
   EaScratch scratch;
+  int compact;                  // the reference-point lists (EA_ROLE_REF): EA_COMPACT_INLINE, _DEFER or _ONLY
+  const ea_track_info* compact_gate;   // EA_COMPACT_ONLY: frame i's lists are built only where compact_gate[i].key_reasons != 0
 };
+// EA_COMPACT_DEFER runs the edge kernels of the reference role (ref_bits and the depth pyramid in the slots) without building the
+// point lists; a later EA_COMPACT_ONLY call with the same slots and level-0 depth builds them for the frames its gate selects.
+enum { EA_COMPACT_INLINE = 0, EA_COMPACT_DEFER = 1, EA_COMPACT_ONLY = 2 };
 // enqueue the whole preprocessing pipeline for n frames; returns number of kernel launches via *launches
 // Optional second lane for big batches: the distance transforms (DRAM / latency-bound, few warps) of one part of the frames run on
 // an auxiliary stream beside the edge kernels (issue-bound) of the next part.  Streams and events belong to the context.
@@ -210,4 +215,4 @@ int ea_solve_batch_device_ordered(ea_context* c, int n, ea_frameset* ref, const 
 cudaError_t ea_launch_order_by_work(const ea_summary* d_summaries, int n, int n_levels, int32_t* d_order, cudaStream_t stream);
 int ea_preprocess_impl(ea_frameset* fs, int n, const int32_t* d_slots, const uint8_t* d_bgr, const void* d_depth, int roles,
                        const uint8_t* d_mask = nullptr, const uint8_t* d_now_mask = nullptr, cudaStream_t stream = nullptr,
-                       int in_channels = 3);
+                       int in_channels = 3, int compact = EA_COMPACT_INLINE, const ea_track_info* compact_gate = nullptr);

@@ -437,10 +437,13 @@ __global__ void __launch_bounds__(CP_THREADS) k_compact(const uint32_t* __restri
                                                         size_t frame_stride_px, const int32_t* __restrict__ src_slots,
                                                         const int32_t* __restrict__ dst_slots, float4* __restrict__ pts,
                                                         int* __restrict__ n_pts, int level, int* __restrict__ overflow,
-                                                        int w, int h, int words, int cap, int zero_to_one, float depth_one) {
+                                                        int w, int h, int words, int cap, int zero_to_one, float depth_one,
+                                                        const ea_track_info* __restrict__ gate) {
   __shared__ int warp_sums[CP_THREADS / 32];
   __shared__ int total_s;
-  const int f = blockIdx.x, slot = dst_slots[f];
+  const int f = blockIdx.x;
+  if (gate && gate[f].key_reasons == 0) return;                      // EA_COMPACT_ONLY: not promoted, no list needed
+  const int slot = dst_slots[f];
   const uint32_t* bits = ref_bits + size_t(slot) * h * words;
   const D* dep = depth + (src_slots ? size_t(src_slots[f]) : size_t(f)) * frame_stride_px;
   uint2* out = reinterpret_cast<uint2*>(pts + size_t(slot) * cap);   // 8-byte pixel points at the head of the slot's 16 B x cap area
@@ -1005,6 +1008,16 @@ static void launch_edge_mask2(const EaPrepArgs& A, const EaPrepLevel& L, const u
   else k_edge_mask2<D, TW, REF><<<grid, TW, 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
 }
 
+// the point lists of one level from the ref_bits plane and the depth (level 0: the caller's input by frame; above: the slot's pyramid)
+template <typename D>
+static void launch_compact(const EaPrepArgs& A, int l, cudaStream_t stream) {
+  const EaPrepLevel& L = A.lv[l];
+  const D* d = (l == 0) ? static_cast<const D*>(A.in_depth) : static_cast<const D*>(L.depth);
+  k_compact<D><<<A.n, CP_THREADS, 0, stream>>>(L.ref_bits, d, size_t(L.w) * L.h, (l == 0) ? nullptr : A.slots, A.slots, L.pts, A.n_pts, l,
+                                               A.overflow, L.w, L.h, L.words, L.cap, A.zero_to_one, A.depth_one,
+                                               A.compact == EA_COMPACT_ONLY ? A.compact_gate : nullptr);
+}
+
 template <typename D>
 static cudaError_t launch_edges_and_points(const EaPrepArgs& A, cudaStream_t stream, int& nl) {
   const bool want_ref = (A.roles & EA_ROLE_REF) != 0;
@@ -1067,8 +1080,8 @@ static cudaError_t launch_edges_and_points(const EaPrepArgs& A, cudaStream_t str
       k_mask_ref_bits<<<dim3(unsigned((L.h * L.words + 255) / 256), unsigned(A.n)), 256, 0, stream>>>(L.edge_bits, A.slots, A.in_now_mask, A.lv[0].w, A.lv[0].h, L.w, L.h, L.words, l, 1);
       ++nl;
     }
-    if (want_ref) {
-      k_compact<D><<<A.n, CP_THREADS, 0, stream>>>(L.ref_bits, d, pxl, ss, A.slots, L.pts, A.n_pts, l, A.overflow, L.w, L.h, L.words, L.cap, A.zero_to_one, A.depth_one);
+    if (want_ref && A.compact == EA_COMPACT_INLINE) {
+      launch_compact<D>(A, l, stream);
       ++nl;
     }
   }
@@ -1133,6 +1146,16 @@ cudaError_t ea_launch_preprocess(const EaPrepArgs& A, int sm_count, cudaStream_t
   int nl = 0;
   const bool want_ref = (A.roles & EA_ROLE_REF) != 0, want_now = (A.roles & EA_ROLE_NOW) != 0;
   if (want_ref && !A.in_depth) return cudaErrorInvalidValue;
+  if (A.compact == EA_COMPACT_ONLY) {
+    if (!want_ref || !A.compact_gate) return cudaErrorInvalidValue;
+    for (int l = 0; l < A.n_levels; ++l) {
+      if (A.depth_type == 1) launch_compact<float>(A, l, stream);
+      else launch_compact<uint16_t>(A, l, stream);
+      ++nl;
+    }
+    if (launches) *launches = nl;
+    return cudaGetLastError();
+  }
   // Two halves, two lanes: the chamfer kernel (DRAM- and latency-bound, ~40 % of the issue slots) of the first half runs beside
   // the edge kernels (issue-bound, a sixth of the DRAM bandwidth) of the second half.  Only the Laplacian + chamfer pipeline (its
   // work buffers are all indexed by slot), and only when both halves still fill the GPU: from EA_PREP_SPLIT (default 8) frames per

@@ -286,7 +286,7 @@ int ea_solve_views_batch(ea_context* ctx, int n_problems, const int32_t* view_of
 /* ---- tracker: the caller of the path (src/ea.cpp:87-131 consumer loop, re-stated) ------ */
 /* n_streams independent cameras; every step each stream gets one new frame which is aligned
  * to that stream's key frame (warm-started from the previous pose); every keyframe_interval-th
- * frame becomes the new key frame. */
+ * frame becomes the new key frame (unless ea_tracker_set_keyframe_policy chose the per-stream rule below). */
 int ea_tracker_create(ea_context* ctx, const ea_frame_params* fp, const ea_solve_params* sp, int n_streams,
                       int keyframe_interval, ea_tracker** out);
 int ea_tracker_destroy(ea_tracker* tr);
@@ -317,6 +317,47 @@ int ea_tracker_set_inputs_ready(ea_tracker* t, int ready);
 int ea_tracker_probe_gather(ea_tracker* tr, int level, int repeats, float* ms, double* point_gathers);
 int ea_tracker_get_poses(ea_tracker* tr, double* poses7, ea_summary* summaries); /* syncs */
 int ea_tracker_frame_index(ea_tracker* tr, int* n_frames_seen);
+
+/* Key-frame policy mode (opt-in; the default is the fixed keyframe_interval schedule of ea_tracker_create).  Every stream
+ * decides on the device, inside the asynchronous step, when its own key frame changes, and keeps its world trajectory.
+ *   poses7 (ea_tracker_get_poses / _wait) keep their meaning: key frame -> frame, X_frame = R X_key + t.
+ *   world pose of frame t: frame -> world, X_world = R_w X_frame + t_w; the world is the camera of the stream's frame 0 after
+ *   create / reset.  world_T_frame = world_T_key o inverse(pose7), composed in fp64 with a normalised quaternion.
+ * Rule: frame 0 is a key frame (EA_KEY_FIRST).  Frame t >= 1 is aligned to its stream's current key frame (warm start: the
+ * previous pose, identity after the stream's key frame changed); it then becomes the stream's new key frame if any enabled
+ * criterion fires (a threshold of 0 turns its criterion off; comparisons are strict):
+ *   EA_KEY_INTERVAL     max_interval > 0 and t - key_frame >= max_interval
+ *   EA_KEY_TRANSLATION  |t(pose7)| > max_translation (metres)
+ *   EA_KEY_ROTATION     2 atan2(|q_xyz|, |q_w|) > max_rotation (radians)
+ *   EA_KEY_COST         at sp.finest_level: n_residuals > 0 and final_cost / n_residuals > max_cost_per_residual
+ *   EA_KEY_LOST         always on: sp.finest_level terminated with EA_TERM_FAILURE_EVAL_X0, EA_TERM_FAILURE_INVALID_STEPS or
+ *                       EA_TERM_SKIPPED_NO_POINTS.  The pose is not trusted: the translation, rotation and cost criteria are not
+ *                       evaluated, the frame's world pose is held at the previous frame's, and the frame becomes the new key
+ *                       frame there (the stream re-anchors).
+ * Any frame may become a key frame, so every step needs depth (NULL depth: EA_ERR_INVALID_ARG) and every frame after the first
+ * is preprocessed for both roles; its point lists are built after the policy kernel, only if it was promoted.  The depth passed to
+ * ea_tracker_step_device is therefore read until that frame's alignment has finished (ea_tracker_get_poses / ea_sync order it).  The host path uploads depth on every step: for 640x480 GRAY8 frames with u16 depth the upload
+ * per stream and frame grows from about 0.37 MB (depth on every 10th frame) to about 0.92 MB (arithmetic from the sizes). */
+typedef struct ea_keyframe_policy {
+  int32_t max_interval;            /* frames since the key frame; 0 = no limit */
+  int32_t reserved;
+  double max_translation;          /* metres, 0 = off */
+  double max_rotation;             /* radians, 0 = off */
+  double max_cost_per_residual;    /* final_cost / n_residuals at the finest solved level, 0 = off */
+} ea_keyframe_policy;
+enum { EA_KEY_FIRST = 1, EA_KEY_INTERVAL = 2, EA_KEY_TRANSLATION = 4, EA_KEY_ROTATION = 8, EA_KEY_COST = 16, EA_KEY_LOST = 32 };
+typedef struct ea_track_info {
+  int32_t key_frame;   /* frame index of the key frame this frame was aligned to (frame 0: 0) */
+  int32_t key_reasons; /* EA_KEY_* bits that made this frame a key frame; 0 = not one */
+} ea_track_info;
+/* p == NULL: the fixed interval again.  Only before the first step (after create / reset), else EA_ERR_STATE.  Negative or
+ * non-finite thresholds and a negative max_interval: EA_ERR_INVALID_ARG.  ea_tracker_reset keeps the policy. */
+int ea_tracker_set_keyframe_policy(ea_tracker* tr, const ea_keyframe_policy* p);
+/* world7 [n_streams][7] and info [n_streams] of the latest step (HOST, either may be NULL); syncs.  EA_ERR_STATE outside
+ * policy mode. */
+int ea_tracker_get_trajectory(ea_tracker* tr, double* world7, ea_track_info* info);
+/* the same for frame `frame` submitted with ea_tracker_step_host(..., NULL, NULL): the 2-deep ring of ea_tracker_wait */
+int ea_tracker_wait_trajectory(ea_tracker* tr, int frame, double* world7, ea_track_info* info);
 
 /* ---- point-sharded single pair across ranks: one persistent cooperative kernel per rank, the 29 normal-equation sums
  * all-reduced inside the kernel through peer-mapped NVLink memory (NCCL only bootstraps the exchange of the cudaIpc
