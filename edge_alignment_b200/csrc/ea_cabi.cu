@@ -74,7 +74,7 @@ int ea_create(int device, ea_context** out) {
   c->own_stream = true;
   CU(cudaMalloc(&c->d_pose, 7 * sizeof(double)));
   CU(cudaMalloc(&c->d_failed, sizeof(int)));
-  CU(cudaMalloc(&c->d_work, sizeof(int)));
+  CU(cudaMalloc(&c->d_work, 2 * sizeof(int)));
   CU(cudaMalloc(&c->d_sums, size_t(1024) * EA_SUMS * sizeof(double)));
   {
     const char* h = getenv("EA_SOLVE_HELPERS");       // "0": no tail helpers (A/B measurements)
@@ -84,8 +84,8 @@ int ea_create(int device, ea_context** out) {
     }
   }
   if (getenv("EA_SOLVE_DEBUG")) {
-    CU(cudaMalloc(&c->d_debug, size_t(1024) * 6 * sizeof(unsigned long long)));
-    CU(cudaMemset(c->d_debug, 0, size_t(1024) * 6 * sizeof(unsigned long long)));
+    CU(cudaMalloc(&c->d_debug, size_t(2) * EA_DEBUG_ROWS * 6 * sizeof(unsigned long long)));
+    CU(cudaMemset(c->d_debug, 0, size_t(2) * EA_DEBUG_ROWS * 6 * sizeof(unsigned long long)));
   }
   guard.c = nullptr;
   *out = c;
@@ -95,12 +95,14 @@ int ea_destroy(ea_context* c) {
   if (!c) return EA_OK;
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
-  if (c->d_debug && c->debug_launches > 0) {
-    const double n = double(c->debug_launches);
-    fprintf(stderr, "[EA_SOLVE_DEBUG] %ld launches; per launch, mean over CTAs, kcycles of thread 0: eval %.1f  wait+totals %.1f  LM %.1f  wait2 %.1f  lifetime %.1f; evaluations %.1f\n",
-            c->debug_launches, c->debug_sum[0] / n / 1e3, c->debug_sum[1] / n / 1e3, c->debug_sum[2] / n / 1e3, c->debug_sum[3] / n / 1e3, c->debug_sum[5] / n / 1e3, c->debug_sum[4] / n);
+  for (int ph = 0; ph < 2; ++ph) {
+    if (!c->d_debug || c->debug_launches[ph] == 0) continue;
+    const double n = double(c->debug_launches[ph]);
+    const double* d = c->debug_sum[ph];
+    fprintf(stderr, "[EA_SOLVE_DEBUG]%s %ld launches; per launch, mean over CTAs, kcycles of thread 0: eval %.1f  wait+totals %.1f  LM %.1f  wait2 %.1f  lifetime %.1f; evaluations %.1f\n",
+            ph ? " coarse phase:" : "", c->debug_launches[ph], d[0] / n / 1e3, d[1] / n / 1e3, d[2] / n / 1e3, d[3] / n / 1e3, d[5] / n / 1e3, d[4] / n);
   }
-  cudaFree(c->d_debug); cudaFree(c->d_boards); cudaFree(c->d_views);
+  cudaFree(c->d_handoff); cudaFree(c->d_debug); cudaFree(c->d_boards); cudaFree(c->d_views);
   for (int k = 0; k < EA_PREP_MAX_PARTS; ++k) {
     if (c->prep_pipe.aux[k]) { cudaStreamSynchronize(c->prep_pipe.aux[k]); cudaStreamDestroy(c->prep_pipe.aux[k]); }
     if (c->prep_pipe.ev_front[k]) cudaEventDestroy(c->prep_pipe.ev_front[k]);
@@ -785,25 +787,50 @@ int ea_solve_batch_device_ordered(ea_context* c, int n, ea_frameset* ref, const 
   // tail helpers: CTAs that find the work queue empty serve the ones still solving.  They shorten the launch, not the work:
   // a caller that has other kernels ready to take over the idle SMs (the tracker's overlapped preprocessing) turns them off.
   A.boards = tail_helpers ? static_cast<EaHelpBoard*>(c->d_boards) : nullptr;
+  // Big batches over several levels solve the coarse levels in smaller CTAs, several per SM, so that one pair's serial LM step
+  // hides behind another pair's evaluation; level `finest` keeps the full-width kernel (ea_launch_solve_batch).
+  // EA_SOLVE_SPLIT=0: one launch over every level (A/B knob).  The results are the same either way.
+  static const bool split_on = !(getenv("EA_SOLVE_SPLIT") && getenv("EA_SOLVE_SPLIT")[0] == '0');
+  const bool split = split_on && cluster <= 1 && A.coarsest > A.finest && n >= 2 * c->sm_count;
+  if (split) {
+    if (c->handoff_cap < n) {
+      CU(cudaStreamSynchronize(c->stream));
+      cudaFree(c->d_handoff);
+      c->d_handoff = nullptr; c->handoff_cap = 0;
+      CU(cudaMalloc(&c->d_handoff, size_t(n) * sizeof(unsigned)));
+      CU(cudaMemsetAsync(c->d_handoff, 0, size_t(n) * sizeof(unsigned), c->stream));
+      c->handoff_cap = n;
+    }
+    A.handoff = c->d_handoff;
+    A.handoff_epoch = ++c->handoff_epoch;
+    if (A.handoff_epoch == 0) A.handoff_epoch = ++c->handoff_epoch;   // 0 is what a fresh array holds
+  }
   e = ea_launch_solve_batch(A, cluster, c->sm_count, c->stream);
   if (c->d_debug && e == cudaSuccess) {   // development aid: synchronous read-back of the cycle counters
     const int grid = std::min(n, c->sm_count);
     std::vector<unsigned long long> h(size_t(grid) * 6);
     cudaStreamSynchronize(c->stream);
     cudaMemcpy(h.data(), c->d_debug, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
-    for (int k = 0; k < 6; ++k) { double sum = 0; for (int b = 0; b < grid; ++b) sum += double(h[size_t(b) * 6 + k]); c->debug_sum[k] += sum / grid; }
+    for (int k = 0; k < 6; ++k) { double sum = 0; for (int b = 0; b < grid; ++b) sum += double(h[size_t(b) * 6 + k]); c->debug_sum[0][k] += sum / grid; }
+    if (split) {   // the coarse phase's rows
+      const int cgrid = std::min(n, c->sm_count * (EA_SOLVE_THREADS / EA_SOLVE_COARSE_THREADS));
+      std::vector<unsigned long long> hc(size_t(cgrid) * 6);
+      cudaMemcpy(hc.data(), c->d_debug + size_t(EA_DEBUG_ROWS) * 6, hc.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
+      for (int k = 0; k < 6; ++k) { double sum = 0; for (int b = 0; b < cgrid; ++b) sum += double(hc[size_t(b) * 6 + k]); c->debug_sum[1][k] += sum / cgrid; }
+      c->debug_launches[1]++;
+    }
     {   // owner-lifetime distribution of this launch (the launch ends with the last owner): mean / 75th / 90th percentile / max
       std::vector<double> life(static_cast<size_t>(grid));
       double mean = 0.0;
       for (int b = 0; b < grid; ++b) { life[size_t(b)] = double(h[size_t(b) * 6 + 5]); mean += life[size_t(b)] / grid; }
       std::sort(life.begin(), life.end());
-      if (c->debug_launches % 7 == 3)
-        fprintf(stderr, "[EA_SOLVE_DEBUG] launch %ld: owner lifetimes (kcycles) mean %.0f  p50 %.0f  p75 %.0f  p90 %.0f  p97 %.0f  max %.0f\n", c->debug_launches,
+      if (c->debug_launches[0] % 7 == 3)
+        fprintf(stderr, "[EA_SOLVE_DEBUG] launch %ld: owner lifetimes (kcycles) mean %.0f  p50 %.0f  p75 %.0f  p90 %.0f  p97 %.0f  max %.0f\n", c->debug_launches[0],
                 mean / 1e3, life[size_t(grid / 2)] / 1e3, life[size_t(grid * 3 / 4)] / 1e3, life[size_t(grid * 9 / 10)] / 1e3, life[size_t(grid * 97 / 100)] / 1e3, life[size_t(grid - 1)] / 1e3);
     }
-    c->debug_launches++;
+    c->debug_launches[0]++;
   }
-  c->launches++;
+  c->launches += split ? 2 : 1;
   if (e != cudaSuccess) return ea_fail(EA_ERR_CUDA, "solve launch: %s", cudaGetErrorString(e));
   return EA_OK;
 }

@@ -22,6 +22,11 @@ struct EaSolveArgs {
   int* work_counter;            // device: next pair index of the dynamic work queue (zeroed per launch)
   struct EaHelpBoard* boards;   // [grid] tail-helper boards of the persistent kernel (zeroed per launch), or null: no helpers
   unsigned long long* debug;    // null, or [grid][6] cycle counters of each CTA's thread 0 (EA_SOLVE_DEBUG=1, development aid)
+  // Coarse / fine split (ea_launch_solve_batch): the coarse phase publishes handoff[pair] = handoff_epoch with release
+  // semantics once the pair's pose after level finest + 1 is written; the fine phase acquires it before reading the pose.
+  unsigned* handoff;            // [n_pairs] device, or null: no split
+  unsigned handoff_epoch;       // tag of this launch (never 0, so that a zeroed array holds no hand-over)
+  int handoff_role;             // 0: none; 1: coarse phase (publishes); 2: fine phase (waits)
   ea_summary* summaries;        // [n_pairs][n_levels] device or null
   double* trace;                // [trace_cap][EA_TRACE_DOUBLES] device or null: one record per evaluation (single-pair solves only)
   int* trace_count;             // device counter of records written
@@ -35,6 +40,9 @@ struct EaSolveArgs {
   EaEvalConsts loss;                 // sp's loss in fp32 (ea_eval_consts), for the evaluation loop
 };
 
+// Non-cluster launches with A.handoff set and more than one level run as a coarse and a fine phase: A.work_counter then holds
+// two counters, and A.debug two blocks of EA_DEBUG_ROWS rows (fine phase first).
+#define EA_DEBUG_ROWS 1024
 cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm_count, cudaStream_t stream);
 size_t ea_help_boards_bytes(int sm_count);
 cudaError_t ea_launch_gather_probe(const EaSolveArgs& A, int level, int slices, int repeats, float* d_sink, cudaStream_t stream);
@@ -122,9 +130,11 @@ struct ea_context {
   // small scratch
   double* d_pose = nullptr;      // [7]
   int* d_failed = nullptr;
-  int* d_work = nullptr;         // work-queue counter of the batched solve
+  int* d_work = nullptr;         // [2] work-queue counters of the batched solve (fine / whole, coarse phase)
+  unsigned* d_handoff = nullptr; int handoff_cap = 0; unsigned handoff_epoch = 0;   // coarse -> fine hand-over words (EaSolveArgs)
   void* d_boards = nullptr; size_t boards_bytes = 0;        // tail-helper boards of the persistent solve kernel
-  unsigned long long* d_debug = nullptr; double debug_sum[6] = {0, 0, 0, 0, 0, 0}; long debug_launches = 0;   // EA_SOLVE_DEBUG=1
+  // EA_SOLVE_DEBUG=1: [2][EA_DEBUG_ROWS][6] cycle counters, and their sums per phase {fine or whole launch, coarse phase}
+  unsigned long long* d_debug = nullptr; double debug_sum[2][6] = {}; long debug_launches[2] = {0, 0};
   double* d_sums = nullptr;      // [max blocks][EA_SUMS]
   int32_t* d_idx = nullptr;      // scratch slot indices
   size_t idx_cap = 0;

@@ -71,13 +71,34 @@ struct alignas(2 * EA_STAGE_SLOT * 8) EaSolveSmem {
   double part[EA_MAX_CHUNKS][EA_SOLVE_WARPS][EA_NSUM];     // per chunk, per warp: lane-slot sums
   double cpart[EA_MAX_CHUNKS][EA_SOLVE_WARPS];             // per chunk, per warp: cost
   double sums[EA_SUMS + 3];                 // evaluation totals
-  double cluster_sums[8][EA_SUMS + 3];      // rank 0 only: one row per cluster rank
+  union {
+    double cluster_sums[8][EA_SUMS + 3];    // cluster launch, rank 0 only: one row per cluster rank
+    double vcost[EA_SOLVE_THREADS];         // CTAs narrower than EA_SOLVE_THREADS: per virtual thread fp64 cost (ea_eval_slice)
+  };
   EaLmState lm;                             // boss only
   int pair, level, truncated;               // boss only
   unsigned long long help_epoch;            // owner: evaluations published on its board so far
   int help_owner, help_index, help_fail;    // helper: the board it serves and its slot there (1-based); owner: a helper went missing
   long long dbg[6], dbg_t, dbg_t0;          // EA_SOLVE_DEBUG cycle counters (thread 0)
 };
+
+// ---- coarse / fine hand-over ------------------------------------------------------------------------------------------
+// The fine phase is launched as a programmatic dependent of the coarse phase and starts while coarse CTAs still finish their
+// last pairs, so it reads no pose before the coarse phase has published it.  Bounded spin: a pair whose hand-over never comes
+// fails instead of hanging the GPU.
+__device__ __forceinline__ void ea_st_release32(unsigned* p, unsigned v) {
+  asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __noinline__ bool ea_wait_handoff(const EaSolveArgs& A, const int pair) {
+  long long spins = 0;
+  for (;;) {
+    unsigned v;
+    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(A.handoff + pair) : "memory");
+    if (v == A.handoff_epoch) return true;
+    if (++spins > EA_BOARD_SPIN_LIMIT) return false;
+    __nanosleep(200);
+  }
+}
 
 // Boss: move to the next (pair, level) that has points and publish its first evaluation, or EXIT.
 template <bool INL>
@@ -88,6 +109,10 @@ __device__ __forceinline__ void ea_boss_next_impl(const EaSolveArgs& A, EaSolveS
       if (ticket >= A.n_pairs) { out.cmd = EA_CMD_EXIT; S.pair = -1; return; }
       const int pair = A.order ? A.order[ticket] : ticket;   // longest-expected-first when the caller knows better
       S.pair = pair; S.level = A.coarsest;
+      if (A.handoff_role == 2 && !ea_wait_handoff(A, pair)) {   // the coarse phase never handed this pair over
+        if (A.summaries) { ea_summary z = {}; z.termination = EA_TERM_FAILURE_PEER; A.summaries[size_t(pair) * A.n_levels + A.finest] = z; }
+        continue;
+      }
       const int pi = A.pose_index ? A.pose_index[pair] : pair;
 #pragma unroll 1
       for (int i = 0; i < 7; ++i) S.lm.x[i] = A.poses[size_t(pi) * 7 + i];
@@ -98,6 +123,7 @@ __device__ __forceinline__ void ea_boss_next_impl(const EaSolveArgs& A, EaSolveS
       const int pi = A.pose_index ? A.pose_index[pair] : pair;
 #pragma unroll 1
       for (int i = 0; i < 7; ++i) A.poses[size_t(pi) * 7 + i] = S.lm.x[i];
+      if (A.handoff_role == 1) ea_st_release32(&A.handoff[pair], A.handoff_epoch);
       new_pair_needed = true;
       continue;
     }
@@ -169,6 +195,7 @@ __device__ __forceinline__ void ea_boss_step_warp(const EaSolveArgs& A, EaSolveS
 
 // One worker's share of an evaluation: chunks [cb, ce) of M, walked in M's direction; per-chunk partials into S.part / S.cpart.
 // chain_next_eval: the same CTA evaluates the same chunks of the next evaluation of this (pair, level): prefetch its first point.
+// A CTA of THREADS < EA_SOLVE_THREADS evaluates as a virtual CTA of EA_SOLVE_THREADS threads: the same chunks, partials and sums.
 template <int THREADS>
 __device__ __forceinline__ void ea_eval_chunks(const EaSolveArgs& A, EaSolveSmem& S, const EaMsg& M, const EaPose& P, const int cb, const int ce,
                                                const int chunk, const bool pre_valid, const bool chain_next_eval) {
@@ -176,15 +203,18 @@ __device__ __forceinline__ void ea_eval_chunks(const EaSolveArgs& A, EaSolveSmem
   const bool rev = EA_ALTERNATE_SWEEP && M.rev, nrev = EA_ALTERNATE_SWEEP ? !rev : rev;
   const int lo = cb * chunk, hi = min(ce * chunk, M.n_res);
   if (M.pts_mode == EA_POINTS_XYZ)
-    ea_eval_slice<true, THREADS>(M.pts, M.dt, M.affine, ng, A.inv_depth_scale, A.loss, A.sp.point_stride, P, lo, hi, S.part[cb], S.cpart[cb], rev, nullptr, false, false, false,
-                                 chunk / THREADS, THREADS / 32);
+    ea_eval_slice<true, THREADS, EA_SOLVE_THREADS>(M.pts, M.dt, M.affine, ng, A.inv_depth_scale, A.loss, A.sp.point_stride, P, lo, hi, S.part[cb], S.cpart[cb], rev, nullptr,
+                                                   false, false, false, chunk / EA_SOLVE_THREADS, EA_SOLVE_WARPS, S.vcost);
   else
-    ea_eval_slice<false, THREADS>(M.pts, M.dt, M.affine, ng, A.inv_depth_scale, A.loss, A.sp.point_stride, P, lo, hi, S.part[cb], S.cpart[cb], rev, &S.stage[0][0], pre_valid, chain_next_eval, nrev,
-                                  chunk / THREADS, THREADS / 32);
+    ea_eval_slice<false, THREADS, EA_SOLVE_THREADS>(M.pts, M.dt, M.affine, ng, A.inv_depth_scale, A.loss, A.sp.point_stride, P, lo, hi, S.part[cb], S.cpart[cb], rev, &S.stage[0][0],
+                                                    pre_valid, chain_next_eval, nrev, chunk / EA_SOLVE_THREADS, EA_SOLVE_WARPS, S.vcost);
 }
 
+// A CTA narrower than EA_SOLVE_THREADS (the coarse phase) shares its SM with EA_SOLVE_THREADS / THREADS - 1 others: while one
+// runs its serial LM step, the others evaluate.
 template <int THREADS, bool CLUSTER>
-__global__ void __launch_bounds__(THREADS, EA_SOLVE_MIN_CTAS) ea_k_solve_batch(const __grid_constant__ EaSolveArgs A) {
+__global__ void __launch_bounds__(THREADS, THREADS < EA_SOLVE_THREADS ? EA_SOLVE_THREADS / THREADS : EA_SOLVE_MIN_CTAS)
+ea_k_solve_batch(const __grid_constant__ EaSolveArgs A) {
   __shared__ EaSolveSmem S;
   cg::cluster_group cluster = cg::this_cluster();
   const unsigned crank = CLUSTER ? cluster.block_rank() : 0u;
@@ -201,6 +231,10 @@ __global__ void __launch_bounds__(THREADS, EA_SOLVE_MIN_CTAS) ea_k_solve_batch(c
     }
   };
   unsigned g = 0;
+  // coarse phase: release the fine phase at once.  Its CTAs need a whole SM, so each takes one as soon as the coarse CTAs
+  // there have left, while others still finish their last pairs (measured: released by the boss thread when the coarse queue
+  // ran dry, the fine phase waited for the whole coarse tail, 7.51 against 6.86 ms per launch).
+  if (A.handoff_role == 1) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   if (tid == 0) S.args = A;
   __syncthreads();
   if (boss) {
@@ -233,7 +267,7 @@ __global__ void __launch_bounds__(THREADS, EA_SOLVE_MIN_CTAS) ea_k_solve_batch(c
       if (M.pts_mode == EA_POINTS_XYZ) ea_eval_slice<true, THREADS>(M.pts, M.dt, M.affine, ng, A.inv_depth_scale, A.loss, A.sp.point_stride, P, j0, j1, S.part[0], S.cpart[0], rev);
       else ea_eval_slice<false, THREADS>(M.pts, M.dt, M.affine, ng, A.inv_depth_scale, A.loss, A.sp.point_stride, P, j0, j1, S.part[0], S.cpart[0], rev, &S.stage[0][0], M.same != 0, true, nrev);
     } else {
-      K = ea_chunking(M.n_res, THREADS, chunk);
+      K = ea_chunking(M.n_res, EA_SOLVE_THREADS, chunk);
       cb = (K * M.nh) / (M.nh + 1);             // the owner is the last of nh + 1 workers: chunks [cb, K)
       ea_eval_chunks<THREADS>(A, S, M, P, cb, K, chunk, M.same != 0, true);
     }
@@ -264,7 +298,7 @@ __global__ void __launch_bounds__(THREADS, EA_SOLVE_MIN_CTAS) ea_k_solve_batch(c
         {   // the owner's chunks: four independent 16-term chains (unrolled so that they overlap), added in chunk order
           double ct[EA_MAX_CHUNKS];
 #pragma unroll
-          for (int c = 0; c < EA_MAX_CHUNKS; ++c) ct[c] = (c >= cb && c < K) ? ea_cta_total<THREADS / 32>(S.part[c], S.cpart[c], lane) : 0.0;
+          for (int c = 0; c < EA_MAX_CHUNKS; ++c) ct[c] = (c >= cb && c < K) ? ea_cta_total<EA_SOLVE_WARPS>(S.part[c], S.cpart[c], lane) : 0.0;
 #pragma unroll
           for (int c = 0; c < EA_MAX_CHUNKS; ++c) if (c >= cb && c < K) tot += ct[c];
         }
@@ -282,7 +316,7 @@ __global__ void __launch_bounds__(THREADS, EA_SOLVE_MIN_CTAS) ea_k_solve_batch(c
           // share the next evaluation with the registered helpers when it has chunks to give away
           int nh = 0;
           if (nm.cmd == EA_CMD_EVAL && reg > 0) {
-            int ch2; const int K2 = ea_chunking(nm.n_res, THREADS, ch2);
+            int ch2; const int K2 = ea_chunking(nm.n_res, EA_SOLVE_THREADS, ch2);
             nh = min(min(reg, EA_MAX_HELPERS), K2 - 1);
           }
           if (lane == 0) { nm.nh = nh; if (nh != M.nh) nm.same = 0; }
@@ -333,7 +367,9 @@ __global__ void __launch_bounds__(THREADS, EA_SOLVE_MIN_CTAS) ea_k_solve_batch(c
     for (int k = 0; k < 6; ++k) A.debug[size_t(blockIdx.x) * 6 + k] = (unsigned long long)S.dbg[k];
   }
   if (CLUSTER) { cluster.sync(); return; }  // no CTA may exit while a peer can still touch its shared memory
-  if (!helpers_on) return;
+  // fine phase: what the stream runs after this grid also runs after the coarse phase
+  auto end_of_fine_phase = [&]() { if (A.handoff_role == 2) asm volatile("griddepcontrol.wait;" ::: "memory"); };
+  if (!helpers_on) { end_of_fine_phase(); return; }
   // ================================================= helper loop ================================================
   // The queue is empty (tickets only grow, so no CTA will ever own a new pair): serve the CTAs that still own one.
   for (;;) {
@@ -393,13 +429,13 @@ __global__ void __launch_bounds__(THREADS, EA_SOLVE_MIN_CTAS) ea_k_solve_batch(c
       const EaMsg& M = S.msg[0];
       const EaPose P = M.P;
       int chunk;
-      const int K = ea_chunking(M.n_res, THREADS, chunk);
+      const int K = ea_chunking(M.n_res, EA_SOLVE_THREADS, chunk);
       const int cb = (K * (index - 1)) / (nh + 1), ce = (K * index) / (nh + 1);
       ea_eval_chunks<THREADS>(A, S, M, P, cb, ce, chunk, false, false);
       __syncthreads();
       if (warp == 0) {
         for (int c = cb; c < ce; ++c) {
-          const double tot = ea_cta_total<THREADS / 32>(S.part[c], S.cpart[c], lane);
+          const double tot = ea_cta_total<EA_SOLVE_WARPS>(S.part[c], S.cpart[c], lane);
           __stcg(&B->chunk[c][lane], lane < EA_SUMS ? tot : 0.0);
         }
         __threadfence();
@@ -409,6 +445,7 @@ __global__ void __launch_bounds__(THREADS, EA_SOLVE_MIN_CTAS) ea_k_solve_batch(c
       __syncthreads();
     }
   }
+  end_of_fine_phase();
 }
 
 // Per-point outputs for ea_eval (parity tests / EAResidue facade): same device functions as the solve.
@@ -519,7 +556,8 @@ size_t ea_help_boards_bytes(int sm_count) { return size_t(sm_count) * EA_SOLVE_M
 
 cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm_count, cudaStream_t stream) {
   if (A.n_pairs <= 0) return cudaSuccess;
-  cudaError_t e = cudaMemsetAsync(A.work_counter, 0, sizeof(int), stream);
+  const bool split = A.handoff != nullptr && cluster_size <= 1 && A.coarsest > A.finest;
+  cudaError_t e = cudaMemsetAsync(A.work_counter, 0, (split ? 2 : 1) * sizeof(int), stream);
   if (e != cudaSuccess) return e;
   if (A.boards && cluster_size <= 1) {
     e = cudaMemsetAsync(A.boards, 0, ea_help_boards_bytes(sm_count), stream);
@@ -531,12 +569,41 @@ cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm
   cudaLaunchAttribute attr[1];
   if (cluster_size <= 1) {
     // persistent CTAs (EA_SOLVE_MIN_CTAS per SM) pulling pairs from the work queue
-    int max_ctas = sm_count * EA_SOLVE_MIN_CTAS;
     static const int env_ctas = getenv("EA_SOLVE_MAX_CTAS") ? atoi(getenv("EA_SOLVE_MAX_CTAS")) : 0;   // experiment knob (DESIGN.md 8)
-    if (env_ctas > 0 && env_ctas < max_ctas) max_ctas = env_ctas;
-    cfg.gridDim = dim3(unsigned(A.n_pairs < max_ctas ? A.n_pairs : max_ctas));
+    auto grid_of = [&](const int per_sm) {
+      int max_ctas = sm_count * per_sm;
+      if (env_ctas > 0 && env_ctas < max_ctas) max_ctas = env_ctas;
+      return dim3(unsigned(A.n_pairs < max_ctas ? A.n_pairs : max_ctas));
+    };
+    if (!split) {
+      cfg.gridDim = grid_of(EA_SOLVE_MIN_CTAS);
+      cfg.numAttrs = 0;
+      return cudaLaunchKernelEx(&cfg, ea_k_solve_batch<EA_SOLVE_THREADS, false>, A);
+    }
+    // Coarse / fine split: levels coarsest .. finest + 1 in CTAs of EA_SOLVE_COARSE_THREADS (several per SM, no tail helpers,
+    // own work counter and debug rows), then level `finest` in the full-width kernel, launched as a programmatic dependent so
+    // that its CTAs take the SMs the coarse phase leaves (ea_wait_handoff orders each pair's pose).
+    EaSolveArgs Ac = A;
+    Ac.finest = A.finest + 1;
+    Ac.work_counter = A.work_counter + 1;
+    Ac.boards = nullptr;
+    Ac.debug = A.debug ? A.debug + size_t(EA_DEBUG_ROWS) * 6 : nullptr;
+    Ac.handoff_role = 1;
+    cfg.blockDim = dim3(EA_SOLVE_COARSE_THREADS);
+    cfg.gridDim = grid_of(EA_SOLVE_THREADS / EA_SOLVE_COARSE_THREADS);
     cfg.numAttrs = 0;
-    return cudaLaunchKernelEx(&cfg, ea_k_solve_batch<EA_SOLVE_THREADS, false>, A);
+    e = cudaLaunchKernelEx(&cfg, ea_k_solve_batch<EA_SOLVE_COARSE_THREADS, false>, Ac);
+    if (e != cudaSuccess) return e;
+    EaSolveArgs Af = A;
+    Af.coarsest = A.finest;
+    Af.handoff_role = 2;
+    cfg.blockDim = dim3(EA_SOLVE_THREADS);
+    cfg.gridDim = grid_of(EA_SOLVE_MIN_CTAS);
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, ea_k_solve_batch<EA_SOLVE_THREADS, false>, Af);
   }
   int n_clusters = A.n_pairs;
   const int max_clusters = (sm_count * EA_SOLVE_MIN_CTAS) / cluster_size;

@@ -11,6 +11,9 @@
 #ifndef EA_SOLVE_THREADS
 #define EA_SOLVE_THREADS 512   // threads per CTA of every kernel built on ea_eval_slice (128 registers each: one CTA fills an SM)
 #endif
+#ifndef EA_SOLVE_COARSE_THREADS
+#define EA_SOLVE_COARSE_THREADS 256   // threads per CTA of the batched solve's coarse phase (EA_SOLVE_THREADS / this many per SM)
+#endif
 
 #define EA_CMD_EVAL 0
 #define EA_CMD_DONE 1
@@ -583,32 +586,40 @@ __device__ __forceinline__ void ea_eval_point(const typename EaPtStream<XYZ>::T 
 // pre_valid: slot 0 already holds (or is about to receive) this call's first point, requested by the previous call;
 // prefetch_next: request the first point of the NEXT evaluation of the same range (direction next_reverse) into slot 0 before
 // returning, so that its latency hides behind the CTA barrier and the serial LM step.
-template <bool XYZ, int THREADS>
+//
+// VTHREADS > THREADS: a narrower CTA reproduces the iteration space, the partials and every rounding of a VTHREADS-thread CTA.
+// Real warp w plays the virtual warps w, w + THREADS / 32, ..., each with its own part / cpart rows; the loop walks one flush
+// block (EA_FLUSH_EVERY virtual iterations) of one virtual warp, flushes it, then the same block of the next virtual warp, so
+// every fp32 partial and fp64 addition is the wide CTA's, and the working set stays within one block of the point list.  The
+// per-thread fp64 cost of each virtual thread waits in vcost (shared, [VTHREADS]) between its blocks.
+template <bool XYZ, int THREADS, int VTHREADS = THREADS>
 __device__ __forceinline__ void ea_eval_slice(const void* __restrict__ pts, const float* __restrict__ dt_pad, const float2 affine,
                                               const EaLevelGeom& ng,
                                               double inv_depth_scale, const EaEvalConsts& loss, const int stride, const EaPose& P, const int j0,
                                               const int j1, double (*part)[EA_NSUM], double* cpart, const bool reverse = false,
                                               uint2* stage = nullptr, const bool pre_valid = false,
                                               const bool prefetch_next = false, const bool next_reverse = false,
-                                              const int chunk_iters = 0, const int part_stride = 0) {
+                                              const int chunk_iters = 0, const int part_stride = 0, double* vcost = nullptr) {
   static_assert(THREADS <= EA_STAGE_SLOT, "staging slot too small");
+  static_assert(VTHREADS % THREADS == 0, "the virtual CTA is a whole number of real CTAs wide");
+  constexpr int V = VTHREADS / THREADS, WARPS = THREADS / 32;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int W = ng.w, H = ng.h, pitch = ea_dt_pitch(W);
   const float* dt_base = ea_gather_base(dt_pad, pitch);
   const float afx = affine.x * P.fx, afy = affine.x * P.fy;
   typedef EaPtStream<XYZ> PS;
-  // virtual iteration space: residual of (iteration it, thread t) = j0 + it * THREADS + t   (forward)
-  //                                                                 vend - 1 - (it * THREADS + t)   (reverse)
+  // virtual iteration space: residual of (iteration it, thread t) = j0 + it * VTHREADS + t   (forward)
+  //                                                                 vend - 1 - (it * VTHREADS + t)   (reverse)
   const int n = j1 - j0;
-  const int n_it = (n + THREADS - 1) / THREADS;
-  const int cspan = chunk_iters > 0 ? chunk_iters * THREADS : 0;
+  const int n_it = (n + VTHREADS - 1) / VTHREADS;
+  const int cspan = chunk_iters > 0 ? chunk_iters * VTHREADS : 0;
   const int n_chunks = cspan > 0 ? (n + cspan - 1) / cspan : 1;
   const int vend = cspan > 0 ? j0 + n_chunks * cspan : j1;
-  const int it_first_rev = (vend - j1) / THREADS;             // reverse: whole iterations of padding above j1 are skipped
-  auto residual_of = [&](const int it, const bool rev) { return rev ? vend - 1 - (it * THREADS + tid) : j0 + it * THREADS + tid; };
+  const int it_first_rev = (vend - j1) / VTHREADS;            // reverse: whole iterations of padding above j1 are skipped
+  auto residual_of = [&](const int it, const bool rev) { return rev ? vend - 1 - (it * VTHREADS + tid) : j0 + it * VTHREADS + tid; };
   const int it0 = reverse ? it_first_rev : 0;
-  const int it1 = reverse ? (vend - j0 + THREADS - 1) / THREADS : n_it;
-  const int rstep = reverse ? -THREADS : THREADS;
+  const int it1 = reverse ? (vend - j0 + VTHREADS - 1) / VTHREADS : n_it;
+  const int rstep = reverse ? -VTHREADS : VTHREADS;
   EaEvalAcc A;
 #pragma unroll
   for (int k = 0; k < EA_NSUM; ++k) A.acc[k] = 0.0f;
@@ -616,7 +627,8 @@ __device__ __forceinline__ void ea_eval_slice(const void* __restrict__ pts, cons
   // The fp64 accumulators of the 32 slots live in shared memory (part itself): they are touched once per flush, and the
   // registers they would hold across the loop body are what keeps the prefetched point out of local memory.
   double cost64 = 0.0;
-  for (int k = 0; k < n_chunks; ++k) part[size_t(k) * part_stride + warp][lane] = 0.0;
+  for (int k = 0; k < n_chunks; ++k)
+    for (int v = 0; v < V; ++v) part[size_t(k) * part_stride + warp + v * WARPS][lane] = 0.0;
   typename PS::T p_next = PS::pad();
   int rj = residual_of(it0, reverse);                          // this thread's residual in the current iteration
   const bool staged = !XYZ && stage != nullptr;
@@ -629,6 +641,61 @@ __device__ __forceinline__ void ea_eval_slice(const void* __restrict__ pts, cons
   } else {
     if (unsigned(rj - j0) < unsigned(n)) p_next = PS::load(pts, size_t(rj) * stride);
   }
+  if constexpr (V > 1) {
+    for (int v = 0; v < V; ++v) vcost[v * THREADS + tid] = 0.0;
+    const int rbase = reverse ? vend - 1 - tid : j0 + tid;
+    // first residual of virtual warp v's share of iteration it
+    auto residual_v = [&](const int it, const int v) { const int o = it * VTHREADS + v * THREADS; return reverse ? rbase - o : rbase + o; };
+#pragma unroll 1
+    for (int lo = it0; lo < it1;) {
+      const int hi = min(it1, (lo | (EA_FLUSH_EVERY - 1)) + 1);   // the flush block [lo, hi) on the virtual iteration grid
+#pragma unroll 1
+      for (int v = 0; v < V; ++v) {
+#pragma unroll 1
+        for (int it = lo; it < hi; ++it) {
+          const bool valid = unsigned(rj - j0) < unsigned(n);
+          typename PS::T p = p_next;
+          // the next visit: this virtual warp's next iteration, else the next virtual warp's block, else the next block
+          rj = it + 1 < hi ? rj + rstep : (v + 1 < V ? residual_v(lo, v + 1) : residual_v(hi, 0));
+          if (staged) {
+            ea_cp_async_wait_all();
+            if constexpr (!XYZ) { p = ea_lds_u2(st_cur); }
+            st_cur ^= unsigned(EA_STAGE_SLOT * 8);
+            if (unsigned(rj - j0) < unsigned(n)) ea_cp_async8(st_cur, pts8 + size_t(unsigned(rj)) * stride8);
+            ea_cp_async_commit();
+          } else {
+            if (unsigned(rj - j0) < unsigned(n)) p_next = PS::load(pts, size_t(rj) * stride);
+          }
+          if (it == it0 || it + 1 == it1) {
+            if constexpr (!XYZ) { if (!valid) p = PS::pad(); }
+            ea_eval_point<XYZ, true>(p, valid, W, H, pitch, inv_depth_scale, P, dt_base, affine, afx, afy, loss, A);
+          } else {
+            ea_eval_point<XYZ, false>(p, true, W, H, pitch, inv_depth_scale, P, dt_base, affine, afx, afy, loss, A);
+          }
+        }
+        // the flush of block [lo, hi) for virtual warp v: the same operations as the wide CTA's flush at iteration hi - 1
+        A.acc[27] = A.zmin < 0 ? 1.0f : 0.0f;
+        A.zmin = 0x7fffffff;
+        double& c64v = vcost[v * THREADS + tid];
+        c64v += double(A.cost);
+        A.cost = 0.0f;
+        const int csh = 31 - __clz(chunk_iters | 1);
+        const int kc = chunk_iters > 0 ? (reverse ? n_chunks - 1 - ((hi - 1) >> csh) : ((hi - 1) >> csh)) : 0;
+        const int vwarp = warp + v * WARPS;
+        double* slot = &part[size_t(kc) * part_stride + vwarp][lane];
+        *slot += double(ea_warp_transpose_reduce(A.acc, lane));
+#pragma unroll
+        for (int k = 0; k < EA_NSUM; ++k) A.acc[k] = 0.0f;
+        if (hi == it1 || (chunk_iters > 0 && (hi & (chunk_iters - 1)) == 0)) {
+          const double c64 = ea_warp_sum(c64v);
+          if (lane == 0) cpart[size_t(kc) * part_stride + vwarp] = c64;
+          c64v = 0.0;
+        }
+      }
+      lo = hi;
+    }
+    if (it1 <= it0) { if (lane == 0) for (int v = 0; v < V; ++v) cpart[warp + v * WARPS] = 0.0; }
+  } else {   // a CTA as wide as the iteration space
   for (int it = it0; it < it1; ++it) {
     const bool valid = unsigned(rj - j0) < unsigned(n);
     typename PS::T p = p_next;
@@ -668,6 +735,7 @@ __device__ __forceinline__ void ea_eval_slice(const void* __restrict__ pts, cons
     }
   }
   if (it1 <= it0) { if (lane == 0) cpart[warp] = 0.0; }        // empty range
+  }
   if (staged && prefetch_next) {
     const int rn = residual_of(next_reverse ? it_first_rev : 0, next_reverse);
     ea_cp_async_wait_all();                                      // (nothing of this call is still reading or filling slot 0)

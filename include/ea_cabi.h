@@ -91,7 +91,8 @@ typedef enum ea_termination {
   EA_TERM_FAILURE_EVAL_X0 = 6, /* functor returned false at x0 (utils.h:70-73) */
   EA_TERM_FAILURE_INVALID_STEPS = 7,
   EA_TERM_SKIPPED_NO_POINTS = 8,
-  EA_TERM_FAILURE_PEER = 9      /* point-sharded solve: a peer rank stopped answering the all-reduce */
+  EA_TERM_FAILURE_PEER = 9      /* point-sharded solve: a peer rank stopped answering the all-reduce; batched solve: the
+                                   coarse levels of the pair were never handed over to its finest level */
 } ea_termination;
 
 /* Preprocessing configuration: every literal of utils.cpp:38-83,201-281 and
