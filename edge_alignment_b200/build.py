@@ -29,8 +29,7 @@ def needs_build():
 
 
 def build(force=False, verbose=False):
-    extra = os.environ.get("EA_NVCC_EXTRA", "").split()     # tuning experiments only (e.g. -DEA_SOLVE_THREADS=512)
-    if not force and not extra and not needs_build():
+    if not force and not needs_build():
         return SO
     os.makedirs(os.path.join(HERE, "_obj"), exist_ok=True)
     objs = []
@@ -41,7 +40,7 @@ def build(force=False, verbose=False):
             continue
         obj = os.path.join(HERE, "_obj", s.replace(".cu", ".o"))
         objs.append(obj)
-        cmd = [nvcc()] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
+        cmd = [nvcc()] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
         procs.append((cmd, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
     for cmd, p in procs:
         out, _ = p.communicate()

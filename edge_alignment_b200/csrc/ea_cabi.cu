@@ -76,13 +76,7 @@ int ea_create(int device, ea_context** out) {
   CU(cudaMalloc(&c->d_failed, sizeof(int)));
   CU(cudaMalloc(&c->d_work, 2 * sizeof(int)));
   CU(cudaMalloc(&c->d_sums, size_t(1024) * EA_SUMS * sizeof(double)));
-  {
-    const char* h = getenv("EA_SOLVE_HELPERS");       // "0": no tail helpers (A/B measurements)
-    if (!(h && h[0] == '0')) {
-      c->boards_bytes = ea_help_boards_bytes(c->sm_count);
-      CU(cudaMalloc(&c->d_boards, c->boards_bytes));
-    }
-  }
+  CU(cudaMalloc(&c->d_boards, ea_help_boards_bytes(c->sm_count)));
   if (getenv("EA_SOLVE_DEBUG")) {
     CU(cudaMalloc(&c->d_debug, size_t(2) * EA_DEBUG_ROWS * 6 * sizeof(unsigned long long)));
     CU(cudaMemset(c->d_debug, 0, size_t(2) * EA_DEBUG_ROWS * 6 * sizeof(unsigned long long)));
@@ -325,8 +319,7 @@ int ea_preprocess_impl(ea_frameset* fs, int n, const int32_t* d_slots, const uin
       // (highest priority: the long-lived one-warp chamfer CTAs take the slots the short edge CTAs free, instead of queueing behind them)
       int pr_lo = 0, pr_hi = 0;
       CU(cudaDeviceGetStreamPriorityRange(&pr_lo, &pr_hi));
-      static const int env_prio = getenv("EA_PREP_PRIO") ? atoi(getenv("EA_PREP_PRIO")) : 1;
-      CU(cudaStreamCreateWithPriority(&P.aux[k], cudaStreamNonBlocking, env_prio ? pr_hi : pr_lo));
+      CU(cudaStreamCreateWithPriority(&P.aux[k], cudaStreamNonBlocking, pr_hi));
       CU(cudaEventCreateWithFlags(&P.ev_front[k], cudaEventDisableTiming));
       CU(cudaEventCreateWithFlags(&P.ev_dt[k], cudaEventDisableTiming));
     }
@@ -689,7 +682,7 @@ int ea_eval(ea_context* c, ea_frameset* ref, int ref_slot, ea_frameset* now, int
   return EA_OK;
 }
 
-static int fill_solve_args(ea_context* c, ea_frameset* ref, ea_frameset* now, const ea_solve_params* sp, EaSolveArgs& A, int* cluster) {
+static int fill_solve_args(ea_frameset* ref, ea_frameset* now, const ea_solve_params* sp, EaSolveArgs& A, int* cluster) {
   int rc = ea_check_solve_params(sp);
   if (!rc) rc = check_pairable(ref, now);
   if (rc) return rc;
@@ -704,7 +697,6 @@ static int fill_solve_args(ea_context* c, ea_frameset* ref, ea_frameset* now, co
   A.sp = *sp;
   A.loss = ea_eval_consts(sp->loss_type, sp->loss_scale, sp->point_stride);
   *cluster = sp->cluster_size;
-  (void)c;
   return EA_OK;
 }
 
@@ -734,7 +726,7 @@ int ea_probe_gather_device(ea_context* c, int n, ea_frameset* ref, const int32_t
   ea_solve_params_default(&sp);
   EaSolveArgs A;
   int cluster = 0;
-  int rc = fill_solve_args(c, ref, now, &sp, A, &cluster);
+  int rc = fill_solve_args(ref, now, &sp, A, &cluster);
   if (rc) return rc;
   if (level < 0 || level >= ref->p.n_levels) return ea_fail(EA_ERR_INVALID_ARG, "level %d out of range", level);
   CU(cudaSetDevice(c->device));
@@ -771,7 +763,7 @@ int ea_solve_batch_device_ordered(ea_context* c, int n, ea_frameset* ref, const 
   if (n <= 0) return EA_OK;
   EaSolveArgs A;
   int cluster = 0;
-  int rc = fill_solve_args(c, ref, now, sp, A, &cluster);
+  int rc = fill_solve_args(ref, now, sp, A, &cluster);
   if (rc) return rc;
   CU(cudaSetDevice(c->device));
   A.ref_slots = d_ref_slots; A.now_slots = d_now_slots; A.pose_index = d_pose_index; A.poses = d_poses7;
@@ -788,10 +780,9 @@ int ea_solve_batch_device_ordered(ea_context* c, int n, ea_frameset* ref, const 
   // a caller that has other kernels ready to take over the idle SMs (the tracker's overlapped preprocessing) turns them off.
   A.boards = tail_helpers ? static_cast<EaHelpBoard*>(c->d_boards) : nullptr;
   // Big batches over several levels solve the coarse levels in smaller CTAs, several per SM, so that one pair's serial LM step
-  // hides behind another pair's evaluation; level `finest` keeps the full-width kernel (ea_launch_solve_batch).
-  // EA_SOLVE_SPLIT=0: one launch over every level (A/B knob).  The results are the same either way.
-  static const bool split_on = !(getenv("EA_SOLVE_SPLIT") && getenv("EA_SOLVE_SPLIT")[0] == '0');
-  const bool split = split_on && cluster <= 1 && A.coarsest > A.finest && n >= 2 * c->sm_count;
+  // hides behind another pair's evaluation; level `finest` keeps the full-width kernel (ea_launch_solve_batch).  The results
+  // are those of one launch over every level.
+  const bool split = cluster <= 1 && A.coarsest > A.finest && n >= 2 * c->sm_count;
   if (split) {
     if (c->handoff_cap < n) {
       CU(cudaStreamSynchronize(c->stream));

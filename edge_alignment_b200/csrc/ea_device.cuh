@@ -220,13 +220,8 @@ __device__ __forceinline__ const float* ea_gather_base(const float* dt_pad, cons
 __device__ __forceinline__ void ea_gather(const float* __restrict__ base, const int off, const int pitch, float (&t)[16]) {
   // one 32-bit element offset per footprint row, widened against the single 64-bit base (IMAD.WIDE), the four columns as
   // immediates: 7 integer instructions for the 16 addresses
-#ifdef EA_EXPERIMENT_L1_RESIDENT   // timing experiment only (wrong results): every gather lands in a 64 KB window => always L1 hits
-  const int off_ = off & 0x3fff;
-#else
-  const int off_ = off;
-#endif
-  const int o1 = off_ + pitch, o2 = o1 + pitch, o3 = o2 + pitch;
-  const float* p0 = base + off_;
+  const int o1 = off + pitch, o2 = o1 + pitch, o3 = o2 + pitch;
+  const float* p0 = base + off;
   const float* p1 = base + o1;
   const float* p2 = base + o2;
   const float* p3 = base + o3;

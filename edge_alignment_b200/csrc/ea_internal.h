@@ -102,7 +102,7 @@ enum { EA_COMPACT_INLINE = 0, EA_COMPACT_DEFER = 1, EA_COMPACT_ONLY = 2 };
 // enqueue the whole preprocessing pipeline for n frames; returns number of kernel launches via *launches
 // Optional second lane for big batches: the distance transforms (DRAM / latency-bound, few warps) of one part of the frames run on
 // an auxiliary stream beside the edge kernels (issue-bound) of the next part.  Streams and events belong to the context.
-#define EA_PREP_MAX_PARTS 4
+#define EA_PREP_MAX_PARTS 2
 struct EaPrepPipe {
   cudaStream_t aux[EA_PREP_MAX_PARTS] = {};
   cudaEvent_t ev_front[EA_PREP_MAX_PARTS] = {}, ev_dt[EA_PREP_MAX_PARTS] = {};
@@ -132,7 +132,7 @@ struct ea_context {
   int* d_failed = nullptr;
   int* d_work = nullptr;         // [2] work-queue counters of the batched solve (fine / whole, coarse phase)
   unsigned* d_handoff = nullptr; int handoff_cap = 0; unsigned handoff_epoch = 0;   // coarse -> fine hand-over words (EaSolveArgs)
-  void* d_boards = nullptr; size_t boards_bytes = 0;        // tail-helper boards of the persistent solve kernel
+  void* d_boards = nullptr;       // tail-helper boards of the persistent solve kernel
   // EA_SOLVE_DEBUG=1: [2][EA_DEBUG_ROWS][6] cycle counters, and their sums per phase {fine or whole launch, coarse phase}
   unsigned long long* d_debug = nullptr; double debug_sum[2][6] = {}; long debug_launches[2] = {0, 0};
   double* d_sums = nullptr;      // [max blocks][EA_SUMS]

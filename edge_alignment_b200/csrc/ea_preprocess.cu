@@ -776,9 +776,7 @@ __device__ __forceinline__ void dtw_row_scan(int (&d)[P], const int (&cval)[P], 
 }
 
 // FULL: every lane's strip lies inside the image (w == 32 * P, e.g. 640 px at P = 20): the per-pixel bound checks drop out.
-#ifndef DTW_L2_AHEAD
 #define DTW_L2_AHEAD 4      // rows of L2 prefetch distance (measured: see profiles)
-#endif
 // SEG: lanes per frame.  A row of 32 * P pixels takes the whole warp; the coarser pyramid levels of a 640-pixel frame (320, 160,
 // 80 pixels) would leave most strips empty -- and paid 2-3x the instructions per pixel of level 0 -- so they run as 2 / 4 / 8
 // frames side by side in one warp, each on SEG = 16 / 8 / 4 lanes with the same full 20-pixel strips (segmented shuffles).
@@ -994,8 +992,7 @@ static bool edge_kernel_fuses_pyramid(const EaPrepArgs& A, int l) {
   if (l + 1 >= A.n_levels || A.edge_detector != EA_EDGE_LAPLACIAN) return false;
   const EaPrepLevel& L = A.lv[l];
   const EaPrepLevel& N = A.lv[l + 1];
-  static const int env_fuse = getenv("EA_PYR_FUSE") ? atoi(getenv("EA_PYR_FUSE")) : 1;
-  return env_fuse && (L.w & 3) == 0 && L.w >= 8 && L.h >= 4 && gray_words_ok(A, l) && (N.w & 3) == 0 && (reinterpret_cast<uintptr_t>(N.bgr) & 3) == 0;
+  return (L.w & 3) == 0 && L.w >= 8 && L.h >= 4 && gray_words_ok(A, l) && (N.w & 3) == 0 && (reinterpret_cast<uintptr_t>(N.bgr) & 3) == 0;
 }
 
 // the fused edge kernel of one level for CN-channel input (k_edge_mask2 on BGR, k_edge_mask2_gray on gray)
@@ -1111,20 +1108,17 @@ static cudaError_t launch_dt(const EaPrepArgs& A, cudaStream_t stream, int& nl) 
     return cudaGetLastError();
   }
   const EaPrepLevel& L0 = A.lv[0];
-  static const int env_block = getenv("EA_DT_BLOCK") ? atoi(getenv("EA_DT_BLOCK")) : 0;   // A/B knob: force the block kernel
-  if (L0.w <= 32 * DTW_PMAX && !env_block) {   // one warp per (frame, level); level 0 CTAs are scheduled first
+  if (L0.w <= 32 * DTW_PMAX) {   // one warp per (frame, level); level 0 CTAs are scheduled first
     k_chamfer_dt_warp<<<dim3(unsigned(A.n), unsigned(A.n_levels)), 32, 0, stream>>>(A);
     ++nl;
     return cudaGetLastError();
   }
   // wider images: every level of every frame in one launch, CTA (frame, level); block sized for level 0
-  int P = (L0.w <= 4096) ? 4 : 8;
-  if (const char* e = getenv("EA_DT_P")) { const int v = atoi(e); if ((v == 2 || v == 4 || v == 8) && v > P) P = v; }   // tuning knob
+  const int P = (L0.w <= 4096) ? 4 : 8;
   const int threads = (((L0.w + P - 1) / P + 31) / 32) * 32;
   if (threads > 1024) return cudaErrorInvalidValue;
   dim3 grid(unsigned(A.n), unsigned(A.n_levels));
-  if (P == 2) k_chamfer_dt<2><<<grid, threads, 0, stream>>>(A);
-  else if (P == 4) k_chamfer_dt<4><<<grid, threads, 0, stream>>>(A);
+  if (P == 4) k_chamfer_dt<4><<<grid, threads, 0, stream>>>(A);
   else k_chamfer_dt<8><<<grid, threads, 0, stream>>>(A);
   ++nl;
   for (int l = 0; l < A.n_levels; ++l) { ea_launch_dt_fill_pad(A.lv[l], A.slots, A.n, stream); ++nl; }
@@ -1158,18 +1152,17 @@ cudaError_t ea_launch_preprocess(const EaPrepArgs& A, int sm_count, cudaStream_t
   }
   // Two halves, two lanes: the chamfer kernel (DRAM- and latency-bound, ~40 % of the issue slots) of the first half runs beside
   // the edge kernels (issue-bound, a sixth of the DRAM bandwidth) of the second half.  Only the Laplacian + chamfer pipeline (its
-  // work buffers are all indexed by slot), and only when both halves still fill the GPU: from EA_PREP_SPLIT (default 8) frames per
-  // SM; 0 turns it off.
-  static const int env_split = getenv("EA_PREP_SPLIT") ? atoi(getenv("EA_PREP_SPLIT")) : 8;
-  const bool split = env_split > 0 && pipe && pipe->ready && want_now && A.edge_detector == EA_EDGE_LAPLACIAN && A.dt_kind != EA_DT_EXACT &&
-                     A.lv[0].w <= 32 * DTW_PMAX && A.n >= env_split * sm_count;
+  // work buffers are all indexed by slot), and only when both halves still fill the GPU: from 8 frames per SM (at 4 the halves
+  // no longer fill it, DESIGN.md 4.4).
+  const int split_frames_per_sm = 8;
+  const bool split = pipe && pipe->ready && want_now && A.edge_detector == EA_EDGE_LAPLACIAN && A.dt_kind != EA_DT_EXACT &&
+                     A.lv[0].w <= 32 * DTW_PMAX && A.n >= split_frames_per_sm * sm_count;
   cudaError_t e = cudaSuccess;
   if (!split) {
     e = launch_front(A, stream, nl);
     if (e == cudaSuccess && want_now) e = launch_dt(A, stream, nl);
   } else {
-    static const int env_parts = getenv("EA_PREP_PARTS") ? atoi(getenv("EA_PREP_PARTS")) : 2;
-    const int K = env_parts < 2 ? 2 : env_parts > EA_PREP_MAX_PARTS ? EA_PREP_MAX_PARTS : env_parts;
+    const int K = EA_PREP_MAX_PARTS;
     int forked = 0;                                       // parts whose distance transforms are on their lane
     for (int k = 0; k < K && e == cudaSuccess; ++k) {
       const int f0 = int((long long)A.n * k / K), f1 = int((long long)A.n * (k + 1) / K);
@@ -1189,7 +1182,6 @@ cudaError_t ea_launch_preprocess(const EaPrepArgs& A, int sm_count, cudaStream_t
       if (e == cudaSuccess) e = je;
     }
   }
-  (void)sm_count;
   if (launches) *launches = nl;
   return e != cudaSuccess ? e : cudaGetLastError();
 }

@@ -140,10 +140,10 @@ __global__ void __launch_bounds__(THREADS, 1) k_shard_solve(EaLevelDesc rd, EaLe
 #pragma unroll
       for (int i = 0; i < int(sizeof(EaPose) / 8); ++i) dst[i] = __ldcg(src + i);
     }
-    if (xyz) ea_eval_slice<true, THREADS>(rd.pts, dt_pad, affine, ng, inv_depth_scale, loss, sp.point_stride, P, j0, j1, part, cpart, EA_ALTERNATE_SWEEP && !(e & 1));
+    if (xyz) ea_eval_slice<true, THREADS>(rd.pts, dt_pad, affine, ng, inv_depth_scale, loss, sp.point_stride, P, j0, j1, part, cpart, !(e & 1));
     else {
-      const bool rev = EA_ALTERNATE_SWEEP && !(e & 1);
-      ea_eval_slice<false, THREADS>(rd.pts, dt_pad, affine, ng, inv_depth_scale, loss, sp.point_stride, P, j0, j1, part, cpart, rev, &stage[0][0], e > 1, true, EA_ALTERNATE_SWEEP ? !rev : rev);
+      const bool rev = !(e & 1);
+      ea_eval_slice<false, THREADS>(rd.pts, dt_pad, affine, ng, inv_depth_scale, loss, sp.point_stride, P, j0, j1, part, cpart, rev, &stage[0][0], e > 1, true, !rev);
     }
     __syncthreads();
     if (warp == 0) {
@@ -379,7 +379,7 @@ int ea_shard_create(ea_context* ctx, const uint8_t id128[128], int rank, int wor
   if (!rc && cudaHostAlloc((void**)&s->h_done, sizeof(int), cudaHostAllocDefault) != cudaSuccess) rc = ea_fail(EA_ERR_CUDA, "ea_shard_create: cudaHostAlloc failed");
   if (!rc) rc = shard_open_peers(s);
   if (!rc) {
-    const char* mode = getenv("EA_SHARD_MODE");      // "nccl": force the host-driven path (A/B measurements)
+    const char* mode = getenv("EA_SHARD_MODE");      // "nccl": force the host-driven path (the one GPUs without peer access take)
     if (mode && !strcmp(mode, "nccl")) s->in_kernel = false;
     int khz = 0;
     cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, ctx->device);

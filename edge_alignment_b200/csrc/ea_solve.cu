@@ -13,17 +13,12 @@
 #include <cooperative_groups.h>
 
 #include "ea_internal.h"
-#include <cstdlib>
 
 #include "ea_solve.cuh"
 
 namespace cg = cooperative_groups;
 
 #define EA_SOLVE_WARPS (EA_SOLVE_THREADS / 32)
-#ifndef EA_SOLVE_MIN_CTAS
-#define EA_SOLVE_MIN_CTAS 1
-#endif
-// points per thread between fp32->fp64 flushes of the normal-equation slots
 #define EA_CMD_EXIT 2
 
 struct EaMsg {  // boss -> all threads of the cluster
@@ -156,15 +151,7 @@ __device__ __noinline__ void ea_boss_next(const EaSolveArgs& A, EaSolveSmem& S, 
 // warp 0's branch of the kernel: as a call it received its arguments and the kernel's live values through the stack frame.
 __device__ __forceinline__ void ea_boss_step_warp(const EaSolveArgs& A, EaSolveSmem& S, const EaMsg& cur, EaMsg& out, const int lane) {
   const int acc0 = S.lm.accepted, rej0 = S.lm.rejected;
-#ifdef EA_LM_PROFILE
-  const long long t_in = clock64();
-#endif
   const int cmd = ea_lm_advance_warp(S.lm, S.sums, A.sp, lane);
-#ifdef EA_LM_PROFILE
-  __syncwarp();
-  if (lane == 0) { S.lm.prof[6] += clock64() - t_in; S.lm.prof[7] += 1; }
-  __syncwarp();
-#endif
   if (A.trace && lane == 0) {   // iteration log of a single-pair solve (ea_solve_traced): what Ceres prints with minimizer_progress_to_stdout
     const int k = (*A.trace_count)++;
     if (k < A.trace_cap) {
@@ -200,7 +187,7 @@ template <int THREADS>
 __device__ __forceinline__ void ea_eval_chunks(const EaSolveArgs& A, EaSolveSmem& S, const EaMsg& M, const EaPose& P, const int cb, const int ce,
                                                const int chunk, const bool pre_valid, const bool chain_next_eval) {
   const EaLevelGeom& ng = A.now_geom[M.level];
-  const bool rev = EA_ALTERNATE_SWEEP && M.rev, nrev = EA_ALTERNATE_SWEEP ? !rev : rev;
+  const bool rev = M.rev != 0, nrev = !rev;
   const int lo = cb * chunk, hi = min(ce * chunk, M.n_res);
   if (M.pts_mode == EA_POINTS_XYZ)
     ea_eval_slice<true, THREADS, EA_SOLVE_THREADS>(M.pts, M.dt, M.affine, ng, A.inv_depth_scale, A.loss, A.sp.point_stride, P, lo, hi, S.part[cb], S.cpart[cb], rev, nullptr,
@@ -213,7 +200,7 @@ __device__ __forceinline__ void ea_eval_chunks(const EaSolveArgs& A, EaSolveSmem
 // A CTA narrower than EA_SOLVE_THREADS (the coarse phase) shares its SM with EA_SOLVE_THREADS / THREADS - 1 others: while one
 // runs its serial LM step, the others evaluate.
 template <int THREADS, bool CLUSTER>
-__global__ void __launch_bounds__(THREADS, THREADS < EA_SOLVE_THREADS ? EA_SOLVE_THREADS / THREADS : EA_SOLVE_MIN_CTAS)
+__global__ void __launch_bounds__(THREADS, THREADS < EA_SOLVE_THREADS ? EA_SOLVE_THREADS / THREADS : 1)
 ea_k_solve_batch(const __grid_constant__ EaSolveArgs A) {
   __shared__ EaSolveSmem S;
   cg::cluster_group cluster = cg::this_cluster();
@@ -249,9 +236,6 @@ ea_k_solve_batch(const __grid_constant__ EaSolveArgs A) {
   // (counters live in shared memory: the evaluation loop has no registers to spare)
   const bool dbg_on = A.debug != nullptr && tid == 0;
   if (dbg_on) { for (int k = 0; k < 6; ++k) S.dbg[k] = 0; S.dbg_t0 = clock64(); S.dbg_t = S.dbg_t0; }
-#ifdef EA_LM_PROFILE
-  if (tid == 0) for (int k = 0; k < 8; ++k) S.lm.prof[k] = 0;
-#endif
   auto lap = [&](int k) { if (dbg_on) { const long long t = clock64(); S.dbg[k] += t - S.dbg_t; S.dbg_t = t; } };
   // ================================================= owner loop =================================================
   for (;;) {
@@ -263,7 +247,7 @@ ea_k_solve_batch(const __grid_constant__ EaSolveArgs A) {
       // a cluster shares the evaluation by rank: one slice, one partial per CTA
       const int j0 = int((long long)M.n_res * crank / csize), j1 = int((long long)M.n_res * (crank + 1) / csize);
       const EaLevelGeom& ng = A.now_geom[M.level];
-      const bool rev = EA_ALTERNATE_SWEEP && M.rev, nrev = EA_ALTERNATE_SWEEP ? !rev : rev;
+      const bool rev = M.rev != 0, nrev = !rev;
       if (M.pts_mode == EA_POINTS_XYZ) ea_eval_slice<true, THREADS>(M.pts, M.dt, M.affine, ng, A.inv_depth_scale, A.loss, A.sp.point_stride, P, j0, j1, S.part[0], S.cpart[0], rev);
       else ea_eval_slice<false, THREADS>(M.pts, M.dt, M.affine, ng, A.inv_depth_scale, A.loss, A.sp.point_stride, P, j0, j1, S.part[0], S.cpart[0], rev, &S.stage[0][0], M.same != 0, true, nrev);
     } else {
@@ -357,11 +341,6 @@ ea_k_solve_batch(const __grid_constant__ EaSolveArgs A) {
     if (dbg_on) S.dbg[4] += 1;
     g += 1;
   }
-#ifdef EA_LM_PROFILE
-  if (dbg_on && blockIdx.x == 0 && S.dbg[4] > 0)
-    printf("[EA_LM_PROFILE] CTA 0, %lld evaluations; cycles per evaluation: tests %lld, update %lld, build %lld, LDLT %lld, model %lld, plus+stores %lld | advance_warp mean %lld\n",
-           S.dbg[4], S.lm.prof[0] / S.dbg[4], S.lm.prof[1] / S.dbg[4], S.lm.prof[2] / S.dbg[4], S.lm.prof[3] / S.dbg[4], S.lm.prof[4] / S.dbg[4], S.lm.prof[5] / S.dbg[4], S.lm.prof[6] / S.dbg[4]);
-#endif
   if (dbg_on) {
     S.dbg[5] = clock64() - S.dbg_t0;
     for (int k = 0; k < 6; ++k) A.debug[size_t(blockIdx.x) * 6 + k] = (unsigned long long)S.dbg[k];
@@ -544,15 +523,12 @@ __global__ void __launch_bounds__(256) ea_k_gather_probe(const __grid_constant__
 }
 
 cudaError_t ea_launch_gather_probe(const EaSolveArgs& A, int level, int slices, int repeats, float* d_sink, cudaStream_t stream) {
-  // EA_PROBE_SMEM_KB: occupancy experiment (dynamic shared memory only limits the number of resident CTAs)
-  static const int smem_kb = getenv("EA_PROBE_SMEM_KB") ? atoi(getenv("EA_PROBE_SMEM_KB")) : 0;
-  if (smem_kb > 48) cudaFuncSetAttribute(ea_k_gather_probe, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_kb * 1024);
-  ea_k_gather_probe<<<unsigned(A.n_pairs * slices), 256, size_t(smem_kb) * 1024, stream>>>(A, level, slices, repeats, d_sink);
+  ea_k_gather_probe<<<unsigned(A.n_pairs * slices), 256, 0, stream>>>(A, level, slices, repeats, d_sink);
   return cudaGetLastError();
 }
 
 // ---- host launchers -----------------------------------------------------------------------------------
-size_t ea_help_boards_bytes(int sm_count) { return size_t(sm_count) * EA_SOLVE_MIN_CTAS * sizeof(EaHelpBoard); }
+size_t ea_help_boards_bytes(int sm_count) { return size_t(sm_count) * sizeof(EaHelpBoard); }
 
 cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm_count, cudaStream_t stream) {
   if (A.n_pairs <= 0) return cudaSuccess;
@@ -568,15 +544,13 @@ cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   if (cluster_size <= 1) {
-    // persistent CTAs (EA_SOLVE_MIN_CTAS per SM) pulling pairs from the work queue
-    static const int env_ctas = getenv("EA_SOLVE_MAX_CTAS") ? atoi(getenv("EA_SOLVE_MAX_CTAS")) : 0;   // experiment knob (DESIGN.md 8)
+    // persistent CTAs (per_sm per SM) pulling pairs from the work queue
     auto grid_of = [&](const int per_sm) {
-      int max_ctas = sm_count * per_sm;
-      if (env_ctas > 0 && env_ctas < max_ctas) max_ctas = env_ctas;
+      const int max_ctas = sm_count * per_sm;
       return dim3(unsigned(A.n_pairs < max_ctas ? A.n_pairs : max_ctas));
     };
     if (!split) {
-      cfg.gridDim = grid_of(EA_SOLVE_MIN_CTAS);
+      cfg.gridDim = grid_of(1);
       cfg.numAttrs = 0;
       return cudaLaunchKernelEx(&cfg, ea_k_solve_batch<EA_SOLVE_THREADS, false>, A);
     }
@@ -598,7 +572,7 @@ cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm
     Af.coarsest = A.finest;
     Af.handoff_role = 2;
     cfg.blockDim = dim3(EA_SOLVE_THREADS);
-    cfg.gridDim = grid_of(EA_SOLVE_MIN_CTAS);
+    cfg.gridDim = grid_of(1);
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
@@ -606,7 +580,7 @@ cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm
     return cudaLaunchKernelEx(&cfg, ea_k_solve_batch<EA_SOLVE_THREADS, false>, Af);
   }
   int n_clusters = A.n_pairs;
-  const int max_clusters = (sm_count * EA_SOLVE_MIN_CTAS) / cluster_size;
+  const int max_clusters = sm_count / cluster_size;
   if (n_clusters > max_clusters) n_clusters = max_clusters;
   if (n_clusters < 1) n_clusters = 1;
   cfg.gridDim = dim3(unsigned(n_clusters * cluster_size));
@@ -642,9 +616,7 @@ cudaError_t ea_launch_eval_sums(const EaLevelDesc& rd, const EaLevelDesc& nd, co
   return cudaGetLastError();
 }
 
-#ifndef EA_ORDER_FIXED_COST
 #define EA_ORDER_FIXED_COST 8000   // measured: 0 -> 6000 -> 12000 gives 7.41 -> 7.35 -> 7.34 ms per 1184-pair launch
-#endif
 // ---- longest-first ordering for the next launch: sort pairs by the work their last solve needed -----------------
 // One CTA, bitonic sort of (work, index) in shared memory; n <= 4096.
 __global__ void __launch_bounds__(1024) ea_k_order_by_work(const ea_summary* __restrict__ summaries, int n, int n_levels, int32_t* __restrict__ order) {

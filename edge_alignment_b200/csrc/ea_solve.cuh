@@ -8,12 +8,8 @@
 
 #include "ea_device.cuh"
 
-#ifndef EA_SOLVE_THREADS
 #define EA_SOLVE_THREADS 512   // threads per CTA of every kernel built on ea_eval_slice (128 registers each: one CTA fills an SM)
-#endif
-#ifndef EA_SOLVE_COARSE_THREADS
 #define EA_SOLVE_COARSE_THREADS 256   // threads per CTA of the batched solve's coarse phase (EA_SOLVE_THREADS / this many per SM)
-#endif
 
 #define EA_CMD_EVAL 0
 #define EA_CMD_DONE 1
@@ -28,15 +24,7 @@ struct EaLmState {
   double dl_mu, dl_alpha, dl_step_norm, dl_grad[6], dl_gn[6];   // DoglegStrategy state (trust_region_strategy == 1)
   int phase, iter, accepted, rejected, invalid_run, reuse_diag, evals, term;
   int dl_reuse, pad;
-#ifdef EA_LM_PROFILE
-  long long prof[8];   // cycles per section of ea_lm_advance_warp's fast track (development aid)
-#endif
 };
-#ifdef EA_LM_PROFILE
-#define EA_LM_LAP(k) do { const long long t_ = clock64(); if (lane == 0) S.prof[k] += t_ - lm_t_; lm_t_ = t_; } while (0)
-#else
-#define EA_LM_LAP(k) do { } while (0)
-#endif
 
 __device__ inline void ea_quat_plus(const double* x, const double* d, double* out) {
   // ceres::QuaternionParameterization::Plus -- delta is a half-angle vector, left multiplication:
@@ -371,9 +359,6 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
   // (S, sums and the parameters never alias: without the qualifiers every store into S -- and there is one per state field --
   // orders the loads behind it, which serialises six clamp chains and most of the section boundaries)
   const unsigned full = 0xffffffffu;
-#ifdef EA_LM_PROFILE
-  long long lm_t_ = clock64();
-#endif
   // the serial state machine serves: the dogleg strategy, failed evaluations, rejected steps, near-tolerance decisions
   bool fast = (sp.trust_region_strategy == 0) && !(sums[27] > 0.0);
   const int phase = S.phase;
@@ -404,7 +389,6 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
     __syncwarp();
     return cmd;
   }
-  EA_LM_LAP(0);
   if (phase == 0) {
     // ---- IterationZero: the state at x0, Jacobi scaling from the first Jacobian (one sqrt + one division per lane) ----
     double mine = 1.0;
@@ -444,7 +428,6 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
   // ---- loop head of the next iteration ----
   if (iter >= sp.max_num_iterations) { if (lane == 0) { S.term = EA_TERM_NO_CONVERGENCE; S.iter = iter; S.reuse_diag = 0; } __syncwarp(); return EA_CMD_DONE; }
   if (radius < sp.min_trust_region_radius) { if (lane == 0) { S.term = EA_TERM_CONVERGENCE_MIN_RADIUS; S.iter = iter; S.reuse_diag = 0; } __syncwarp(); return EA_CMD_DONE; }
-  EA_LM_LAP(1);
   // ---- LevenbergMarquardtStrategy::ComputeStep on (S H S + diag / radius) y = S b ----
   double U[21], bs[6], y[6], delta[6];
   const double inv_radius = 1.0 / radius;
@@ -460,11 +443,9 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
   // lane j stores diag[j], recomputed from shared memory with the same operations (picking element `lane` of a register
   // array would put the array in local memory)
   if (lane < 6) S.diag[lane] = fmin(fmax(S.scale[lane] * sums[ea_tri(lane, lane)] * S.scale[lane], dg_lo), dg_hi);
-  EA_LM_LAP(2);
   bool ok = ea_ldlt_solve6_packed(U, bs, y);
 #pragma unroll
   for (int a = 0; a < 6; ++a) delta[a] = -y[a] * S.scale[a];
-  EA_LM_LAP(3);
   // model_cost_change = -(delta^T b + 1/2 delta^T H delta): the serial code's order, as six independent row chains.  The sums
   // are read from their copies in the state (S.H, S.b, as the serial code does): reading `sums` again let the compiler keep
   // the 27 values loaded for U in registers across the factorisation.
@@ -479,7 +460,6 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
   }
   const double model = -(lin + 0.5 * quad);
   ok = ok && (model > 0.0);
-  EA_LM_LAP(4);
   if (!ok) {     // HandleInvalidStep: rare; the serial loop recomputes this step, finds it invalid and carries on from there
     __syncwarp();
     int cmd = 0;
@@ -497,7 +477,6 @@ static __device__ __noinline__ int ea_lm_advance_warp(EaLmState& __restrict__ S,
     for (int i = 0; i < 7; ++i) S.cand[i] = cand[i];
   }
   __syncwarp();
-  EA_LM_LAP(5);
   return EA_CMD_EVAL;
 }
 
@@ -513,16 +492,9 @@ __device__ __forceinline__ uint2 ea_lds_u2(const unsigned saddr) {
   return v;
 }
 
-#ifndef EA_STAGE_SLOT
 #define EA_STAGE_SLOT 512   // points per staging slot (uint2 stage[2][EA_STAGE_SLOT], 8 KB, aligned to 8 KB); a power of two >= the CTA size
-#endif
 // ---- slice evaluation shared by every solve kernel ----------------------------------------------------------
-#ifndef EA_FLUSH_EVERY
 #define EA_FLUSH_EVERY 16  // points per thread between fp32 -> fp64 flushes of the normal-equation slots (measured: 8 -> 16 = -1.7 %)
-#endif
-#ifndef EA_ALTERNATE_SWEEP
-#define EA_ALTERNATE_SWEEP 1
-#endif
 
 // Per-thread accumulators of the evaluation loop between two flushes.
 struct EaEvalAcc {
@@ -748,9 +720,7 @@ __device__ __forceinline__ void ea_eval_slice(const void* __restrict__ pts, cons
 // THREADS * EA_FLUSH_EVERY, so chunk ends coincide with the fp32 -> fp64 flushes).  Every chunk is reduced on its own, in a
 // fixed order, by whichever CTA evaluates it, and the chunk totals are added in chunk order: the sums do not depend on how
 // many CTAs shared the evaluation (tail helpers, ea_solve.cu).
-#ifndef EA_MAX_CHUNKS
 #define EA_MAX_CHUNKS 4
-#endif
 __device__ __forceinline__ int ea_chunking(const int n_res, const int threads, int& size) {
   // size = unit << s with the smallest s that leaves at most EA_MAX_CHUNKS chunks (a power-of-two number of iterations per
   // chunk: the loop finds its chunk with a shift)

@@ -18,7 +18,6 @@
 // (and keep the tables of the latest solve intact for ea_tracker_probe_gather); two key tables keep K_t, which the solve
 // read, apart from K_{t+1}.
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <new>
 
@@ -299,7 +298,6 @@ static int tracker_step(ea_tracker* t, const uint8_t* d_bgr, const void* d_depth
   const int32_t* d_new_slots = policy ? t->d_new_tab[t->frame % 3] : t->d_slots[cur];
   const int fb = t->frame & 1;
   const bool overlap = input_ready != nullptr || t->inputs_ready != 0;   // frame t+1's preprocessing may run beside frame t's solve
-  static const int force_helpers = getenv("EA_TAIL_HELPERS") ? atoi(getenv("EA_TAIL_HELPERS")) : -1;   // experiment knob
   cudaStream_t ps = t->prep_stream;
   if (input_ready) {
     CU(cudaStreamWaitEvent(ps, input_ready, 0));
@@ -323,7 +321,7 @@ static int tracker_step(ea_tracker* t, const uint8_t* d_bgr, const void* d_depth
                                        t->have_order ? t->d_order : nullptr, &t->sp, t->d_summaries,
                                        // many pairs per SM and the next frame's preprocessing waiting for the SMs the solve gives
                                        // up in its tail: helpers would only keep those SMs away from it (measured: -7 % throughput)
-                                       force_helpers > 0 || (force_helpers < 0 && !(overlap && t->n_streams >= 2 * c->sm_count)));
+                                       !(overlap && t->n_streams >= 2 * c->sm_count));
     if (rc) return rc;
     if (t->n_streams > 1 && t->n_streams <= 4096) {
       cudaError_t oe = ea_launch_order_by_work(t->d_summaries, t->n_streams, t->n_levels, t->d_order, s);

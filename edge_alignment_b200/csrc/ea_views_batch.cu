@@ -21,9 +21,7 @@
 #include "ea_internal.h"
 #include "ea_solve.cuh"
 
-#ifndef VB_THREADS
 #define VB_THREADS 256
-#endif
 #define VB_MIN_CTAS 2          // 2 x 256 threads at 128 registers fill an SM; one problem's LM step overlaps the other's sweep
 #define VB_TILE_ITERS 16       // points per lane between two fp32 -> fp64 flushes (EA_FLUSH_EVERY of the production loop)
 #define VB_CMD_EXIT 2
