@@ -97,11 +97,7 @@ int ea_destroy(ea_context* c) {
             ph ? " coarse phase:" : "", c->debug_launches[ph], d[0] / n / 1e3, d[1] / n / 1e3, d[2] / n / 1e3, d[3] / n / 1e3, d[5] / n / 1e3, d[4] / n);
   }
   cudaFree(c->d_handoff); cudaFree(c->d_debug); cudaFree(c->d_boards); cudaFree(c->d_views);
-  for (int k = 0; k < EA_PREP_MAX_PARTS; ++k) {
-    if (c->prep_pipe.aux[k]) { cudaStreamSynchronize(c->prep_pipe.aux[k]); cudaStreamDestroy(c->prep_pipe.aux[k]); }
-    if (c->prep_pipe.ev_front[k]) cudaEventDestroy(c->prep_pipe.ev_front[k]);
-    if (c->prep_pipe.ev_dt[k]) cudaEventDestroy(c->prep_pipe.ev_dt[k]);
-  }
+  ea_release_prep_lanes(c);
   cudaFree(c->d_pose); cudaFree(c->d_failed); cudaFree(c->d_work); cudaFree(c->d_sums); cudaFree(c->d_idx); cudaFree(c->d_tmp);
   if (c->own_stream) cudaStreamDestroy(c->stream);
   delete c;
@@ -292,45 +288,6 @@ static int check_slots(ea_frameset* fs, int n, const int32_t* slots) {
 }
 
 }  // extern "C"
-int ea_preprocess_impl(ea_frameset* fs, int n, const int32_t* d_slots, const uint8_t* d_bgr, const void* d_depth, int roles,
-                       const uint8_t* d_mask, const uint8_t* d_now_mask, cudaStream_t stream, int in_channels, int compact,
-                       const ea_track_info* compact_gate) {
-  ea_context* c = fs->ctx;
-  if (!stream) stream = c->stream;
-  EaPrepArgs A;
-  std::memset(&A, 0, sizeof A);
-  for (int l = 0; l < fs->p.n_levels; ++l) A.lv[l] = fs->lv[l];
-  A.n_levels = fs->p.n_levels; A.slots = d_slots; A.in_bgr = d_bgr; A.in_channels = in_channels; A.in_depth = d_depth; A.in_mask = d_mask; A.in_now_mask = d_now_mask;
-  A.n_pts = fs->d_npts; A.dt_minmax = fs->d_minmax; A.dt_affine = fs->d_affine; A.overflow = fs->d_overflow;
-  A.n = n; A.roles = roles; A.grad_threshold = fs->p.grad_threshold; A.use_median = fs->p.use_median;
-  A.dt_normalize = fs->p.dt_normalize;
-  A.edge_detector = fs->p.edge_detector; A.dt_kind = fs->p.dt_kind;
-  A.canny.low = fs->p.canny_low; A.canny.high = fs->p.canny_high; A.canny.l2 = fs->p.canny_l2;
-  A.canny.on_color = (fs->p.edge_detector == EA_EDGE_CANNY_COLOR);
-  A.scratch = fs->scratch;
-  A.compact = compact; A.compact_gate = compact_gate;
-  A.depth_type = fs->p.depth_type; A.zero_to_one = fs->p.zero_depth_to_one;
-  A.depth_one = fs->p.depth_type == EA_DEPTH_F32 ? 1.0f : float(fs->p.depth_scale);
-  if (A.edge_detector != EA_EDGE_LAPLACIAN) A.use_median = 0;   // the Canny pipelines of the reference have no median step
-  int nl = 0;
-  if (!c->prep_pipe.ready && n >= 2 * c->sm_count) {      // auxiliary lanes of the preprocessing pipeline (big batches only)
-    EaPrepPipe& P = c->prep_pipe;
-    for (int k = 0; k < EA_PREP_MAX_PARTS; ++k) {
-      // (highest priority: the long-lived one-warp chamfer CTAs take the slots the short edge CTAs free, instead of queueing behind them)
-      int pr_lo = 0, pr_hi = 0;
-      CU(cudaDeviceGetStreamPriorityRange(&pr_lo, &pr_hi));
-      CU(cudaStreamCreateWithPriority(&P.aux[k], cudaStreamNonBlocking, pr_hi));
-      CU(cudaEventCreateWithFlags(&P.ev_front[k], cudaEventDisableTiming));
-      CU(cudaEventCreateWithFlags(&P.ev_dt[k], cudaEventDisableTiming));
-    }
-    P.ready = true;
-  }
-  EaProfileScope prof(c, 0, stream);
-  cudaError_t e = ea_launch_preprocess(A, c->sm_count, stream, &nl, &c->prep_pipe);
-  c->launches += nl;
-  if (e != cudaSuccess) return ea_fail(EA_ERR_CUDA, "preprocess launch: %s", cudaGetErrorString(e));
-  return EA_OK;
-}
 
 // The compaction kernel writes packed pixel points: a slot that held caller-supplied 3-D points (ea_frameset_set_points with
 // EA_POINTS_XYZ) goes back to pixel mode when it is preprocessed as a reference frame.
@@ -347,132 +304,75 @@ static int reset_points_mode(ea_frameset* fs, int n, const int32_t* slots) {
   return EA_OK;
 }
 
-extern "C" {
-int ea_frameset_preprocess_device(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* d_bgr, const void* d_depth, int roles) {
+// Behind every preprocessing entry point: checks the call, stages host buffers in the frame set (the staging area is sized for
+// BGR frames; gray frames take the first third of it), copies the slot list to the device and launches.
+static int preprocess_frames(ea_frameset* fs, int n, const int32_t* slots, int roles, EaFrameInput in) {
   int rc = check_slots(fs, n, slots);
   if (rc) return rc;
-  if (!d_bgr) return ea_fail(EA_ERR_INVALID_ARG, "bgr is null");
-  if ((roles & EA_ROLE_REF) && !d_depth) return ea_fail(EA_ERR_INVALID_ARG, "EA_ROLE_REF needs depth");
-  if (!(roles & EA_ROLE_BOTH)) return ea_fail(EA_ERR_INVALID_ARG, "roles must include EA_ROLE_REF and/or EA_ROLE_NOW");
+  if (!in.image) return ea_fail(EA_ERR_INVALID_ARG, "image is null");
+  if (roles != EA_ROLE_REF && roles != EA_ROLE_NOW && roles != EA_ROLE_BOTH)
+    return ea_fail(EA_ERR_INVALID_ARG, "roles must be EA_ROLE_REF, EA_ROLE_NOW or EA_ROLE_BOTH");
+  const bool ref = (roles & EA_ROLE_REF) != 0;
+  if (ref && !in.depth) return ea_fail(EA_ERR_INVALID_ARG, "EA_ROLE_REF needs depth");
+  if (in.ref_mask && !ref) return ea_fail(EA_ERR_INVALID_ARG, "a reference mask only applies to the reference role");
+  if (in.now_mask && !(roles & EA_ROLE_NOW)) return ea_fail(EA_ERR_INVALID_ARG, "a now mask only applies to the now role");
+  if (!ref) in.depth = nullptr;     // nothing else reads it
   ea_context* c = fs->ctx;
   CU(cudaSetDevice(c->device));
-  // slot indices travel through a private staging area so the caller's array may be reused immediately
-  int32_t* d_slots = nullptr;
-  CU(cudaMallocAsync((void**)&d_slots, size_t(n) * sizeof(int32_t), c->stream));
-  CU(cudaMemcpyAsync(d_slots, slots, size_t(n) * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-  rc = ea_preprocess_impl(fs, n, d_slots, d_bgr, d_depth, roles);
-  cudaFreeAsync(d_slots, c->stream);
-  if (rc == EA_OK && (roles & EA_ROLE_REF)) rc = reset_points_mode(fs, n, slots);
+  EaAsyncBuf d_masks(c->stream), d_slots(c->stream);      // released on every return path
+  if (in.on_host) {
+    const size_t px = size_t(fs->p.width) * fs->p.height;
+    if (!fs->stage_bgr) CU(cudaMalloc((void**)&fs->stage_bgr, px * 3 * fs->n_slots));
+    CU(cudaMemcpyAsync(fs->stage_bgr, in.image, px * in.channels * n, cudaMemcpyHostToDevice, c->stream));
+    in.image = fs->stage_bgr;
+    if (in.depth) {
+      if (!fs->stage_depth) CU(cudaMalloc(&fs->stage_depth, px * fs->depth_elem * fs->n_slots));
+      CU(cudaMemcpyAsync(fs->stage_depth, in.depth, px * fs->depth_elem * n, cudaMemcpyHostToDevice, c->stream));
+      in.depth = fs->stage_depth;
+    }
+    const int n_masks = (in.ref_mask ? 1 : 0) + (in.now_mask ? 1 : 0);
+    if (n_masks) CU(d_masks.alloc(px * n * n_masks));
+    uint8_t* m = d_masks.as<uint8_t>();
+    if (in.ref_mask) { CU(cudaMemcpyAsync(m, in.ref_mask, px * n, cudaMemcpyHostToDevice, c->stream)); in.ref_mask = m; m += px * n; }
+    if (in.now_mask) { CU(cudaMemcpyAsync(m, in.now_mask, px * n, cudaMemcpyHostToDevice, c->stream)); in.now_mask = m; }
+    in.on_host = false;
+  }
+  // the slot list goes through a buffer of the call's own, so the caller may reuse its array at once
+  CU(d_slots.alloc(size_t(n) * sizeof(int32_t)));
+  CU(cudaMemcpyAsync(d_slots.p, slots, size_t(n) * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+  rc = ea_launch_preprocess(fs, n, d_slots.as<int32_t>(), roles, in, c->stream, EA_COMPACT_INLINE, nullptr);
+  if (rc == EA_OK && ref) rc = reset_points_mode(fs, n, slots);
   return rc;
+}
+
+extern "C" {
+int ea_frameset_preprocess_host(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* bgr, const void* depth, int roles) {
+  return preprocess_frames(fs, n, slots, roles, {bgr, 3, depth, nullptr, nullptr, true});
+}
+
+int ea_frameset_preprocess_device(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* d_bgr, const void* d_depth, int roles) {
+  return preprocess_frames(fs, n, slots, roles, {d_bgr, 3, d_depth, nullptr, nullptr, false});
 }
 
 int ea_frameset_preprocess_masked(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* bgr, const void* depth,
                                   const uint8_t* mask, int roles) {
-  int rc = check_slots(fs, n, slots);
-  if (rc) return rc;
-  if (!bgr || !depth || !mask) return ea_fail(EA_ERR_INVALID_ARG, "bgr, depth and mask are required");
-  if (!(roles & EA_ROLE_REF)) return ea_fail(EA_ERR_INVALID_ARG, "a mask only applies to the reference role");
-  ea_context* c = fs->ctx;
-  CU(cudaSetDevice(c->device));
-  const size_t px = size_t(fs->p.width) * fs->p.height;
-  if (!fs->stage_bgr) CU(cudaMalloc((void**)&fs->stage_bgr, px * 3 * fs->n_slots));
-  if (!fs->stage_depth) CU(cudaMalloc((void**)&fs->stage_depth, px * fs->depth_elem * fs->n_slots));
-  EaAsyncBuf d_mask(c->stream), d_slots(c->stream);      // released on every return path
-  CU(d_mask.alloc(px * n));
-  CU(d_slots.alloc(size_t(n) * sizeof(int32_t)));
-  CU(cudaMemcpyAsync(fs->stage_bgr, bgr, px * 3 * n, cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(fs->stage_depth, depth, px * fs->depth_elem * n, cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(d_mask.p, mask, px * n, cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(d_slots.p, slots, size_t(n) * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-  rc = ea_preprocess_impl(fs, n, d_slots.as<int32_t>(), fs->stage_bgr, fs->stage_depth, roles, d_mask.as<uint8_t>());
-  if (rc == EA_OK) rc = reset_points_mode(fs, n, slots);
-  return rc;
+  if (!mask) return ea_fail(EA_ERR_INVALID_ARG, "mask is null");
+  return preprocess_frames(fs, n, slots, roles, {bgr, 3, depth, mask, nullptr, true});
 }
 
 int ea_frameset_preprocess_now_masked(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* bgr, const uint8_t* mask) {
-  int rc = check_slots(fs, n, slots);
-  if (rc) return rc;
-  if (!bgr || !mask) return ea_fail(EA_ERR_INVALID_ARG, "bgr and mask are required");
-  ea_context* c = fs->ctx;
-  CU(cudaSetDevice(c->device));
-  const size_t px = size_t(fs->p.width) * fs->p.height;
-  if (!fs->stage_bgr) CU(cudaMalloc((void**)&fs->stage_bgr, px * 3 * fs->n_slots));
-  EaAsyncBuf d_mask(c->stream), d_slots(c->stream);
-  CU(d_mask.alloc(px * n));
-  CU(d_slots.alloc(size_t(n) * sizeof(int32_t)));
-  CU(cudaMemcpyAsync(fs->stage_bgr, bgr, px * 3 * n, cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(d_mask.p, mask, px * n, cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(d_slots.p, slots, size_t(n) * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-  return ea_preprocess_impl(fs, n, d_slots.as<int32_t>(), fs->stage_bgr, nullptr, EA_ROLE_NOW, nullptr, d_mask.as<uint8_t>());
-}
-
-int ea_frameset_preprocess_host(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* bgr, const void* depth, int roles) {
-  int rc = check_slots(fs, n, slots);
-  if (rc) return rc;
-  if (!bgr) return ea_fail(EA_ERR_INVALID_ARG, "bgr is null");
-  if ((roles & EA_ROLE_REF) && !depth) return ea_fail(EA_ERR_INVALID_ARG, "EA_ROLE_REF needs depth");
-  ea_context* c = fs->ctx;
-  CU(cudaSetDevice(c->device));
-  const size_t px = size_t(fs->p.width) * fs->p.height;
-  if (!fs->stage_bgr) CU(cudaMalloc((void**)&fs->stage_bgr, px * 3 * fs->n_slots));
-  if (depth && !fs->stage_depth) CU(cudaMalloc((void**)&fs->stage_depth, px * fs->depth_elem * fs->n_slots));
-  CU(cudaMemcpyAsync(fs->stage_bgr, bgr, px * 3 * n, cudaMemcpyHostToDevice, c->stream));
-  if (depth) CU(cudaMemcpyAsync(fs->stage_depth, depth, px * fs->depth_elem * n, cudaMemcpyHostToDevice, c->stream));
-  return ea_frameset_preprocess_device(fs, n, slots, fs->stage_bgr, depth ? fs->stage_depth : nullptr, roles);
+  if (!mask) return ea_fail(EA_ERR_INVALID_ARG, "mask is null");
+  return preprocess_frames(fs, n, slots, EA_ROLE_NOW, {bgr, 3, nullptr, nullptr, mask, true});
 }
 
 // ---- 8-bit gray input: the same pipeline as on BGR (g, g, g), from a third of the bytes -----------------------------------
-static int check_gray_args(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* gray, const void* depth,
-                           const uint8_t* ref_mask, const uint8_t* now_mask, int roles) {
-  int rc = check_slots(fs, n, slots);
-  if (rc) return rc;
-  if (!gray) return ea_fail(EA_ERR_INVALID_ARG, "gray is null");
-  if (roles < EA_ROLE_REF || roles > EA_ROLE_BOTH) return ea_fail(EA_ERR_INVALID_ARG, "roles must be EA_ROLE_REF, EA_ROLE_NOW or EA_ROLE_BOTH");
-  if ((roles & EA_ROLE_REF) && !depth) return ea_fail(EA_ERR_INVALID_ARG, "EA_ROLE_REF needs depth");
-  if (ref_mask && !(roles & EA_ROLE_REF)) return ea_fail(EA_ERR_INVALID_ARG, "ref_mask only applies to the reference role");
-  if (now_mask && !(roles & EA_ROLE_NOW)) return ea_fail(EA_ERR_INVALID_ARG, "now_mask only applies to the now role");
-  return EA_OK;
+int ea_frameset_preprocess_gray_host(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* gray, const void* depth,
+                                     const uint8_t* ref_mask, const uint8_t* now_mask, int roles) {
+  return preprocess_frames(fs, n, slots, roles, {gray, 1, depth, ref_mask, now_mask, true});
 }
 
 int ea_frameset_preprocess_gray_device(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* d_gray, const void* d_depth, int roles) {
-  int rc = check_gray_args(fs, n, slots, d_gray, d_depth, nullptr, nullptr, roles);
-  if (rc) return rc;
-  ea_context* c = fs->ctx;
-  CU(cudaSetDevice(c->device));
-  EaAsyncBuf d_slots(c->stream);
-  CU(d_slots.alloc(size_t(n) * sizeof(int32_t)));
-  CU(cudaMemcpyAsync(d_slots.p, slots, size_t(n) * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-  rc = ea_preprocess_impl(fs, n, d_slots.as<int32_t>(), d_gray, d_depth, roles, nullptr, nullptr, nullptr, 1);
-  if (rc == EA_OK && (roles & EA_ROLE_REF)) rc = reset_points_mode(fs, n, slots);
-  return rc;
-}
-
-int ea_frameset_preprocess_gray_host(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* gray, const void* depth,
-                                     const uint8_t* ref_mask, const uint8_t* now_mask, int roles) {
-  int rc = check_gray_args(fs, n, slots, gray, depth, ref_mask, now_mask, roles);
-  if (rc) return rc;
-  ea_context* c = fs->ctx;
-  CU(cudaSetDevice(c->device));
-  const size_t px = size_t(fs->p.width) * fs->p.height;
-  const bool ref = (roles & EA_ROLE_REF) != 0;
-  // the staging area is sized for BGR frames; a gray frame set takes the first third of it
-  if (!fs->stage_bgr) CU(cudaMalloc((void**)&fs->stage_bgr, px * 3 * fs->n_slots));
-  if (ref && !fs->stage_depth) CU(cudaMalloc((void**)&fs->stage_depth, px * fs->depth_elem * fs->n_slots));
-  EaAsyncBuf d_masks(c->stream), d_slots(c->stream);
-  const int n_masks = (ref_mask ? 1 : 0) + (now_mask ? 1 : 0);
-  if (n_masks) CU(d_masks.alloc(px * n * n_masks));
-  CU(d_slots.alloc(size_t(n) * sizeof(int32_t)));
-  uint8_t* d_ref_mask = ref_mask ? d_masks.as<uint8_t>() : nullptr;
-  uint8_t* d_now_mask = now_mask ? d_masks.as<uint8_t>() + (ref_mask ? px * n : 0) : nullptr;
-  CU(cudaMemcpyAsync(fs->stage_bgr, gray, px * n, cudaMemcpyHostToDevice, c->stream));
-  if (ref) CU(cudaMemcpyAsync(fs->stage_depth, depth, px * fs->depth_elem * n, cudaMemcpyHostToDevice, c->stream));
-  if (ref_mask) CU(cudaMemcpyAsync(d_ref_mask, ref_mask, px * n, cudaMemcpyHostToDevice, c->stream));
-  if (now_mask) CU(cudaMemcpyAsync(d_now_mask, now_mask, px * n, cudaMemcpyHostToDevice, c->stream));
-  CU(cudaMemcpyAsync(d_slots.p, slots, size_t(n) * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-  rc = ea_preprocess_impl(fs, n, d_slots.as<int32_t>(), fs->stage_bgr, ref ? fs->stage_depth : nullptr, roles, d_ref_mask, d_now_mask,
-                          nullptr, 1);
-  if (rc == EA_OK && ref) rc = reset_points_mode(fs, n, slots);
-  return rc;
+  return preprocess_frames(fs, n, slots, roles, {d_gray, 1, d_depth, nullptr, nullptr, false});
 }
 
 static int check_slot_level(ea_frameset* fs, int slot, int level) {
@@ -682,7 +582,7 @@ int ea_eval(ea_context* c, ea_frameset* ref, int ref_slot, ea_frameset* now, int
   return EA_OK;
 }
 
-static int fill_solve_args(ea_frameset* ref, ea_frameset* now, const ea_solve_params* sp, EaSolveArgs& A, int* cluster) {
+static int fill_solve_args(ea_frameset* ref, ea_frameset* now, const ea_solve_params* sp, EaSolveArgs& A) {
   int rc = ea_check_solve_params(sp);
   if (!rc) rc = check_pairable(ref, now);
   if (rc) return rc;
@@ -696,17 +596,7 @@ static int fill_solve_args(ea_frameset* ref, ea_frameset* now, const ea_solve_pa
   for (int l = 0; l < ref->p.n_levels; ++l) { A.ref_geom[l] = ref->geom[l]; A.now_geom[l] = now->geom[l]; A.ref_cap[l] = ref->lv[l].cap; }
   A.sp = *sp;
   A.loss = ea_eval_consts(sp->loss_type, sp->loss_scale, sp->point_stride);
-  *cluster = sp->cluster_size;
   return EA_OK;
-}
-
-static int auto_cluster(ea_context* c, int n_pairs, int requested) {
-  if (requested > 0) return requested;
-  // few pairs: spread each over a cluster so the whole GPU works on them; many pairs: one CTA per pair
-  if (n_pairs * 8 <= c->sm_count) return 8;
-  if (n_pairs * 4 <= c->sm_count) return 4;
-  if (n_pairs * 2 <= c->sm_count) return 2;
-  return 1;
 }
 
 int ea_solve_batch_device(ea_context* c, int n, ea_frameset* ref, const int32_t* d_ref_slots, ea_frameset* now,
@@ -725,8 +615,7 @@ int ea_probe_gather_device(ea_context* c, int n, ea_frameset* ref, const int32_t
   ea_solve_params sp;
   ea_solve_params_default(&sp);
   EaSolveArgs A;
-  int cluster = 0;
-  int rc = fill_solve_args(ref, now, &sp, A, &cluster);
+  int rc = fill_solve_args(ref, now, &sp, A);
   if (rc) return rc;
   if (level < 0 || level >= ref->p.n_levels) return ea_fail(EA_ERR_INVALID_ARG, "level %d out of range", level);
   CU(cudaSetDevice(c->device));
@@ -762,58 +651,35 @@ int ea_solve_batch_device_ordered(ea_context* c, int n, ea_frameset* ref, const 
   if (!c || !d_ref_slots || !d_now_slots || !d_poses7) return ea_fail(EA_ERR_INVALID_ARG, "null argument");
   if (n <= 0) return EA_OK;
   EaSolveArgs A;
-  int cluster = 0;
-  int rc = fill_solve_args(ref, now, sp, A, &cluster);
+  int rc = fill_solve_args(ref, now, sp, A);
   if (rc) return rc;
   CU(cudaSetDevice(c->device));
   A.ref_slots = d_ref_slots; A.now_slots = d_now_slots; A.pose_index = d_pose_index; A.poses = d_poses7;
   A.summaries = d_summaries; A.n_pairs = n; A.work_counter = c->d_work; A.order = d_order;
-  EaProfileScope prof(c, 1);
-  cudaError_t e;
   A.trace = c->d_trace; A.trace_count = c->d_trace_count; A.trace_cap = c->trace_cap;
-  // auto (measured, DESIGN.md 4.3): few pairs -> a thread-block cluster per pair so the whole GPU works on them and the
-  // per-iteration latency drops (config 1, stride 1: 0.58 ms with clusters of 8 vs 2.4 ms on one CTA); big batches -> one
-  // persistent CTA per pair (no scheduling overhead, best L1 locality).
-  if (cluster == 0) cluster = auto_cluster(c, n, 0);
   A.debug = c->d_debug;
   // tail helpers: CTAs that find the work queue empty serve the ones still solving.  They shorten the launch, not the work:
   // a caller that has other kernels ready to take over the idle SMs (the tracker's overlapped preprocessing) turns them off.
   A.boards = tail_helpers ? static_cast<EaHelpBoard*>(c->d_boards) : nullptr;
-  // Big batches over several levels solve the coarse levels in smaller CTAs, several per SM, so that one pair's serial LM step
-  // hides behind another pair's evaluation; level `finest` keeps the full-width kernel (ea_launch_solve_batch).  The results
-  // are those of one launch over every level.
-  const bool split = cluster <= 1 && A.coarsest > A.finest && n >= 2 * c->sm_count;
-  if (split) {
-    if (c->handoff_cap < n) {
-      CU(cudaStreamSynchronize(c->stream));
-      cudaFree(c->d_handoff);
-      c->d_handoff = nullptr; c->handoff_cap = 0;
-      CU(cudaMalloc(&c->d_handoff, size_t(n) * sizeof(unsigned)));
-      CU(cudaMemsetAsync(c->d_handoff, 0, size_t(n) * sizeof(unsigned), c->stream));
-      c->handoff_cap = n;
-    }
-    A.handoff = c->d_handoff;
-    A.handoff_epoch = ++c->handoff_epoch;
-    if (A.handoff_epoch == 0) A.handoff_epoch = ++c->handoff_epoch;   // 0 is what a fresh array holds
-  }
-  e = ea_launch_solve_batch(A, cluster, c->sm_count, c->stream);
-  if (c->d_debug && e == cudaSuccess) {   // development aid: synchronous read-back of the cycle counters
-    const int grid = std::min(n, c->sm_count);
-    std::vector<unsigned long long> h(size_t(grid) * 6);
+  EaProfileScope prof(c, 1);
+  EaSolveShape shape;
+  const cudaError_t e = ea_launch_solve_batch(c, A, shape);
+  if (c->d_debug && e == cudaSuccess) {   // development aid: synchronous read-back of the cycle counters of every CTA that ran
     cudaStreamSynchronize(c->stream);
-    cudaMemcpy(h.data(), c->d_debug, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
-    for (int k = 0; k < 6; ++k) { double sum = 0; for (int b = 0; b < grid; ++b) sum += double(h[size_t(b) * 6 + k]); c->debug_sum[0][k] += sum / grid; }
-    if (split) {   // the coarse phase's rows
-      const int cgrid = std::min(n, c->sm_count * (EA_SOLVE_THREADS / EA_SOLVE_COARSE_THREADS));
-      std::vector<unsigned long long> hc(size_t(cgrid) * 6);
-      cudaMemcpy(hc.data(), c->d_debug + size_t(EA_DEBUG_ROWS) * 6, hc.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
-      for (int k = 0; k < 6; ++k) { double sum = 0; for (int b = 0; b < cgrid; ++b) sum += double(hc[size_t(b) * 6 + k]); c->debug_sum[1][k] += sum / cgrid; }
-      c->debug_launches[1]++;
+    std::vector<unsigned long long> h[2];
+    for (int ph = 0; ph < 2; ++ph) {      // {whole launch or fine phase, coarse phase}
+      const int grid = shape.grid[ph];
+      if (grid == 0) continue;
+      h[ph].resize(size_t(grid) * 6);
+      cudaMemcpy(h[ph].data(), c->d_debug + size_t(ph) * EA_DEBUG_ROWS * 6, h[ph].size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost);
+      for (int k = 0; k < 6; ++k) { double sum = 0; for (int b = 0; b < grid; ++b) sum += double(h[ph][size_t(b) * 6 + k]); c->debug_sum[ph][k] += sum / grid; }
+      if (ph == 1) c->debug_launches[1]++;
     }
     {   // owner-lifetime distribution of this launch (the launch ends with the last owner): mean / 75th / 90th percentile / max
+      const int grid = shape.grid[0];
       std::vector<double> life(static_cast<size_t>(grid));
       double mean = 0.0;
-      for (int b = 0; b < grid; ++b) { life[size_t(b)] = double(h[size_t(b) * 6 + 5]); mean += life[size_t(b)] / grid; }
+      for (int b = 0; b < grid; ++b) { life[size_t(b)] = double(h[0][size_t(b) * 6 + 5]); mean += life[size_t(b)] / grid; }
       std::sort(life.begin(), life.end());
       if (c->debug_launches[0] % 7 == 3)
         fprintf(stderr, "[EA_SOLVE_DEBUG] launch %ld: owner lifetimes (kcycles) mean %.0f  p50 %.0f  p75 %.0f  p90 %.0f  p97 %.0f  max %.0f\n", c->debug_launches[0],
@@ -821,7 +687,7 @@ int ea_solve_batch_device_ordered(ea_context* c, int n, ea_frameset* ref, const 
     }
     c->debug_launches[0]++;
   }
-  c->launches += split ? 2 : 1;
+  c->launches += shape.launches;
   if (e != cudaSuccess) return ea_fail(EA_ERR_CUDA, "solve launch: %s", cudaGetErrorString(e));
   return EA_OK;
 }

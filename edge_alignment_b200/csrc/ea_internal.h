@@ -40,10 +40,16 @@ struct EaSolveArgs {
   EaEvalConsts loss;                 // sp's loss in fp32 (ea_eval_consts), for the evaluation loop
 };
 
-// Non-cluster launches with A.handoff set and more than one level run as a coarse and a fine phase: A.work_counter then holds
-// two counters, and A.debug two blocks of EA_DEBUG_ROWS rows (fine phase first).
+// A split launch runs as a coarse and a fine phase: A.work_counter then holds two counters, and A.debug two blocks of
+// EA_DEBUG_ROWS rows (fine phase first).
 #define EA_DEBUG_ROWS 1024
-cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm_count, cudaStream_t stream);
+struct EaSolveShape {           // what ea_launch_solve_batch enqueued
+  int launches = 0;
+  int grid[2] = {0, 0};         // CTAs of {the whole launch or the fine phase, the coarse phase (0: no split)}
+};
+// Chooses the batched solve's launch shape for A.n_pairs pairs (cluster size, coarse / fine split; grows and tags the context's
+// hand-over words for a split) and enqueues it on c->stream.
+cudaError_t ea_launch_solve_batch(ea_context* c, EaSolveArgs A, EaSolveShape& shape);
 size_t ea_help_boards_bytes(int sm_count);
 cudaError_t ea_launch_gather_probe(const EaSolveArgs& A, int level, int slices, int repeats, float* d_sink, cudaStream_t stream);
 int ea_probe_gather_device(ea_context* c, int n, ea_frameset* ref, const int32_t* d_ref_slots, ea_frameset* now, const int32_t* d_now_slots,
@@ -99,16 +105,29 @@ struct EaPrepArgs {
 // EA_COMPACT_DEFER runs the edge kernels of the reference role (ref_bits and the depth pyramid in the slots) without building the
 // point lists; a later EA_COMPACT_ONLY call with the same slots and level-0 depth builds them for the frames its gate selects.
 enum { EA_COMPACT_INLINE = 0, EA_COMPACT_DEFER = 1, EA_COMPACT_ONLY = 2 };
-// enqueue the whole preprocessing pipeline for n frames; returns number of kernel launches via *launches
-// Optional second lane for big batches: the distance transforms (DRAM / latency-bound, few warps) of one part of the frames run on
-// an auxiliary stream beside the edge kernels (issue-bound) of the next part.  Streams and events belong to the context.
+// Second lane for big batches: the distance transforms (DRAM / latency-bound, few warps) of one part of the frames run on an
+// auxiliary stream beside the edge kernels (issue-bound) of the next part.  Streams and events belong to the context; the
+// preprocessing launcher creates them the first time it splits a batch, ea_release_prep_lanes destroys them.
 #define EA_PREP_MAX_PARTS 2
 struct EaPrepPipe {
   cudaStream_t aux[EA_PREP_MAX_PARTS] = {};
   cudaEvent_t ev_front[EA_PREP_MAX_PARTS] = {}, ev_dt[EA_PREP_MAX_PARTS] = {};
   bool ready = false;
 };
-cudaError_t ea_launch_preprocess(const EaPrepArgs& A, int sm_count, cudaStream_t stream, int* launches, const EaPrepPipe* pipe = nullptr);
+void ea_release_prep_lanes(ea_context* c);
+// The frames of one preprocessing call, at the frame set's level-0 geometry.
+struct EaFrameInput {
+  const uint8_t* image;         // [n][h][w][channels]
+  int channels;                 // 3: BGR; 1: gray
+  const void* depth;            // [n][h][w] of the frame set's depth_type, or null; read by the reference role only
+  const uint8_t* ref_mask;      // [n][h][w] or null: reference points only where mask > 0
+  const uint8_t* now_mask;      // [n][h][w] or null: now-frame edges only where mask > 1
+  bool on_host;                 // host buffers (staged through the frame set) rather than device buffers
+};
+// Enqueues the preprocessing of n frames into the slots d_slots[0..n) (device) on `stream` and counts its launches in the
+// context.  The inputs are device buffers (in.on_host is not read); the arguments are the caller's to validate.
+int ea_launch_preprocess(ea_frameset* fs, int n, const int32_t* d_slots, int roles, const EaFrameInput& in, cudaStream_t stream,
+                         int compact, const ea_track_info* compact_gate);
 __host__ __device__ inline float* ea_dt_origin(const EaPrepLevel& L, int slot) {   // pixel (0,0) of a slot's padded DT
   return L.dt + size_t(slot) * L.dt_slot + size_t(EA_DT_PAD) * L.dt_pitch + EA_DT_PAD;
 }
@@ -223,6 +242,3 @@ int ea_solve_batch_device_ordered(ea_context* c, int n, ea_frameset* ref, const 
                                    const int32_t* d_now_slots, double* d_poses7, const int32_t* d_pose_index,
                                    const int32_t* d_order, const ea_solve_params* sp, ea_summary* d_summaries, bool tail_helpers = true);
 cudaError_t ea_launch_order_by_work(const ea_summary* d_summaries, int n, int n_levels, int32_t* d_order, cudaStream_t stream);
-int ea_preprocess_impl(ea_frameset* fs, int n, const int32_t* d_slots, const uint8_t* d_bgr, const void* d_depth, int roles,
-                       const uint8_t* d_mask = nullptr, const uint8_t* d_now_mask = nullptr, cudaStream_t stream = nullptr,
-                       int in_channels = 3, int compact = EA_COMPACT_INLINE, const ea_track_info* compact_gate = nullptr);

@@ -8,6 +8,7 @@
 // Integer stages are bit-exact restatements of OpenCV's portable code paths (pinned in tests/golden).
 // HBM-bound byte/integer work: coalesced loads, shared-memory staging, no tensor cores.
 #include <cstdlib>
+#include <cstring>
 
 #include "ea_internal.h"
 
@@ -1136,8 +1137,53 @@ static EaPrepArgs prep_slice(const EaPrepArgs& A, int f0, int n) {
   return S;
 }
 
-cudaError_t ea_launch_preprocess(const EaPrepArgs& A, int sm_count, cudaStream_t stream, int* launches, const EaPrepPipe* pipe) {
-  int nl = 0;
+static EaPrepArgs prep_args(const ea_frameset* fs, int n, const int32_t* d_slots, int roles, const EaFrameInput& in, int compact,
+                            const ea_track_info* compact_gate) {
+  const ea_frame_params& p = fs->p;
+  EaPrepArgs A;
+  std::memset(&A, 0, sizeof A);
+  for (int l = 0; l < p.n_levels; ++l) A.lv[l] = fs->lv[l];
+  A.n_levels = p.n_levels; A.slots = d_slots; A.in_bgr = in.image; A.in_channels = in.channels; A.in_depth = in.depth;
+  A.in_mask = in.ref_mask; A.in_now_mask = in.now_mask;
+  A.n_pts = fs->d_npts; A.dt_minmax = fs->d_minmax; A.dt_affine = fs->d_affine; A.overflow = fs->d_overflow;
+  A.n = n; A.roles = roles; A.grad_threshold = p.grad_threshold; A.use_median = p.use_median;
+  A.dt_normalize = p.dt_normalize;
+  A.edge_detector = p.edge_detector; A.dt_kind = p.dt_kind;
+  A.canny.low = p.canny_low; A.canny.high = p.canny_high; A.canny.l2 = p.canny_l2;
+  A.canny.on_color = (p.edge_detector == EA_EDGE_CANNY_COLOR);
+  A.scratch = fs->scratch;
+  A.compact = compact; A.compact_gate = compact_gate;
+  A.depth_type = p.depth_type; A.zero_to_one = p.zero_depth_to_one;
+  A.depth_one = p.depth_type == EA_DEPTH_F32 ? 1.0f : float(p.depth_scale);
+  if (A.edge_detector != EA_EDGE_LAPLACIAN) A.use_median = 0;   // the Canny pipelines of the reference have no median step
+  return A;
+}
+
+// highest priority: the long-lived one-warp chamfer CTAs take the slots the short edge CTAs free, instead of queueing behind them
+static int create_lanes(EaPrepPipe& P) {
+  int pr_lo = 0, pr_hi = 0;
+  CU(cudaDeviceGetStreamPriorityRange(&pr_lo, &pr_hi));
+  for (int k = 0; k < EA_PREP_MAX_PARTS; ++k) {
+    CU(cudaStreamCreateWithPriority(&P.aux[k], cudaStreamNonBlocking, pr_hi));
+    CU(cudaEventCreateWithFlags(&P.ev_front[k], cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&P.ev_dt[k], cudaEventDisableTiming));
+  }
+  P.ready = true;
+  return EA_OK;
+}
+
+void ea_release_prep_lanes(ea_context* c) {
+  EaPrepPipe& P = c->prep_pipe;
+  for (int k = 0; k < EA_PREP_MAX_PARTS; ++k) {
+    if (P.aux[k]) { cudaStreamSynchronize(P.aux[k]); cudaStreamDestroy(P.aux[k]); }
+    if (P.ev_front[k]) cudaEventDestroy(P.ev_front[k]);
+    if (P.ev_dt[k]) cudaEventDestroy(P.ev_dt[k]);
+  }
+  P = EaPrepPipe{};
+}
+
+// the whole pipeline for A's frames; lanes: null, or the auxiliary lanes that take the distance transforms of each half
+static cudaError_t launch_pipeline(const EaPrepArgs& A, const EaPrepPipe* lanes, cudaStream_t stream, int& nl) {
   const bool want_ref = (A.roles & EA_ROLE_REF) != 0, want_now = (A.roles & EA_ROLE_NOW) != 0;
   if (want_ref && !A.in_depth) return cudaErrorInvalidValue;
   if (A.compact == EA_COMPACT_ONLY) {
@@ -1147,18 +1193,10 @@ cudaError_t ea_launch_preprocess(const EaPrepArgs& A, int sm_count, cudaStream_t
       else launch_compact<uint16_t>(A, l, stream);
       ++nl;
     }
-    if (launches) *launches = nl;
     return cudaGetLastError();
   }
-  // Two halves, two lanes: the chamfer kernel (DRAM- and latency-bound, ~40 % of the issue slots) of the first half runs beside
-  // the edge kernels (issue-bound, a sixth of the DRAM bandwidth) of the second half.  Only the Laplacian + chamfer pipeline (its
-  // work buffers are all indexed by slot), and only when both halves still fill the GPU: from 8 frames per SM (at 4 the halves
-  // no longer fill it, DESIGN.md 4.4).
-  const int split_frames_per_sm = 8;
-  const bool split = pipe && pipe->ready && want_now && A.edge_detector == EA_EDGE_LAPLACIAN && A.dt_kind != EA_DT_EXACT &&
-                     A.lv[0].w <= 32 * DTW_PMAX && A.n >= split_frames_per_sm * sm_count;
   cudaError_t e = cudaSuccess;
-  if (!split) {
+  if (!lanes) {
     e = launch_front(A, stream, nl);
     if (e == cudaSuccess && want_now) e = launch_dt(A, stream, nl);
   } else {
@@ -1169,21 +1207,43 @@ cudaError_t ea_launch_preprocess(const EaPrepArgs& A, int sm_count, cudaStream_t
       const EaPrepArgs H = prep_slice(A, f0, f1 - f0);
       e = launch_front(H, stream, nl);
       if (e != cudaSuccess) break;
-      e = cudaEventRecord(pipe->ev_front[k], stream);
-      if (e == cudaSuccess) e = cudaStreamWaitEvent(pipe->aux[k], pipe->ev_front[k], 0);
+      e = cudaEventRecord(lanes->ev_front[k], stream);
+      if (e == cudaSuccess) e = cudaStreamWaitEvent(lanes->aux[k], lanes->ev_front[k], 0);
       if (e != cudaSuccess) break;
       forked = k + 1;
-      e = launch_dt(H, pipe->aux[k], nl);
+      e = launch_dt(H, lanes->aux[k], nl);
     }
     // join, also after an error: whatever reached a lane is ordered before the caller's next work on `stream`
     for (int k = 0; k < forked; ++k) {
-      cudaError_t je = cudaEventRecord(pipe->ev_dt[k], pipe->aux[k]);
-      if (je == cudaSuccess) je = cudaStreamWaitEvent(stream, pipe->ev_dt[k], 0);
+      cudaError_t je = cudaEventRecord(lanes->ev_dt[k], lanes->aux[k]);
+      if (je == cudaSuccess) je = cudaStreamWaitEvent(stream, lanes->ev_dt[k], 0);
       if (e == cudaSuccess) e = je;
     }
   }
-  if (launches) *launches = nl;
   return e != cudaSuccess ? e : cudaGetLastError();
+}
+
+int ea_launch_preprocess(ea_frameset* fs, int n, const int32_t* d_slots, int roles, const EaFrameInput& in, cudaStream_t stream,
+                         int compact, const ea_track_info* compact_gate) {
+  ea_context* c = fs->ctx;
+  const EaPrepArgs A = prep_args(fs, n, d_slots, roles, in, compact, compact_gate);
+  // Two halves, two lanes: the chamfer kernel (DRAM- and latency-bound, ~40 % of the issue slots) of the first half runs beside
+  // the edge kernels (issue-bound, a sixth of the DRAM bandwidth) of the second half.  Only the Laplacian + chamfer pipeline (its
+  // work buffers are all indexed by slot), and only when both halves still fill the GPU: from 8 frames per SM (at 4 the halves
+  // no longer fill it, DESIGN.md 4.4).
+  const int split_frames_per_sm = 8;
+  const bool split = compact != EA_COMPACT_ONLY && (roles & EA_ROLE_NOW) && A.edge_detector == EA_EDGE_LAPLACIAN &&
+                     A.dt_kind != EA_DT_EXACT && A.lv[0].w <= 32 * DTW_PMAX && n >= split_frames_per_sm * c->sm_count;
+  if (split && !c->prep_pipe.ready) {
+    const int rc = create_lanes(c->prep_pipe);
+    if (rc) return rc;
+  }
+  int nl = 0;
+  EaProfileScope prof(c, 0, stream);
+  const cudaError_t e = launch_pipeline(A, split ? &c->prep_pipe : nullptr, stream, nl);
+  c->launches += nl;
+  if (e != cudaSuccess) return ea_fail(EA_ERR_CUDA, "preprocess launch: %s", cudaGetErrorString(e));
+  return EA_OK;
 }
 
 cudaError_t ea_launch_dt_normalized_copy(const float* origin, int pitch, const float2* affine, int w, int h, float* out, cudaStream_t stream) {

@@ -530,9 +530,37 @@ cudaError_t ea_launch_gather_probe(const EaSolveArgs& A, int level, int slices, 
 // ---- host launchers -----------------------------------------------------------------------------------
 size_t ea_help_boards_bytes(int sm_count) { return size_t(sm_count) * sizeof(EaHelpBoard); }
 
-cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm_count, cudaStream_t stream) {
+cudaError_t ea_launch_solve_batch(ea_context* c, EaSolveArgs A, EaSolveShape& shape) {
+  shape = EaSolveShape{};
   if (A.n_pairs <= 0) return cudaSuccess;
-  const bool split = A.handoff != nullptr && cluster_size <= 1 && A.coarsest > A.finest;
+  const int sm_count = c->sm_count;
+  const cudaStream_t stream = c->stream;
+  // Few pairs (measured, DESIGN.md 4.3): a thread-block cluster per pair so that the whole GPU works on them and the
+  // per-iteration latency drops (config 1, stride 1: 0.58 ms with clusters of 8 vs 2.4 ms on one CTA); many pairs: one
+  // persistent CTA per pair (no scheduling overhead, best L1 locality).
+  int cluster_size = A.sp.cluster_size;
+  if (cluster_size == 0)
+    cluster_size = A.n_pairs * 8 <= sm_count ? 8 : A.n_pairs * 4 <= sm_count ? 4 : A.n_pairs * 2 <= sm_count ? 2 : 1;
+  // Big batches over several levels solve the coarse levels in smaller CTAs, several per SM, so that one pair's serial LM step
+  // hides behind another pair's evaluation; level `finest` keeps the full-width kernel.  The results are those of one launch
+  // over every level.
+  const bool split = cluster_size <= 1 && A.coarsest > A.finest && A.n_pairs >= 2 * sm_count;
+  if (split) {
+    if (c->handoff_cap < A.n_pairs) {
+      cudaError_t e = cudaStreamSynchronize(stream);
+      if (e != cudaSuccess) return e;
+      cudaFree(c->d_handoff);
+      c->d_handoff = nullptr; c->handoff_cap = 0;
+      e = cudaMalloc(&c->d_handoff, size_t(A.n_pairs) * sizeof(unsigned));
+      if (e == cudaSuccess) e = cudaMemsetAsync(c->d_handoff, 0, size_t(A.n_pairs) * sizeof(unsigned), stream);
+      if (e != cudaSuccess) return e;
+      c->handoff_cap = A.n_pairs;
+    }
+    A.handoff = c->d_handoff;
+    A.handoff_epoch = ++c->handoff_epoch;
+    if (A.handoff_epoch == 0) A.handoff_epoch = ++c->handoff_epoch;   // 0 is what a fresh array holds
+  }
+  shape.launches = split ? 2 : 1;
   cudaError_t e = cudaMemsetAsync(A.work_counter, 0, (split ? 2 : 1) * sizeof(int), stream);
   if (e != cudaSuccess) return e;
   if (A.boards && cluster_size <= 1) {
@@ -545,12 +573,10 @@ cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm
   cudaLaunchAttribute attr[1];
   if (cluster_size <= 1) {
     // persistent CTAs (per_sm per SM) pulling pairs from the work queue
-    auto grid_of = [&](const int per_sm) {
-      const int max_ctas = sm_count * per_sm;
-      return dim3(unsigned(A.n_pairs < max_ctas ? A.n_pairs : max_ctas));
-    };
+    auto grid_of = [&](const int per_sm) { return A.n_pairs < sm_count * per_sm ? A.n_pairs : sm_count * per_sm; };
+    shape.grid[0] = grid_of(1);
     if (!split) {
-      cfg.gridDim = grid_of(1);
+      cfg.gridDim = dim3(unsigned(shape.grid[0]));
       cfg.numAttrs = 0;
       return cudaLaunchKernelEx(&cfg, ea_k_solve_batch<EA_SOLVE_THREADS, false>, A);
     }
@@ -563,8 +589,9 @@ cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm
     Ac.boards = nullptr;
     Ac.debug = A.debug ? A.debug + size_t(EA_DEBUG_ROWS) * 6 : nullptr;
     Ac.handoff_role = 1;
+    shape.grid[1] = grid_of(EA_SOLVE_THREADS / EA_SOLVE_COARSE_THREADS);
     cfg.blockDim = dim3(EA_SOLVE_COARSE_THREADS);
-    cfg.gridDim = grid_of(EA_SOLVE_THREADS / EA_SOLVE_COARSE_THREADS);
+    cfg.gridDim = dim3(unsigned(shape.grid[1]));
     cfg.numAttrs = 0;
     e = cudaLaunchKernelEx(&cfg, ea_k_solve_batch<EA_SOLVE_COARSE_THREADS, false>, Ac);
     if (e != cudaSuccess) return e;
@@ -572,7 +599,7 @@ cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm
     Af.coarsest = A.finest;
     Af.handoff_role = 2;
     cfg.blockDim = dim3(EA_SOLVE_THREADS);
-    cfg.gridDim = grid_of(1);
+    cfg.gridDim = dim3(unsigned(shape.grid[0]));
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
@@ -583,7 +610,8 @@ cudaError_t ea_launch_solve_batch(const EaSolveArgs& A, int cluster_size, int sm
   const int max_clusters = sm_count / cluster_size;
   if (n_clusters > max_clusters) n_clusters = max_clusters;
   if (n_clusters < 1) n_clusters = 1;
-  cfg.gridDim = dim3(unsigned(n_clusters * cluster_size));
+  shape.grid[0] = n_clusters * cluster_size;
+  cfg.gridDim = dim3(unsigned(shape.grid[0]));
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = unsigned(cluster_size);
   attr[0].val.clusterDim.y = 1;

@@ -308,8 +308,8 @@ static int tracker_step(ea_tracker* t, const uint8_t* d_bgr, const void* d_depth
   if (t->frame >= 3) CU(cudaStreamWaitEvent(ps, t->ev_solved[fb], 0));   // last reader of this slot set: the solve of frame - 2
   // policy mode: frames after the first build their point lists only once the policy kernel has promoted them
   const bool defer = policy && !first;
-  int rc = ea_preprocess_impl(t->fs, t->n_streams, d_new_slots, d_bgr, d_depth, roles, nullptr, nullptr, ps, t->channels,
-                              defer ? EA_COMPACT_DEFER : EA_COMPACT_INLINE);
+  const EaFrameInput in{d_bgr, t->channels, d_depth, nullptr, nullptr, false};
+  int rc = ea_launch_preprocess(t->fs, t->n_streams, d_new_slots, roles, in, ps, defer ? EA_COMPACT_DEFER : EA_COMPACT_INLINE, nullptr);
   if (rc) return rc;
   CU(cudaEventRecord(t->ev_prep[fb], ps));
   if (consumed && !defer) CU(cudaEventRecord(consumed, ps));    // the input buffers may be overwritten from here on
@@ -342,8 +342,7 @@ static int tracker_step(ea_tracker* t, const uint8_t* d_bgr, const void* d_depth
     }
     CU(cudaEventRecord(t->ev_solved[fb], s));
     if (defer) {    // the point lists of the promoted frames (the level-0 depth is still the caller's input)
-      rc = ea_preprocess_impl(t->fs, t->n_streams, d_new_slots, d_bgr, d_depth, EA_ROLE_REF, nullptr, nullptr, s, t->channels,
-                              EA_COMPACT_ONLY, t->d_info);
+      rc = ea_launch_preprocess(t->fs, t->n_streams, d_new_slots, EA_ROLE_REF, in, s, EA_COMPACT_ONLY, t->d_info);
       if (rc) return rc;
       if (consumed) CU(cudaEventRecord(consumed, s));
     }
