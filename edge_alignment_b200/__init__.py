@@ -5,7 +5,7 @@ reference's class names (include/edge_alignment/).  This Python package only bin
 It never imports oracle/ and has no CPU fallback.
 """
 from . import _lib  # noqa: F401
-from .api import (Context, EaError, FrameSet, Shard, Tracker, frame_params, pixel_points, solve_params, IDENTITY)  # noqa: F401
+from .api import (Context, EaError, FrameSet, Shard, Tracker, frame_params, image_layout, pixel_points, solve_params, IDENTITY)  # noqa: F401
 from ._lib import (STRATEGY_DOGLEG, STRATEGY_LM, LOSS_CAUCHY, LOSS_HUBER, LOSS_TRIVIAL, NORM_01, NORM_255, NORM_NONE, POINTS_PIXEL, POINTS_XYZ,  # noqa: F401
                    ROLE_BOTH, ROLE_NOW, ROLE_REF, EDGE_LAPLACIAN, EDGE_CANNY_GRAY, EDGE_CANNY_COLOR, DT_CHAMFER3, DT_EXACT, DEPTH_U16, DEPTH_F32,
-                   IMAGE_BGR8, IMAGE_GRAY8, KEY_FIRST, KEY_INTERVAL, KEY_TRANSLATION, KEY_ROTATION, KEY_COST, KEY_LOST)
+                   IMAGE_BGR8, IMAGE_GRAY8, IMAGE_NV12, IMAGE_YUYV, IMAGE_UYVY, ImageLayout, KEY_FIRST, KEY_INTERVAL, KEY_TRANSLATION, KEY_ROTATION, KEY_COST, KEY_LOST)

@@ -21,7 +21,7 @@ EDGE_LAPLACIAN, EDGE_CANNY_GRAY, EDGE_CANNY_COLOR = 0, 1, 2
 DT_CHAMFER3, DT_EXACT = 0, 1
 DEPTH_U16, DEPTH_F32 = 0, 1
 POINTS_PIXEL, POINTS_XYZ = 0, 1
-IMAGE_BGR8, IMAGE_GRAY8 = 0, 1
+IMAGE_BGR8, IMAGE_GRAY8, IMAGE_NV12, IMAGE_YUYV, IMAGE_UYVY = 0, 1, 2, 3, 4
 KEY_FIRST, KEY_INTERVAL, KEY_TRANSLATION, KEY_ROTATION, KEY_COST, KEY_LOST = 1, 2, 4, 8, 16, 32
 TERMINATION = {0: "NONE", 1: "CONVERGENCE_GRADIENT", 2: "CONVERGENCE_FUNCTION", 3: "CONVERGENCE_PARAMETER",
                4: "CONVERGENCE_MIN_RADIUS", 5: "NO_CONVERGENCE", 6: "FAILURE_EVAL_X0", 7: "FAILURE_INVALID_STEPS",
@@ -69,6 +69,10 @@ class KeyframePolicy(C.Structure):
                 ("max_rotation", C.c_double), ("max_cost_per_residual", C.c_double)]
 
 
+class ImageLayout(C.Structure):
+    _fields_ = [("format", C.c_int32), ("reserved", C.c_int32), ("row_pitch", C.c_int64), ("frame_stride", C.c_int64)]
+
+
 class TrackInfo(C.Structure):
     _fields_ = [("key_frame", C.c_int32), ("key_reasons", C.c_int32)]
 
@@ -100,6 +104,8 @@ PROTOTYPES = {
     "ea_frameset_preprocess_device": (_i, [_vp, _i, _i32p, _vp, _vp, _i]),
     "ea_frameset_preprocess_gray_host": (_i, [_vp, _i, _i32p, _vp, _vp, _vp, _vp, _i]),
     "ea_frameset_preprocess_gray_device": (_i, [_vp, _i, _i32p, _vp, _vp, _i]),
+    "ea_frameset_preprocess_image_host": (_i, [_vp, _i, _i32p, C.POINTER(ImageLayout), _vp, _vp, _vp, _vp, _i]),
+    "ea_frameset_preprocess_image_device": (_i, [_vp, _i, _i32p, C.POINTER(ImageLayout), _vp, _vp, _vp, _vp, _i]),
     "ea_frameset_set_points": (_i, [_vp, _i, _i, _f32p, _i, _i]),
     "ea_frameset_set_dt": (_i, [_vp, _i, _i, _f32p]),
     "ea_frameset_get_num_points": (_i, [_vp, _i, _i, _pi]),
@@ -122,6 +128,7 @@ PROTOTYPES = {
     "ea_tracker_step_device": (_i, [_vp, _vp, _vp]),
     "ea_tracker_set_inputs_ready": (_i, [_vp, _i]),
     "ea_tracker_set_image_format": (_i, [_vp, _i]),
+    "ea_tracker_set_image_layout": (_i, [_vp, C.POINTER(ImageLayout)]),
     "ea_tracker_probe_gather": (_i, [_vp, _i, _i, C.POINTER(C.c_float), C.POINTER(C.c_double)]),
     "ea_tracker_get_poses": (_i, [_vp, _f64p, C.POINTER(Summary)]),
     "ea_tracker_frame_index": (_i, [_vp, _pi]),

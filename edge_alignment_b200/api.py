@@ -49,6 +49,33 @@ def solve_params(**kw):
     return p
 
 
+def image_layout(fmt, row_pitch=0, frame_stride=0):
+    """ea_image_layout: format IMAGE_*, bytes from a row to the next and from a frame to the next (0 = dense)."""
+    return L.ImageLayout(format=fmt, reserved=0, row_pitch=row_pitch, frame_stride=frame_stride)
+
+
+def _image_arg(image, layout):
+    """(address, ImageLayout) of an image argument.  image: a numpy array or torch tensor [n][h][...] of u8 whose first two
+    strides are the frame stride and the row pitch (bytes within a row dense), or an address (int) with an ImageLayout.
+    layout: an ImageLayout as is, or an IMAGE_* format whose row pitch and frame stride are taken from the array."""
+    if isinstance(image, int):
+        if not isinstance(layout, L.ImageLayout):
+            raise TypeError("an image given as an address needs an ImageLayout")
+        return image, layout
+    if hasattr(image, "data_ptr"):
+        addr, shape, strides = image.data_ptr(), tuple(image.shape), [s * image.element_size() for s in image.stride()]
+    else:
+        addr, shape, strides = image.ctypes.data, image.shape, list(image.strides)
+    if isinstance(layout, L.ImageLayout):
+        return addr, layout
+    inner = 1
+    for d in range(len(shape) - 1, 1, -1):
+        if strides[d] != inner:
+            raise ValueError("the bytes of an image row must be dense (strides %s)" % (strides,))
+        inner *= shape[d]
+    return addr, image_layout(layout, strides[1], strides[0])
+
+
 class Context:
     def __init__(self, device=0):
         self._h = C.c_void_p()
@@ -251,6 +278,30 @@ class FrameSet:
         slots = np.ascontiguousarray(slots, np.int32)
         _check(L.lib().ea_frameset_preprocess_gray_device(self._h, len(slots), _ptr(slots, C.c_int32), d_gray, d_depth or None, roles))
 
+    def _dense(self, a, dtype):
+        return None if a is None else np.ascontiguousarray(a, dtype)
+
+    def preprocess_image_host(self, slots, image, layout, depth=None, roles=L.ROLE_BOTH, ref_mask=None, now_mask=None):
+        """Host frames in any ea_image_layout (NV12 / YUYV / UYVY, pitched GRAY8 / BGR8): the same results as
+        preprocess_gray_host on their luma.  image: see _image_arg (a strided array gives its own pitch and stride).
+        depth and the masks are dense [n][h][w]."""
+        slots = np.ascontiguousarray(slots, np.int32)
+        addr, lay = _image_arg(image, layout)
+        depth = self._dense(depth, np.float32 if self.params.depth_type == L.DEPTH_F32 else np.uint16)
+        ref_mask, now_mask = self._dense(ref_mask, np.uint8), self._dense(now_mask, np.uint8)
+        p = lambda a: None if a is None else a.ctypes.data
+        _check(L.lib().ea_frameset_preprocess_image_host(self._h, len(slots), _ptr(slots, C.c_int32), C.byref(lay), addr, p(depth),
+                                                         p(ref_mask), p(now_mask), roles))
+        self.ctx.sync()   # numpy buffers may be pageable and short-lived
+
+    def preprocess_image_device(self, slots, d_image, layout, d_depth=0, roles=L.ROLE_BOTH, d_ref_mask=0, d_now_mask=0):
+        """Device frames in any ea_image_layout, read where they lie.  d_image: a CUDA tensor (see _image_arg) or an address
+        with an ImageLayout; d_depth / d_ref_mask / d_now_mask: device addresses (ints) of dense [n][h][w] buffers, or 0."""
+        slots = np.ascontiguousarray(slots, np.int32)
+        addr, lay = _image_arg(d_image, layout)
+        _check(L.lib().ea_frameset_preprocess_image_device(self._h, len(slots), _ptr(slots, C.c_int32), C.byref(lay), addr,
+                                                           d_depth or None, d_ref_mask or None, d_now_mask or None, roles))
+
     def set_points(self, slot, pts4, level=0, mode=L.POINTS_PIXEL):
         pts4 = np.ascontiguousarray(pts4, np.float32).reshape(-1, 4)
         _check(L.lib().ea_frameset_set_points(self._h, slot, level, _ptr(pts4, C.c_float), len(pts4), mode))
@@ -304,6 +355,12 @@ class Tracker:
         """IMAGE_BGR8 ([n_streams][h][w][3]) or IMAGE_GRAY8 ([n_streams][h][w]) for step_host / step_device; only before the
         first step (after creation or reset)."""
         _check(L.lib().ea_tracker_set_image_format(self._h, image_format))
+
+    def set_image_layout(self, fmt, row_pitch=0, frame_stride=0):
+        """Frames of step_host / step_device in an ea_image_layout (fmt: IMAGE_*, or an ImageLayout): stream s at
+        image + s * frame_stride.  Only before the first step (after creation or reset)."""
+        lay = fmt if isinstance(fmt, L.ImageLayout) else image_layout(fmt, row_pitch, frame_stride)
+        _check(L.lib().ea_tracker_set_image_layout(self._h, C.byref(lay)))
 
     def close(self):
         if self._h:

@@ -2,6 +2,7 @@
 // multi-stream tracker.  Host C++ only orchestrates; all arithmetic of the path runs in the kernels of
 // ea_preprocess.cu / ea_solve.cu.  No CPU fallback: every entry point fails loudly without a device.
 #include <cstdarg>
+#include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <cmath>
@@ -304,12 +305,65 @@ static int reset_points_mode(ea_frameset* fs, int n, const int32_t* slots) {
   return EA_OK;
 }
 
+// ---- image layouts -------------------------------------------------------------------------------------------------------
+size_t ea_layout_row_bytes(const ea_image_layout& L, int w) {
+  static const int bpp[] = {3, 1, 1, 2, 2};   // BGR8, GRAY8, NV12 (luma), YUYV, UYVY
+  return size_t(w) * bpp[L.format];
+}
+
+int ea_resolve_layout(const ea_image_layout* in, int w, int h, bool on_device, ea_image_layout* out) {
+  if (!in) return ea_fail(EA_ERR_INVALID_ARG, "image layout is null");
+  ea_image_layout L = *in;
+  if (L.format < EA_IMAGE_BGR8 || L.format > EA_IMAGE_UYVY) return ea_fail(EA_ERR_INVALID_ARG, "unknown image format %d", L.format);
+  if (L.reserved != 0) return ea_fail(EA_ERR_INVALID_ARG, "ea_image_layout.reserved must be 0");
+  if (L.format == EA_IMAGE_NV12 && (h & 1)) return ea_fail(EA_ERR_INVALID_ARG, "NV12 frames need an even height (h = %d)", h);
+  if ((L.format == EA_IMAGE_YUYV || L.format == EA_IMAGE_UYVY) && (w & 1))
+    return ea_fail(EA_ERR_INVALID_ARG, "YUYV / UYVY frames need an even width (w = %d)", w);
+  const int64_t row = int64_t(ea_layout_row_bytes(L, w));
+  if (L.row_pitch == 0) L.row_pitch = row;
+  if (L.row_pitch < row || L.row_pitch > INT32_MAX)
+    return ea_fail(EA_ERR_INVALID_ARG, "row_pitch %lld: must be in [%lld, 2^31)", (long long)L.row_pitch, (long long)row);
+  if (L.frame_stride == 0) L.frame_stride = L.format == EA_IMAGE_NV12 ? 3 * int64_t(h) * L.row_pitch / 2 : int64_t(h) * L.row_pitch;
+  // the host path copies the frames as one 3-D copy of rows that are row_pitch apart, frames included
+  if (L.frame_stride < int64_t(h) * L.row_pitch || L.frame_stride % L.row_pitch != 0)
+    return ea_fail(EA_ERR_INVALID_ARG, "frame_stride %lld: must be a multiple of row_pitch %lld and at least h * row_pitch",
+                   (long long)L.frame_stride, (long long)L.row_pitch);
+  // the BGR kernels on device memory read dense frames only
+  if (on_device && L.format == EA_IMAGE_BGR8 && (L.row_pitch != row || L.frame_stride != int64_t(h) * row))
+    return ea_fail(EA_ERR_INVALID_ARG, "BGR8 frames in device memory must be dense");
+  *out = L;
+  return EA_OK;
+}
+
+ea_image_layout ea_staged_layout(const ea_image_layout& L, int w, int h) {
+  ea_image_layout S = L;
+  if (S.format == EA_IMAGE_NV12) S.format = EA_IMAGE_GRAY8;
+  S.row_pitch = int64_t(ea_layout_row_bytes(L, w));
+  S.frame_stride = int64_t(h) * S.row_pitch;
+  return S;
+}
+
+cudaError_t ea_upload_frames(uint8_t* dst, const uint8_t* src, const ea_image_layout& L, int w, int h, int n, cudaStream_t stream) {
+  const size_t row = ea_layout_row_bytes(L, w), pitch = size_t(L.row_pitch), rows = size_t(L.frame_stride) / pitch;
+  if (pitch == row && rows == size_t(h)) return cudaMemcpyAsync(dst, src, row * h * n, cudaMemcpyHostToDevice, stream);   // dense
+  if (rows == size_t(h))        // rows evenly spaced across frames
+    return cudaMemcpy2DAsync(dst, row, src, pitch, row, size_t(h) * n, cudaMemcpyHostToDevice, stream);
+  cudaMemcpy3DParms p = {};
+  p.srcPtr = make_cudaPitchedPtr(const_cast<uint8_t*>(src), pitch, row, rows);
+  p.dstPtr = make_cudaPitchedPtr(dst, row, row, size_t(h));
+  p.extent = make_cudaExtent(row, size_t(h), size_t(n));
+  p.kind = cudaMemcpyHostToDevice;
+  return cudaMemcpy3DAsync(&p, stream);
+}
+
 // Behind every preprocessing entry point: checks the call, stages host buffers in the frame set (the staging area is sized for
-// BGR frames; gray frames take the first third of it), copies the slot list to the device and launches.
+// BGR frames; the other formats take the first third or two of it), copies the slot list to the device and launches.
 static int preprocess_frames(ea_frameset* fs, int n, const int32_t* slots, int roles, EaFrameInput in) {
   int rc = check_slots(fs, n, slots);
   if (rc) return rc;
   if (!in.image) return ea_fail(EA_ERR_INVALID_ARG, "image is null");
+  rc = ea_resolve_layout(&in.layout, fs->p.width, fs->p.height, !in.on_host, &in.layout);
+  if (rc) return rc;
   if (roles != EA_ROLE_REF && roles != EA_ROLE_NOW && roles != EA_ROLE_BOTH)
     return ea_fail(EA_ERR_INVALID_ARG, "roles must be EA_ROLE_REF, EA_ROLE_NOW or EA_ROLE_BOTH");
   const bool ref = (roles & EA_ROLE_REF) != 0;
@@ -323,8 +377,9 @@ static int preprocess_frames(ea_frameset* fs, int n, const int32_t* slots, int r
   if (in.on_host) {
     const size_t px = size_t(fs->p.width) * fs->p.height;
     if (!fs->stage_bgr) CU(cudaMalloc((void**)&fs->stage_bgr, px * 3 * fs->n_slots));
-    CU(cudaMemcpyAsync(fs->stage_bgr, in.image, px * in.channels * n, cudaMemcpyHostToDevice, c->stream));
+    CU(ea_upload_frames(fs->stage_bgr, in.image, in.layout, fs->p.width, fs->p.height, n, c->stream));
     in.image = fs->stage_bgr;
+    in.layout = ea_staged_layout(in.layout, fs->p.width, fs->p.height);
     if (in.depth) {
       if (!fs->stage_depth) CU(cudaMalloc(&fs->stage_depth, px * fs->depth_elem * fs->n_slots));
       CU(cudaMemcpyAsync(fs->stage_depth, in.depth, px * fs->depth_elem * n, cudaMemcpyHostToDevice, c->stream));
@@ -345,34 +400,49 @@ static int preprocess_frames(ea_frameset* fs, int n, const int32_t* slots, int r
   return rc;
 }
 
+static ea_image_layout dense(int format) { return ea_image_layout{format, 0, 0, 0}; }
+
 extern "C" {
 int ea_frameset_preprocess_host(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* bgr, const void* depth, int roles) {
-  return preprocess_frames(fs, n, slots, roles, {bgr, 3, depth, nullptr, nullptr, true});
+  return preprocess_frames(fs, n, slots, roles, {bgr, dense(EA_IMAGE_BGR8), depth, nullptr, nullptr, true});
 }
 
 int ea_frameset_preprocess_device(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* d_bgr, const void* d_depth, int roles) {
-  return preprocess_frames(fs, n, slots, roles, {d_bgr, 3, d_depth, nullptr, nullptr, false});
+  return preprocess_frames(fs, n, slots, roles, {d_bgr, dense(EA_IMAGE_BGR8), d_depth, nullptr, nullptr, false});
 }
 
 int ea_frameset_preprocess_masked(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* bgr, const void* depth,
                                   const uint8_t* mask, int roles) {
   if (!mask) return ea_fail(EA_ERR_INVALID_ARG, "mask is null");
-  return preprocess_frames(fs, n, slots, roles, {bgr, 3, depth, mask, nullptr, true});
+  return preprocess_frames(fs, n, slots, roles, {bgr, dense(EA_IMAGE_BGR8), depth, mask, nullptr, true});
 }
 
 int ea_frameset_preprocess_now_masked(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* bgr, const uint8_t* mask) {
   if (!mask) return ea_fail(EA_ERR_INVALID_ARG, "mask is null");
-  return preprocess_frames(fs, n, slots, EA_ROLE_NOW, {bgr, 3, nullptr, nullptr, mask, true});
+  return preprocess_frames(fs, n, slots, EA_ROLE_NOW, {bgr, dense(EA_IMAGE_BGR8), nullptr, nullptr, mask, true});
 }
 
 // ---- 8-bit gray input: the same pipeline as on BGR (g, g, g), from a third of the bytes -----------------------------------
 int ea_frameset_preprocess_gray_host(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* gray, const void* depth,
                                      const uint8_t* ref_mask, const uint8_t* now_mask, int roles) {
-  return preprocess_frames(fs, n, slots, roles, {gray, 1, depth, ref_mask, now_mask, true});
+  return preprocess_frames(fs, n, slots, roles, {gray, dense(EA_IMAGE_GRAY8), depth, ref_mask, now_mask, true});
 }
 
 int ea_frameset_preprocess_gray_device(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* d_gray, const void* d_depth, int roles) {
-  return preprocess_frames(fs, n, slots, roles, {d_gray, 1, d_depth, nullptr, nullptr, false});
+  return preprocess_frames(fs, n, slots, roles, {d_gray, dense(EA_IMAGE_GRAY8), d_depth, nullptr, nullptr, false});
+}
+
+// ---- frames with a row pitch (NV12 / YUYV / UYVY, pitched GRAY8 / BGR8): the luma is read where it lies ---------------------
+int ea_frameset_preprocess_image_host(ea_frameset* fs, int n, const int32_t* slots, const ea_image_layout* layout, const uint8_t* image,
+                                      const void* depth, const uint8_t* ref_mask, const uint8_t* now_mask, int roles) {
+  if (!layout) return ea_fail(EA_ERR_INVALID_ARG, "image layout is null");
+  return preprocess_frames(fs, n, slots, roles, {image, *layout, depth, ref_mask, now_mask, true});
+}
+
+int ea_frameset_preprocess_image_device(ea_frameset* fs, int n, const int32_t* slots, const ea_image_layout* layout, const uint8_t* d_image,
+                                        const void* d_depth, const uint8_t* d_ref_mask, const uint8_t* d_now_mask, int roles) {
+  if (!layout) return ea_fail(EA_ERR_INVALID_ARG, "image layout is null");
+  return preprocess_frames(fs, n, slots, roles, {d_image, *layout, d_depth, d_ref_mask, d_now_mask, false});
 }
 
 static int check_slot_level(ea_frameset* fs, int slot, int level) {

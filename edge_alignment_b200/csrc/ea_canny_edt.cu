@@ -14,12 +14,13 @@ __device__ __forceinline__ int reflect101c(int i, int n) {
 __device__ __forceinline__ int clampi(int i, int n) { return i < 0 ? 0 : (i >= n ? n - 1 : i); }
 
 // cv::blur(3x3) (REFLECT_101, rounded /9) + cv::cvtColor(RGB2GRAY) on BGR data -> 8UC1   (utils.cpp:88-91)
-// CN = 1: gray input; RGB2GRAY of three equal channels is the identity, so the blurred value is the output
+// CN = 1: gray input, read where it lies (EaImage: the caller's luma at level 0); RGB2GRAY of three equal channels is the
+// identity, so the blurred value is the output
 template <int CN>
-__global__ void __launch_bounds__(256) k_box_gray(const uint8_t* __restrict__ bgr, size_t frame_stride_px, const int32_t* __restrict__ src_slots,
+__global__ void __launch_bounds__(256) k_box_gray(const EaImage src, const int32_t* __restrict__ src_slots,
                                                   uint8_t* __restrict__ gray, size_t scratch_stride_px, int w, int h) {
   const int f = blockIdx.y;
-  const uint8_t* img = bgr + (src_slots ? size_t(src_slots[f]) : size_t(f)) * frame_stride_px * CN;
+  const uint8_t* img = src.base + (src_slots ? size_t(src_slots[f]) : size_t(f)) * src.stride + src.offset;
   uint8_t* out = gray + size_t(f) * scratch_stride_px;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < w * h; i += gridDim.x * blockDim.x) {
     const int x = i % w, y = i / w;
@@ -29,7 +30,10 @@ __global__ void __launch_bounds__(256) k_box_gray(const uint8_t* __restrict__ bg
       int acc = 0;
       for (int dy = -1; dy <= 1; ++dy) {
         const int yy = reflect101c(y + dy, h);
-        for (int dx = -1; dx <= 1; ++dx) acc += img[(size_t(yy) * w + reflect101c(x + dx, w)) * CN + c];
+        for (int dx = -1; dx <= 1; ++dx) {
+          if constexpr (CN == 3) acc += img[(size_t(yy) * w + reflect101c(x + dx, w)) * CN + c];
+          else acc += img[size_t(yy) * src.pitch + size_t(reflect101c(x + dx, w)) * src.step];
+        }
       }
       ch[c] = __double2int_rn(double(acc) * (1.0 / 9.0));
     }
@@ -39,23 +43,29 @@ __global__ void __launch_bounds__(256) k_box_gray(const uint8_t* __restrict__ bg
 }
 
 // Sobel 3x3 (BORDER_REPLICATE) per channel, channel of largest magnitude (first on ties)   (canny.cpp)
+// CN = 1: one channel read where it lies (EaImage: the caller's luma at level 0, or the blurred scratch plane)
 template <int CN>
-__global__ void __launch_bounds__(256) k_canny_grad(const uint8_t* __restrict__ src, size_t src_stride_px, const int32_t* __restrict__ src_slots,
+__global__ void __launch_bounds__(256) k_canny_grad(const EaImage src, const int32_t* __restrict__ src_slots,
                                                     bool slot_indexed, int* __restrict__ mag, short2* __restrict__ dxy,
                                                     size_t scratch_stride_px, int w, int h, int l2) {
   const int f = blockIdx.y;
-  const uint8_t* img = src + ((slot_indexed && src_slots) ? size_t(src_slots[f]) : size_t(f)) * src_stride_px * CN;
+  const uint8_t* img = src.base + ((slot_indexed && src_slots) ? size_t(src_slots[f]) : size_t(f)) * src.stride + src.offset;
   int* M = mag + size_t(f) * scratch_stride_px;
   short2* G = dxy + size_t(f) * scratch_stride_px;
+  // byte of channel c of pixel (x, y)
+  auto at = [&](int x, int y, int c) -> int {
+    if constexpr (CN == 3) return img[(size_t(y) * w + x) * CN + c];
+    else return img[size_t(y) * src.pitch + size_t(x) * src.step];
+  };
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < w * h; i += gridDim.x * blockDim.x) {
     const int x = i % w, y = i / w;
     const int xm = clampi(x - 1, w), xp = clampi(x + 1, w), ym = clampi(y - 1, h), yp = clampi(y + 1, h);
     int best = -1, bdx = 0, bdy = 0;
 #pragma unroll
     for (int c = 0; c < CN; ++c) {
-      const int a = img[(size_t(ym) * w + xm) * CN + c], b = img[(size_t(ym) * w + x) * CN + c], cc = img[(size_t(ym) * w + xp) * CN + c];
-      const int d = img[(size_t(y) * w + xm) * CN + c], e = img[(size_t(y) * w + xp) * CN + c];
-      const int g = img[(size_t(yp) * w + xm) * CN + c], hh = img[(size_t(yp) * w + x) * CN + c], k = img[(size_t(yp) * w + xp) * CN + c];
+      const int a = at(xm, ym, c), b = at(x, ym, c), cc = at(xp, ym, c);
+      const int d = at(xm, y, c), e = at(xp, y, c);
+      const int g = at(xm, yp, c), hh = at(x, yp, c), k = at(xp, yp, c);
       const int dx = (cc + 2 * e + k) - (a + 2 * d + g);
       const int dy = (g + 2 * hh + k) - (a + 2 * b + cc);
       const int m = l2 ? dx * dx + dy * dy : abs(dx) + abs(dy);
@@ -251,9 +261,9 @@ __global__ void k_edt_affine(const unsigned* fminmax, const int32_t* dst_slots, 
 
 }  // namespace
 
-// Edge planes of level l by Canny.  src = BGR (or gray, A.in_channels == 1) of that level.  scratch: gray u8 | mag i32 | dxy short2 | map u8, each
-// [n][stride] with stride = level-0 pixels.
-cudaError_t ea_launch_canny_level(const EaPrepArgs& A, int l, const uint8_t* bgr, const void* depth, size_t frame_stride_px,
+// Edge planes of level l by Canny.  img = BGR (or one-channel input's luma) of that level; depth is dense, frame_stride_px pixels
+// per frame.  scratch: gray u8 | mag i32 | dxy short2 | map u8, each [n][stride] with stride = level-0 pixels.
+cudaError_t ea_launch_canny_level(const EaPrepArgs& A, int l, const EaImage& img, const void* depth, size_t frame_stride_px,
                                   bool slot_indexed, const EaCannyCfg& cfg, const EaScratch& S, cudaStream_t stream, int* launches) {
   const EaPrepLevel& L = A.lv[l];
   const int npx = L.w * L.h;
@@ -269,13 +279,14 @@ cudaError_t ea_launch_canny_level(const EaPrepArgs& A, int l, const uint8_t* bgr
   const int low = int(floor(t1)), high = int(floor(t2));
   if (cfg.on_color) {
     // on gray input the channel of largest gradient (first on ties) of (g, g, g) is g itself
-    if (A.in_channels == 1) k_canny_grad<1><<<grid, 256, 0, stream>>>(bgr, frame_stride_px, A.slots, slot_indexed, S.mag, S.dxy, S.stride, L.w, L.h, cfg.l2);
-    else k_canny_grad<3><<<grid, 256, 0, stream>>>(bgr, frame_stride_px, A.slots, slot_indexed, S.mag, S.dxy, S.stride, L.w, L.h, cfg.l2);
+    if (A.in_format != EA_IMAGE_BGR8) k_canny_grad<1><<<grid, 256, 0, stream>>>(img, A.slots, slot_indexed, S.mag, S.dxy, S.stride, L.w, L.h, cfg.l2);
+    else k_canny_grad<3><<<grid, 256, 0, stream>>>(img, A.slots, slot_indexed, S.mag, S.dxy, S.stride, L.w, L.h, cfg.l2);
     ++*launches;
   } else {
-    if (A.in_channels == 1) k_box_gray<1><<<grid, 256, 0, stream>>>(bgr, frame_stride_px, slot_indexed ? A.slots : nullptr, S.gray, S.stride, L.w, L.h);
-    else k_box_gray<3><<<grid, 256, 0, stream>>>(bgr, frame_stride_px, slot_indexed ? A.slots : nullptr, S.gray, S.stride, L.w, L.h);
-    k_canny_grad<1><<<grid, 256, 0, stream>>>(S.gray, S.stride, nullptr, false, S.mag, S.dxy, S.stride, L.w, L.h, cfg.l2);
+    if (A.in_format != EA_IMAGE_BGR8) k_box_gray<1><<<grid, 256, 0, stream>>>(img, slot_indexed ? A.slots : nullptr, S.gray, S.stride, L.w, L.h);
+    else k_box_gray<3><<<grid, 256, 0, stream>>>(img, slot_indexed ? A.slots : nullptr, S.gray, S.stride, L.w, L.h);
+    const EaImage blurred{S.gray, S.stride, size_t(L.w), 1, 0};
+    k_canny_grad<1><<<grid, 256, 0, stream>>>(blurred, nullptr, false, S.mag, S.dxy, S.stride, L.w, L.h, cfg.l2);
     *launches += 2;
   }
   k_canny_nms<<<grid, 256, 0, stream>>>(S.mag, S.dxy, S.map, S.stride, L.w, L.h, low, high);

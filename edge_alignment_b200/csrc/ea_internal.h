@@ -83,9 +83,11 @@ struct EaPrepArgs {
   EaPrepLevel lv[EA_MAX_LEVELS];
   int n_levels;
   const int32_t* slots;         // [n] device: destination slot of frame i
-  const uint8_t* in_bgr;        // [n][h0][w0][in_channels]
-  int in_channels;              // 3: BGR; 1: gray, preprocessed exactly as BGR (g, g, g) would be
-  const void* in_depth;         // [n][h0][w0] u16 raw units or f32 metres (depth_type), or null
+  const uint8_t* in_img;        // frame i's level-0 image at in_img + i * in_stride, its row y at + y * in_pitch (bytes)
+  int in_format;                // EA_IMAGE_BGR8 (dense [h0][w0][3]); EA_IMAGE_GRAY8 (luma plane: gray, NV12); EA_IMAGE_YUYV / _UYVY
+                                // (packed 4:2:2, luma read in place).  One-channel input is preprocessed exactly as BGR (g, g, g)
+  size_t in_pitch, in_stride;
+  const void* in_depth;        // [n][h0][w0] u16 raw units or f32 metres (depth_type), or null
   const uint8_t* in_mask;       // [n][h0][w0] or null: reference points only where mask > 0 (get_aX_mask, utils.cpp:283-369)
   const uint8_t* in_now_mask;   // [n][h0][w0] or null: now-frame edges only where mask > 1 (get_distance_transform2_masked, utils.cpp:124-128)
   int* n_pts;                   // [slots][EA_MAX_LEVELS]
@@ -115,11 +117,35 @@ struct EaPrepPipe {
   bool ready = false;
 };
 void ea_release_prep_lanes(ea_context* c);
+// Where the bytes of a level's image lie: channel c of pixel (x, y) of frame (or slot) f at
+// base[f * stride + y * pitch + x * step + offset + c].  Level 0 is the caller's image where it lies (GRAY8 / NV12: step 1; YUYV:
+// step 2, offset 0; UYVY: step 2, offset 1; BGR: dense, step 3); the pyramid pools above it are dense.
+struct EaImage {
+  const uint8_t* base;
+  size_t stride, pitch;
+  int step, offset;
+};
+inline EaImage ea_level_image(const EaPrepArgs& A, int l) {
+  const int cn = A.in_format == EA_IMAGE_BGR8 ? 3 : 1;
+  if (l > 0) { const EaPrepLevel& L = A.lv[l]; return {L.bgr, size_t(L.w) * L.h * cn, size_t(L.w) * cn, cn, 0}; }
+  const bool packed = A.in_format == EA_IMAGE_YUYV || A.in_format == EA_IMAGE_UYVY;
+  return {A.in_img, A.in_stride, A.in_pitch, packed ? 2 : cn, A.in_format == EA_IMAGE_UYVY ? 1 : 0};
+}
+// ---- image layouts (ea_image_layout, ea_cabi.cu) ----
+// Checks `in` for frames of w x h and fills `out` with its row pitch and frame stride made explicit.  on_device: the layout
+// describes device memory, where BGR8 must be dense.
+int ea_resolve_layout(const ea_image_layout* in, int w, int h, bool on_device, ea_image_layout* out);
+size_t ea_layout_row_bytes(const ea_image_layout& L, int w);   // bytes of a row the kernels read: 3w, w, w, 2w, 2w
+// The layout of frames that ea_upload_frames has packed dense: NV12 becomes GRAY8 (its luma plane).
+ea_image_layout ea_staged_layout(const ea_image_layout& L, int w, int h);
+// Copies the rows the kernels read of n host frames in layout L to dst, packed dense, in one copy on `stream`.
+cudaError_t ea_upload_frames(uint8_t* dst, const uint8_t* src, const ea_image_layout& L, int w, int h, int n, cudaStream_t stream);
+
 // The frames of one preprocessing call, at the frame set's level-0 geometry.
 struct EaFrameInput {
-  const uint8_t* image;         // [n][h][w][channels]
-  int channels;                 // 3: BGR; 1: gray
-  const void* depth;            // [n][h][w] of the frame set's depth_type, or null; read by the reference role only
+  const uint8_t* image;         // frame i at image + i * layout.frame_stride
+  ea_image_layout layout;       // resolved (ea_resolve_layout): row_pitch and frame_stride in bytes
+  const void* depth;           // [n][h][w] of the frame set's depth_type, or null; read by the reference role only
   const uint8_t* ref_mask;      // [n][h][w] or null: reference points only where mask > 0
   const uint8_t* now_mask;      // [n][h][w] or null: now-frame edges only where mask > 1
   bool on_host;                 // host buffers (staged through the frame set) rather than device buffers
@@ -134,7 +160,7 @@ __host__ __device__ inline float* ea_dt_origin(const EaPrepLevel& L, int slot) {
 cudaError_t ea_launch_dt_normalized_copy(const float* origin, int pitch, const float2* affine, int w, int h, float* out, cudaStream_t stream);
 cudaError_t ea_launch_dt_import(const float* src, float* origin, int w, int h, int pitch, cudaStream_t stream);
 cudaError_t ea_launch_dt_fill_pad(const EaPrepLevel& L, const int32_t* d_slots, int n, cudaStream_t stream);
-cudaError_t ea_launch_canny_level(const EaPrepArgs& A, int l, const uint8_t* bgr, const void* depth, size_t frame_stride_px,
+cudaError_t ea_launch_canny_level(const EaPrepArgs& A, int l, const EaImage& img, const void* depth, size_t frame_stride_px,
                                   bool slot_indexed, const EaCannyCfg& cfg, const EaScratch& S, cudaStream_t stream, int* launches);
 cudaError_t ea_launch_exact_edt_level(const EaPrepArgs& A, int l, const EaScratch& S, cudaStream_t stream, int* launches);
 cudaError_t ea_launch_unpack_mask(const uint32_t* bits, int w, int h, int words, int median, uint8_t* out,
@@ -188,7 +214,7 @@ struct ea_frameset {
   unsigned* d_minmax = nullptr;
   float2* d_affine = nullptr;             // [n_slots][EA_MAX_LEVELS]
   int* d_overflow = nullptr;
-  uint8_t* stage_bgr = nullptr;           // [n_slots][h][w][3]  (host-upload staging; gray frames use its first third)
+  uint8_t* stage_bgr = nullptr;           // [n_slots][h][w][3]  (host-upload staging; other formats use the first 1 or 2 thirds)
   void* stage_depth = nullptr;
   size_t depth_elem = 2;                  // bytes per depth sample (2: u16, 4: f32)
   double inv_depth_unit = 1.0 / 5000.0;   // metres per stored depth unit

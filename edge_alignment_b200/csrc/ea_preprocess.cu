@@ -21,43 +21,61 @@ __device__ __forceinline__ int reflect101(int i, int n) {
 }
 
 // ---- pyramid: cv::resize(0.5) INTER_LINEAR on BGR or gray (== 2x2 mean, +2 >> 2, per channel), INTER_NEAREST on depth
-// CN: channels of the image (3: BGR, 1: gray)
+// CN: channels of the image (3: BGR, 1: gray).  A one-channel source is read where it lies (EaImage: the caller's luma at level
+// 0); the depth source is dense, src_frame_stride_px pixels per frame.
 template <typename D, int CN>
-__global__ void __launch_bounds__(256) k_pyr_down(const uint8_t* __restrict__ src_bgr, const D* __restrict__ src_depth,
+__global__ void __launch_bounds__(256) k_pyr_down(const EaImage src, const D* __restrict__ src_depth,
                                                   size_t src_frame_stride_px, const int32_t* __restrict__ src_slots,
                                                   uint8_t* __restrict__ dst_bgr, D* __restrict__ dst_depth,
                                                   const int32_t* __restrict__ dst_slots, int sw, int sh) {
   const int dw = sw >> 1, dh = sh >> 1;
   const int f = blockIdx.y;
-  const size_t sbase = (src_slots ? size_t(src_slots[f]) : size_t(f)) * src_frame_stride_px;
+  const size_t sf = src_slots ? size_t(src_slots[f]) : size_t(f);
+  const size_t sbase = sf * src_frame_stride_px;
   const size_t dbase = size_t(dst_slots[f]) * size_t(dw) * dh;
+  const uint8_t* src_bgr = src.base;
+  const uint8_t* fr = src.base + sf * src.stride + src.offset;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < dw * dh; i += gridDim.x * blockDim.x) {
     const int x = i % dw, y = i / dw;
-    const uint8_t* p = src_bgr + (sbase + size_t(2 * y) * sw + 2 * x) * CN;
-    const uint8_t* q = p + size_t(sw) * CN;
     uint8_t* d = dst_bgr + (dbase + i) * CN;
+    if constexpr (CN == 3) {
+      const uint8_t* p = src_bgr + (sbase + size_t(2 * y) * sw + 2 * x) * CN;
+      const uint8_t* q = p + size_t(sw) * CN;
 #pragma unroll
-    for (int c = 0; c < CN; ++c) d[c] = uint8_t((p[c] + p[CN + c] + q[c] + q[CN + c] + 2) >> 2);
+      for (int c = 0; c < CN; ++c) d[c] = uint8_t((p[c] + p[CN + c] + q[c] + q[CN + c] + 2) >> 2);
+    } else {
+      const uint8_t* p = fr + size_t(2 * y) * src.pitch + size_t(2 * x) * src.step;
+      const uint8_t* q = p + src.pitch;
+      d[0] = uint8_t((p[0] + p[src.step] + q[0] + q[src.step] + 2) >> 2);
+    }
     if (src_depth) dst_depth[dbase + i] = src_depth[sbase + size_t(2 * y) * sw + 2 * x];
   }
 }
 
 // Same arithmetic, four output pixels per thread: 2 x 8 CN source bytes as 8-byte loads, 4 CN result bytes as 4-byte stores
 // (the byte-per-load version above moves 3.3 TB/s on BGR; frames whose rows allow it take this one).  Needs dw % 4 == 0 and
-// 8-byte aligned frame bases.
+// 8-byte aligned frame bases; one-channel input: planar, with 8-byte aligned rows.
 template <typename D, int CN>
-__global__ void __launch_bounds__(256) k_pyr_down4(const uint8_t* __restrict__ src_bgr, const D* __restrict__ src_depth,
+__global__ void __launch_bounds__(256) k_pyr_down4(const EaImage src, const D* __restrict__ src_depth,
                                                    size_t src_frame_stride_px, const int32_t* __restrict__ src_slots,
                                                    uint8_t* __restrict__ dst_bgr, D* __restrict__ dst_depth,
                                                    const int32_t* __restrict__ dst_slots, int sw, int sh) {
   const int dw = sw >> 1, dh = sh >> 1, qw = dw >> 2;
   const int f = blockIdx.y;
-  const size_t sbase = (src_slots ? size_t(src_slots[f]) : size_t(f)) * src_frame_stride_px;
+  const size_t sf = src_slots ? size_t(src_slots[f]) : size_t(f);
+  const size_t sbase = sf * src_frame_stride_px;
   const size_t dbase = size_t(dst_slots[f]) * size_t(dw) * dh;
+  const uint8_t* src_bgr = src.base;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < qw * dh; i += gridDim.x * blockDim.x) {
     const int xq = i % qw, y = i / qw;
-    const uint2* p = reinterpret_cast<const uint2*>(src_bgr + (sbase + size_t(2 * y) * sw + size_t(8 * xq)) * CN);
-    const uint2* q = reinterpret_cast<const uint2*>(src_bgr + (sbase + size_t(2 * y + 1) * sw + size_t(8 * xq)) * CN);
+    const uint2 *p, *q;
+    if constexpr (CN == 3) {
+      p = reinterpret_cast<const uint2*>(src_bgr + (sbase + size_t(2 * y) * sw + size_t(8 * xq)) * CN);
+      q = reinterpret_cast<const uint2*>(src_bgr + (sbase + size_t(2 * y + 1) * sw + size_t(8 * xq)) * CN);
+    } else {
+      p = reinterpret_cast<const uint2*>(src.base + sf * src.stride + size_t(2 * y) * src.pitch + size_t(8 * xq));
+      q = reinterpret_cast<const uint2*>(reinterpret_cast<const uint8_t*>(p) + src.pitch);
+    }
     union { uint2 v[CN]; unsigned char b[8 * CN]; } a, c;
 #pragma unroll
     for (int k = 0; k < CN; ++k) { a.v[k] = __ldg(p + k); c.v[k] = __ldg(q + k); }
@@ -82,15 +100,19 @@ __global__ void __launch_bounds__(256) k_pyr_down4(const uint8_t* __restrict__ s
 // three equal channels is the identity: 9798 + 19235 + 3735 == 1 << 15).
 #define ET_W 32
 #define ET_H 8
+// CN = 1: the image is read where it lies (EaImage); depth is dense, frame_stride_px pixels per frame.
 template <typename D, int CN>
-__global__ void __launch_bounds__(256) k_edge_mask(const uint8_t* __restrict__ bgr, const D* __restrict__ depth,
+__global__ void __launch_bounds__(256) k_edge_mask(const EaImage img, const D* __restrict__ depth,
                                                    size_t frame_stride_px, const int32_t* __restrict__ src_slots,
                                                    const int32_t* __restrict__ dst_slots, uint32_t* __restrict__ edge_bits,
                                                    uint32_t* __restrict__ ref_bits, int w, int h, int words, int thresh, int zero_to_one) {
   __shared__ uint8_t tile[ET_H + 4][(ET_W + 4) * CN + 4];
   __shared__ uint8_t gray[ET_H + 2][ET_W + 2 + 2];
   const int f = blockIdx.z;
-  const size_t sbase = (src_slots ? size_t(src_slots[f]) : size_t(f)) * frame_stride_px;
+  const size_t sf = src_slots ? size_t(src_slots[f]) : size_t(f);
+  const size_t sbase = sf * frame_stride_px;
+  const uint8_t* bgr = img.base;
+  const uint8_t* fr = img.base + sf * img.stride + img.offset;
   const int x0 = blockIdx.x * ET_W, y0 = blockIdx.y * ET_H;
   const int tid = threadIdx.y * ET_W + threadIdx.x;
   // stage the tile with a 2-pixel halo; outside the image map through REFLECT_101 (the composition of the
@@ -99,7 +121,8 @@ __global__ void __launch_bounds__(256) k_edge_mask(const uint8_t* __restrict__ b
     const int row = i / ((ET_W + 4) * CN), b = i % ((ET_W + 4) * CN);
     const int px = b / CN, c = b % CN;
     const int gx = reflect101(x0 - 2 + px, w), gy = reflect101(y0 - 2 + row, h);
-    tile[row][b] = bgr[(sbase + size_t(gy) * w + gx) * CN + c];
+    if constexpr (CN == 3) tile[row][b] = bgr[(sbase + size_t(gy) * w + gx) * CN + c];
+    else tile[row][b] = fr[size_t(gy) * img.pitch + size_t(gx) * img.step];
   }
   __syncthreads();
   for (int i = tid; i < (ET_H + 2) * (ET_W + 2); i += 256) {
@@ -320,10 +343,16 @@ __global__ void __launch_bounds__(TW) k_edge_mask2(const uint8_t* __restrict__ b
 // RGB2GRAY of three equal blurred channels is the identity (9798 + 19235 + 3735 == 1 << 15, rounding constant half of it), so
 // the blur goes straight into the gray tile.  The byte tile is staged REFLECT_101-padded (columns outside the image hold their
 // mirror image), which makes every gray column -- the two halo columns too -- a contiguous 3-tap window: each thread blurs two
-// adjacent columns in 16-bit lanes over one half of the tile's rows.  Phase 3 is k_edge_mask2's.  Needs w % 4 == 0 and a
-// 4-byte aligned image (32-bit row loads, 4 pixels each).
-template <typename D, int TW, bool REF>
-__global__ void __launch_bounds__(TW) k_edge_mask2_gray(const uint8_t* __restrict__ src, const D* __restrict__ depth,
+// adjacent columns in 16-bit lanes over one half of the tile's rows.  Phase 3 is k_edge_mask2's.  Needs w % 4 == 0.
+// LUMA: where the luma bytes lie in the rows (img_pitch bytes apart; frames img_stride bytes apart; depth stays dense).
+//   EA_LUMA_PLANAR  one byte per pixel (gray, the Y plane of NV12): 32-bit row loads, 4-byte aligned image, pitch and stride
+//   EA_LUMA_YUYV    packed 4:2:2, Y at byte 2x (Y0 U Y1 V): one 8-byte load per 4 pixels, 8-byte aligned image, pitch, stride
+//   EA_LUMA_UYVY    packed 4:2:2, Y at byte 2x + 1 (U Y0 V Y1): likewise
+// Only phase 1 depends on it: the staged tile holds the same luma bytes in every layout.
+enum { EA_LUMA_PLANAR = 0, EA_LUMA_YUYV = 1, EA_LUMA_UYVY = 2 };
+template <typename D, int TW, bool REF, int LUMA>
+__global__ void __launch_bounds__(TW) k_edge_mask2_gray(const uint8_t* __restrict__ src, size_t img_stride, unsigned img_pitch,
+                                                          const D* __restrict__ depth,
                                                           size_t frame_stride_px, const int32_t* __restrict__ src_slots,
                                                           const int32_t* __restrict__ dst_slots, uint32_t* __restrict__ edge_bits,
                                                           uint32_t* __restrict__ ref_bits, int w, int h, int words, int thresh, int zero_to_one,
@@ -334,14 +363,17 @@ __global__ void __launch_bounds__(TW) k_edge_mask2_gray(const uint8_t* __restric
   constexpr int RS = TW / NG;         // tile rows staged per pass
   constexpr int NP = (TW + 2) / 2;    // gray column pairs, halo columns included
   constexpr int H2 = (E2_TH + 2) / 2; // gray rows per half
+  constexpr int STEP = LUMA == EA_LUMA_PLANAR ? 1 : 2, OFF = LUMA == EA_LUMA_UYVY ? 1 : 0;
   __shared__ __align__(16) uint8_t tile[E2_PH][PW];
   __shared__ __align__(16) uint8_t gray[E2_TH + 2][GW];
   const int f = blockIdx.z;
-  const size_t sbase = (src_slots ? size_t(src_slots[f]) : size_t(f)) * frame_stride_px;
+  const size_t sf = src_slots ? size_t(src_slots[f]) : size_t(f);
+  const size_t sbase = sf * frame_stride_px;
   const int x0 = blockIdx.x * TW, y0 = blockIdx.y * E2_TH;
   const int t = threadIdx.x;
-  const uint8_t* img = src + sbase;
-  // ---- phase 1: one 32-bit load = 4 pixels; groups outside the image are gathered through REFLECT_101 byte by byte ----
+  const uint8_t* img = src + sf * img_stride;
+  // ---- phase 1: one 32-bit (planar) or 64-bit (packed) load = 4 pixels; groups outside the image are gathered through
+  //      REFLECT_101 byte by byte ----
   {
     const int g = t % NG, rr = t / NG;
     const int col = x0 - 4 + 4 * g;                       // first image column of the group (multiple of 4)
@@ -355,10 +387,19 @@ __global__ void __launch_bounds__(TW) k_edge_mask2_gray(const uint8_t* __restric
         if (y > h + 1) break;
         int ry = abs(y);
         ry = ry >= h ? 2 * h - 2 - ry : ry;
-        const uint8_t* row = img + size_t(unsigned(ry) * unsigned(w));
+        const uint8_t* row = img + size_t(unsigned(ry)) * img_pitch;
         unsigned v;
-        if (inside) v = __ldg(reinterpret_cast<const unsigned*>(row + col));
-        else v = unsigned(row[m0]) | unsigned(row[m1]) << 8 | unsigned(row[m2]) << 16 | unsigned(row[m3]) << 24;
+        if (inside) {
+          if constexpr (LUMA == EA_LUMA_PLANAR) {
+            v = __ldg(reinterpret_cast<const unsigned*>(row + col));
+          } else {
+            const uint2 q = __ldg(reinterpret_cast<const uint2*>(row + 2 * col));
+            v = __byte_perm(q.x, q.y, LUMA == EA_LUMA_YUYV ? 0x6420 : 0x7531);
+          }
+        } else {
+          v = unsigned(row[STEP * m0 + OFF]) | unsigned(row[STEP * m1 + OFF]) << 8 | unsigned(row[STEP * m2 + OFF]) << 16 |
+              unsigned(row[STEP * m3 + OFF]) << 24;
+        }
         *reinterpret_cast<unsigned*>(&tile[r][4 * g]) = v;
       }
     }
@@ -981,10 +1022,13 @@ __global__ void __launch_bounds__(256) k_unpack_mask(const uint32_t* __restrict_
 
 }  // namespace
 
-// the gray edge kernel loads whole 32-bit words of level l's image: a caller's device pointer that is not 4-byte aligned takes the
-// byte path (k_edge_mask) instead
+// the gray edge kernel loads whole 32-bit words (planar) or 64-bit words (packed 4:2:2) of level l's image: a caller's image whose
+// address, row pitch or frame stride is not 4- / 8-byte aligned takes the byte path (k_edge_mask) instead
 static bool gray_words_ok(const EaPrepArgs& A, int l) {
-  return A.in_channels != 1 || (reinterpret_cast<uintptr_t>(l == 0 ? A.in_bgr : A.lv[l].bgr) & 3) == 0;
+  if (A.in_format == EA_IMAGE_BGR8) return true;
+  const EaImage m = ea_level_image(A, l);
+  const uintptr_t align = m.step == 1 ? 3 : 7;
+  return ((reinterpret_cast<uintptr_t>(m.base) | m.stride | m.pitch) & align) == 0;
 }
 // can level l's Laplacian edge kernel (k_edge_mask2 / k_edge_mask2_gray) also emit level l + 1's image / depth from its staged
 // tile?  (Both store whole 32-bit words of level l + 1: 4 BGR pixels in 3 words, or 4 gray pixels in one; next level's width a
@@ -996,14 +1040,21 @@ static bool edge_kernel_fuses_pyramid(const EaPrepArgs& A, int l) {
   return (L.w & 3) == 0 && L.w >= 8 && L.h >= 4 && gray_words_ok(A, l) && (N.w & 3) == 0 && (reinterpret_cast<uintptr_t>(N.bgr) & 3) == 0;
 }
 
-// the fused edge kernel of one level for CN-channel input (k_edge_mask2 on BGR, k_edge_mask2_gray on gray)
+// the fused edge kernel of one level (k_edge_mask2 on BGR, k_edge_mask2_gray in the luma layout of one-channel input)
 template <typename D, int TW, bool REF>
-static void launch_edge_mask2(const EaPrepArgs& A, const EaPrepLevel& L, const uint8_t* b, const D* d, size_t pxl, const int32_t* ss,
+static void launch_edge_mask2(const EaPrepArgs& A, const EaPrepLevel& L, const EaImage& m, const D* d, size_t pxl, const int32_t* ss,
                               uint8_t* nb, D* nd, cudaStream_t stream) {
   dim3 grid(unsigned((L.w + TW - 1) / TW), unsigned((L.h + E2_TH - 1) / E2_TH), unsigned(A.n));
   uint32_t* rb = REF ? L.ref_bits : nullptr;
-  if (A.in_channels == 1) k_edge_mask2_gray<D, TW, REF><<<grid, TW, 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
-  else k_edge_mask2<D, TW, REF><<<grid, TW, 0, stream>>>(b, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
+  const unsigned pitch = unsigned(m.pitch);
+  if (A.in_format == EA_IMAGE_BGR8)
+    k_edge_mask2<D, TW, REF><<<grid, TW, 0, stream>>>(m.base, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
+  else if (m.step == 1)
+    k_edge_mask2_gray<D, TW, REF, EA_LUMA_PLANAR><<<grid, TW, 0, stream>>>(m.base, m.stride, pitch, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
+  else if (m.offset == 0)
+    k_edge_mask2_gray<D, TW, REF, EA_LUMA_YUYV><<<grid, TW, 0, stream>>>(m.base, m.stride, pitch, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
+  else
+    k_edge_mask2_gray<D, TW, REF, EA_LUMA_UYVY><<<grid, TW, 0, stream>>>(m.base, m.stride, pitch, d, pxl, ss, A.slots, L.edge_bits, rb, L.w, L.h, L.words, A.grad_threshold, A.zero_to_one, nb, nd);
 }
 
 // the point lists of one level from the ref_bits plane and the depth (level 0: the caller's input by frame; above: the slot's pyramid)
@@ -1019,7 +1070,7 @@ static void launch_compact(const EaPrepArgs& A, int l, cudaStream_t stream) {
 template <typename D>
 static cudaError_t launch_edges_and_points(const EaPrepArgs& A, cudaStream_t stream, int& nl) {
   const bool want_ref = (A.roles & EA_ROLE_REF) != 0;
-  const bool gray = A.in_channels == 1;
+  const bool gray = A.in_format != EA_IMAGE_BGR8;
   const size_t px0 = size_t(A.lv[0].w) * A.lv[0].h;
   const D* in_depth = static_cast<const D*>(A.in_depth);
   for (int l = 0; l < A.n_levels; ++l) {
@@ -1027,12 +1078,14 @@ static cudaError_t launch_edges_and_points(const EaPrepArgs& A, cudaStream_t str
     const size_t pxl = size_t(L.w) * L.h;
     if (l > 0 && !edge_kernel_fuses_pyramid(A, l - 1)) {      // (otherwise level l - 1's edge kernel has already written this level)
       const EaPrepLevel& S = A.lv[l - 1];
-      const uint8_t* sb = (l == 1) ? A.in_bgr : S.bgr;
+      const EaImage sb = ea_level_image(A, l - 1);
       const D* sd = want_ref ? ((l == 1) ? in_depth : static_cast<const D*>(S.depth)) : nullptr;
       const size_t sstride = (l == 1) ? px0 : size_t(S.w) * S.h;
       const int32_t* sslots = (l == 1) ? nullptr : A.slots;
       D* dd = static_cast<D*>(L.depth);
-      const bool vec4 = ((L.w & 3) == 0) && ((reinterpret_cast<uintptr_t>(sb) & 7) == 0) && ((reinterpret_cast<uintptr_t>(L.bgr) & 3) == 0);
+      // one-channel input: planar rows that are 8-byte aligned (packed 4:2:2 takes the byte kernel)
+      const bool vec4 = ((L.w & 3) == 0) && ((reinterpret_cast<uintptr_t>(sb.base) & 7) == 0) && ((reinterpret_cast<uintptr_t>(L.bgr) & 3) == 0) &&
+                        (!gray || (sb.step == 1 && ((sb.stride | sb.pitch) & 7) == 0));
       if (vec4) {
         dim3 grid(unsigned((pxl / 4 + 255) / 256), unsigned(A.n));
         if (gray) k_pyr_down4<D, 1><<<grid, 256, 0, stream>>>(sb, sd, sstride, sslots, L.bgr, dd, A.slots, S.w, S.h);
@@ -1044,7 +1097,7 @@ static cudaError_t launch_edges_and_points(const EaPrepArgs& A, cudaStream_t str
       }
       ++nl;
     }
-    const uint8_t* b = (l == 0) ? A.in_bgr : L.bgr;
+    const EaImage b = ea_level_image(A, l);
     const D* d = want_ref ? ((l == 0) ? in_depth : static_cast<const D*>(L.depth)) : nullptr;
     const int32_t* ss = (l == 0) ? nullptr : A.slots;
     if (A.edge_detector != EA_EDGE_LAPLACIAN) {
@@ -1130,7 +1183,7 @@ static EaPrepArgs prep_slice(const EaPrepArgs& A, int f0, int n) {
   EaPrepArgs S = A;
   const size_t px0 = size_t(A.lv[0].w) * A.lv[0].h;
   S.n = n; S.slots = A.slots + f0;
-  S.in_bgr = A.in_bgr + size_t(f0) * px0 * A.in_channels;
+  S.in_img = A.in_img + size_t(f0) * A.in_stride;
   if (A.in_depth) S.in_depth = static_cast<const char*>(A.in_depth) + size_t(f0) * px0 * (A.depth_type == 1 ? 4 : 2);
   if (A.in_mask) S.in_mask = A.in_mask + size_t(f0) * px0;
   if (A.in_now_mask) S.in_now_mask = A.in_now_mask + size_t(f0) * px0;
@@ -1143,7 +1196,10 @@ static EaPrepArgs prep_args(const ea_frameset* fs, int n, const int32_t* d_slots
   EaPrepArgs A;
   std::memset(&A, 0, sizeof A);
   for (int l = 0; l < p.n_levels; ++l) A.lv[l] = fs->lv[l];
-  A.n_levels = p.n_levels; A.slots = d_slots; A.in_bgr = in.image; A.in_channels = in.channels; A.in_depth = in.depth;
+  A.n_levels = p.n_levels; A.slots = d_slots; A.in_img = in.image; A.in_depth = in.depth;
+  // NV12 is its luma plane: the kernels read it as GRAY8 with the frame's pitch and stride
+  A.in_format = in.layout.format == EA_IMAGE_NV12 ? EA_IMAGE_GRAY8 : in.layout.format;
+  A.in_pitch = size_t(in.layout.row_pitch); A.in_stride = size_t(in.layout.frame_stride);
   A.in_mask = in.ref_mask; A.in_now_mask = in.now_mask;
   A.n_pts = fs->d_npts; A.dt_minmax = fs->d_minmax; A.dt_affine = fs->d_affine; A.overflow = fs->d_overflow;
   A.n = n; A.roles = roles; A.grad_threshold = p.grad_threshold; A.use_median = p.use_median;

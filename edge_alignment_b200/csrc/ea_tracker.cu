@@ -47,7 +47,7 @@ struct ea_tracker {
   cudaStream_t prep_stream = nullptr;
   cudaEvent_t ev_prep[2] = {nullptr, nullptr}, ev_solved[2] = {nullptr, nullptr};
   int inputs_ready = 0;            // ea_tracker_set_inputs_ready: device inputs are complete at call time (not stream-ordered)
-  int channels = 3;                // image bytes per pixel: 3 (EA_IMAGE_BGR8) or 1 (EA_IMAGE_GRAY8)
+  ea_image_layout layout{EA_IMAGE_BGR8, 0, 0, 0};   // of the step functions' image argument (resolved by ea_tracker_create)
   double* d_poses = nullptr;       // warm-start table [n_streams][7]
   double* d_result = nullptr;      // poses of the latest step [n_streams][7]
   double* d_identity = nullptr;    // [n_streams][7]
@@ -56,7 +56,7 @@ struct ea_tracker {
   bool have_order = false;
   // host-input pipeline: frame t+1 is uploaded on a copy stream while frame t is being aligned
   cudaStream_t copy_stream = nullptr;
-  uint8_t* stage_bgr[2] = {nullptr, nullptr};   // [n_streams][h][w][channels]
+  uint8_t* stage_bgr[2] = {nullptr, nullptr};   // [n_streams] frames packed dense (ea_upload_frames)
   void* stage_depth[2] = {nullptr, nullptr};
   cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_consumed[2] = {nullptr, nullptr}, ev_result[2] = {nullptr, nullptr};
   double* h_poses[2] = {nullptr, nullptr};          // pinned result ring
@@ -212,6 +212,8 @@ int ea_tracker_create(ea_context* ctx, const ea_frame_params* fp, const ea_solve
   CU(cudaMalloc((void**)&t->d_world, id.size() * 8));
   CU(cudaMalloc((void**)&t->d_world_key, id.size() * 8));
   CU(cudaMalloc((void**)&t->d_info, n_streams * sizeof(ea_track_info)));
+  rc = ea_resolve_layout(&t->layout, fp->width, fp->height, true, &t->layout);
+  if (rc) return rc;
   rc = ea_tracker_reset(t);
   if (rc) return rc;
   guard.t = nullptr;
@@ -280,7 +282,8 @@ int ea_tracker_set_keyframe_policy(ea_tracker* t, const ea_keyframe_policy* p) {
 
 // input_ready: event after which the frame buffers are complete (host path: the upload); null => the buffers are ordered by
 // the context stream (default) or already complete (inputs_ready).
-static int tracker_step(ea_tracker* t, const uint8_t* d_bgr, const void* d_depth, cudaEvent_t input_ready, cudaEvent_t consumed) {
+static int tracker_step(ea_tracker* t, const uint8_t* d_bgr, const ea_image_layout& layout, const void* d_depth, cudaEvent_t input_ready,
+                        cudaEvent_t consumed) {
   ea_context* c = t->ctx;
   CU(cudaSetDevice(c->device));
   cudaStream_t s = c->stream;
@@ -308,7 +311,7 @@ static int tracker_step(ea_tracker* t, const uint8_t* d_bgr, const void* d_depth
   if (t->frame >= 3) CU(cudaStreamWaitEvent(ps, t->ev_solved[fb], 0));   // last reader of this slot set: the solve of frame - 2
   // policy mode: frames after the first build their point lists only once the policy kernel has promoted them
   const bool defer = policy && !first;
-  const EaFrameInput in{d_bgr, t->channels, d_depth, nullptr, nullptr, false};
+  const EaFrameInput in{d_bgr, layout, d_depth, nullptr, nullptr, false};
   int rc = ea_launch_preprocess(t->fs, t->n_streams, d_new_slots, roles, in, ps, defer ? EA_COMPACT_DEFER : EA_COMPACT_INLINE, nullptr);
   if (rc) return rc;
   CU(cudaEventRecord(t->ev_prep[fb], ps));
@@ -360,21 +363,34 @@ extern "C" {
 
 int ea_tracker_step_device(ea_tracker* t, const uint8_t* d_bgr, const void* d_depth) {
   if (!t || !d_bgr) return ea_fail(EA_ERR_INVALID_ARG, "null argument");
-  return tracker_step(t, d_bgr, d_depth, nullptr, nullptr);
+  ea_image_layout L;   // BGR8 with a pitch is only read through the host path's copy
+  const int rc = ea_resolve_layout(&t->layout, t->fs->p.width, t->fs->p.height, true, &L);
+  if (rc) return rc;
+  return tracker_step(t, d_bgr, L, d_depth, nullptr, nullptr);
+}
+
+int ea_tracker_set_image_layout(ea_tracker* t, const ea_image_layout* layout) {
+  if (!t) return ea_fail(EA_ERR_INVALID_ARG, "null tracker");
+  ea_image_layout L;
+  const int w = t->fs->p.width, h = t->fs->p.height;
+  int rc = ea_resolve_layout(layout, w, h, false, &L);
+  if (rc) return rc;
+  if (t->frame != 0) return ea_fail(EA_ERR_STATE, "the image layout can only change before the first step (after create or reset)");
+  // the host-path staging buffers are sized for the bytes per frame of the layout; the next step_host allocates them anew
+  if (ea_layout_row_bytes(L, w) != ea_layout_row_bytes(t->layout, w)) {
+    CU(cudaSetDevice(t->ctx->device));
+    CU(cudaStreamSynchronize(t->copy_stream));
+    for (int b = 0; b < 2; ++b) { CU(cudaFree(t->stage_bgr[b])); t->stage_bgr[b] = nullptr; }
+  }
+  t->layout = L;
+  return EA_OK;
 }
 
 int ea_tracker_set_image_format(ea_tracker* t, int image_format) {
   if (!t) return ea_fail(EA_ERR_INVALID_ARG, "null tracker");
   if (image_format != EA_IMAGE_BGR8 && image_format != EA_IMAGE_GRAY8) return ea_fail(EA_ERR_INVALID_ARG, "unknown image format %d", image_format);
-  if (t->frame != 0) return ea_fail(EA_ERR_STATE, "the image format can only change before the first step (after create or reset)");
-  const int channels = image_format == EA_IMAGE_GRAY8 ? 1 : 3;
-  if (channels != t->channels) {   // the host-path staging buffers are sized for the format; the next step_host allocates them anew
-    CU(cudaSetDevice(t->ctx->device));
-    CU(cudaStreamSynchronize(t->copy_stream));
-    for (int b = 0; b < 2; ++b) { CU(cudaFree(t->stage_bgr[b])); t->stage_bgr[b] = nullptr; }
-    t->channels = channels;
-  }
-  return EA_OK;
+  const ea_image_layout dense{image_format, 0, 0, 0};
+  return ea_tracker_set_image_layout(t, &dense);
 }
 
 int ea_tracker_set_inputs_ready(ea_tracker* t, int ready) {
@@ -417,15 +433,15 @@ int ea_tracker_step_host(ea_tracker* t, const uint8_t* bgr, const void* depth, d
   const bool needs_depth = t->policy_on || (frame % t->interval) == 0;
   if (t->policy_on && !depth) return ea_fail(EA_ERR_INVALID_ARG, "key-frame policy mode: any frame may become a key frame, every step needs depth");
   if (needs_depth && !depth) return ea_fail(EA_ERR_INVALID_ARG, "frame %d becomes a key frame and needs depth", frame);
-  const size_t frame_bytes = px * t->channels * n;
+  const size_t frame_bytes = ea_layout_row_bytes(t->layout, fs->p.width) * fs->p.height * n;
   if (!t->stage_bgr[b]) CU(cudaMalloc((void**)&t->stage_bgr[b], frame_bytes));
   if (needs_depth && !t->stage_depth[b]) CU(cudaMalloc((void**)&t->stage_depth[b], px * fs->depth_elem * n));
   // upload on the copy stream once the kernels that read this staging buffer two frames ago are done
   if (frame >= 2) CU(cudaStreamWaitEvent(t->copy_stream, t->ev_consumed[b], 0));
-  CU(cudaMemcpyAsync(t->stage_bgr[b], bgr, frame_bytes, cudaMemcpyHostToDevice, t->copy_stream));
+  CU(ea_upload_frames(t->stage_bgr[b], bgr, t->layout, fs->p.width, fs->p.height, n, t->copy_stream));
   if (needs_depth) CU(cudaMemcpyAsync(t->stage_depth[b], depth, px * fs->depth_elem * n, cudaMemcpyHostToDevice, t->copy_stream));
   CU(cudaEventRecord(t->ev_copied[b], t->copy_stream));
-  int rc = tracker_step(t, t->stage_bgr[b], needs_depth ? t->stage_depth[b] : nullptr, t->ev_copied[b], t->ev_consumed[b]);
+  int rc = tracker_step(t, t->stage_bgr[b], ea_staged_layout(t->layout, fs->p.width, fs->p.height), needs_depth ? t->stage_depth[b] : nullptr, t->ev_copied[b], t->ev_consumed[b]);
   if (rc) return rc;
   // results into the pinned ring; the caller reads them now (poses7 given) or later with ea_tracker_wait
   CU(cudaMemcpyAsync(t->h_poses[b], t->d_result, size_t(n) * 7 * 8, cudaMemcpyDeviceToHost, c->stream));

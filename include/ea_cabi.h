@@ -12,7 +12,8 @@
  * Conventions
  *   - every function returns ea_status (0 == EA_OK); ea_last_error() gives the text
  *   - images: BGR u8 interleaved row-major (cv::imread order, standalone_edge_align.cpp:118), or 8-bit gray
- *     row-major through the *_gray_* entry points / ea_tracker_set_image_format; depth u16 row-major (raw units;
+ *     row-major through the *_gray_* entry points / ea_tracker_set_image_format, or NV12 / YUYV / UYVY frames with a row
+ *     pitch through the *_image_* entry points / ea_tracker_set_image_layout; depth u16 row-major (raw units;
  *     metres = raw / depth_scale, utils.cpp:235)
  *   - pose: 7 doubles {qw,qx,qy,qz,tx,ty,tz} = b_T_a, Eigen/Ceres (w,x,y,z) order
  *     (standalone/PoseManipUtils.cpp:16-27)
@@ -210,12 +211,45 @@ int ea_frameset_preprocess_device(ea_frameset* fs, int n, const int32_t* slots, 
  * ref_mask [n][h][w] u8 or NULL: reference points only where ref_mask > 0 (get_aX_mask, needs EA_ROLE_REF); now_mask
  * [n][h][w] u8 or NULL: now-frame edges only where now_mask > 1 (get_distance_transform2_masked, needs EA_ROLE_NOW).
  * roles: EA_ROLE_REF, EA_ROLE_NOW or EA_ROLE_BOTH.  Asynchronous on the context stream. */
-typedef enum ea_image_format { EA_IMAGE_BGR8 = 0, EA_IMAGE_GRAY8 = 1 } ea_image_format;
+typedef enum ea_image_format {
+  EA_IMAGE_BGR8 = 0, EA_IMAGE_GRAY8 = 1,
+  EA_IMAGE_NV12 = 2, EA_IMAGE_YUYV = 3, EA_IMAGE_UYVY = 4   /* luma read in place: ea_image_layout below */
+} ea_image_format;
 int ea_frameset_preprocess_gray_host(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* gray, const void* depth,
                                      const uint8_t* ref_mask, const uint8_t* now_mask, int roles);
 /* same, inputs already resident in device memory (d_gray 4-byte aligned for the word-wide kernels; any address works) */
 int ea_frameset_preprocess_gray_device(ea_frameset* fs, int n, const int32_t* slots, const uint8_t* d_gray,
                                        const void* d_depth, int roles);
+
+/* Camera and decoder frames read in place: only their luma is preprocessed, and chroma and padding bytes are never read.
+ *   EA_IMAGE_NV12  the luma plane comes first, one byte per pixel at row_pitch; whatever follows it is ignored.  I420, YV12
+ *                  and NV21 frames are therefore passed as EA_IMAGE_NV12 as they are.
+ *   EA_IMAGE_YUYV  packed 4:2:2, bytes Y0 U Y1 V per pixel pair (UVC webcams, RGB-D colour streams); w must be even
+ *   EA_IMAGE_UYVY  packed 4:2:2, bytes U Y0 V Y1 per pixel pair; w must be even
+ * A frame in one of these formats gives exactly what the *_gray_* entry points give on its dense Y plane (points, truncation
+ * flags, edge and median planes, distance transforms, solves).  Caution: a video Y plane (BT.601 or BT.709, often limited
+ * range 16-235) is not cv::cvtColor(BGR2GRAY) of the decoded BGR frame.  The results are those of the luma as delivered, and
+ * grad_threshold applies to those values: there is no range expansion and no colour conversion. */
+typedef struct ea_image_layout {
+  int32_t format;        /* ea_image_format or EA_IMAGE_NV12 / _YUYV / _UYVY */
+  int32_t reserved;      /* 0 */
+  int64_t row_pitch;     /* bytes from a row to the next (NV12: of the luma plane); 0 = dense: w * {3, 1, 1, 2, 2} */
+  int64_t frame_stride;  /* bytes from a frame to the next; 0 = dense: h * row_pitch, NV12 3 * h * row_pitch / 2 */
+} ea_image_layout;
+/* The image of frame i starts at image + i * frame_stride.  EA_ERR_INVALID_ARG (and nothing launched) for an unknown format,
+ * reserved != 0, row_pitch < w * bytes per pixel, frame_stride < h * row_pitch or not a multiple of row_pitch, NV12 with odd h,
+ * YUYV / UYVY with odd w, and BGR8 with a non-dense layout on the device path.  Depth, ref_mask and now_mask are dense
+ * [n][h][w] as for ea_frameset_preprocess_gray_host.  The host path uploads only the bytes the kernels read (the luma rows of
+ * NV12, the pixel rows of GRAY8 / BGR8, the 2w-byte rows of YUYV / UYVY), packed dense, in one copy per call.  The device path
+ * reads the frames where they lie: word-wide loads need a 4-byte (planar) or 8-byte (packed) aligned image, row_pitch and
+ * frame_stride; any other layout takes the byte kernels with the same results. */
+int ea_frameset_preprocess_image_host(ea_frameset* fs, int n, const int32_t* slots, const ea_image_layout* layout,
+                                      const uint8_t* image, const void* depth, const uint8_t* ref_mask,
+                                      const uint8_t* now_mask, int roles);
+/* same, every buffer (masks too) already resident in device memory */
+int ea_frameset_preprocess_image_device(ea_frameset* fs, int n, const int32_t* slots, const ea_image_layout* layout,
+                                        const uint8_t* d_image, const void* d_depth, const uint8_t* d_ref_mask,
+                                        const uint8_t* d_now_mask, int roles);
 
 /* Bypass hooks (parity on oracle-made inputs; CAD point sets as in edge_align_test5..8). */
 int ea_frameset_set_points(ea_frameset* fs, int slot, int level, const float* pts4, int n, int mode);
@@ -307,6 +341,12 @@ int ea_tracker_step_device(ea_tracker* tr, const uint8_t* d_bgr, const void* d_d
  * are those of BGR frames (g, g, g).  Only before the first step (after ea_tracker_create or ea_tracker_reset), else
  * EA_ERR_STATE. */
 int ea_tracker_set_image_format(ea_tracker* tr, int image_format);
+/* The general form of ea_tracker_set_image_format: ea_tracker_step_host / _device take the image in this layout (any format of
+ * ea_image_layout, with a row pitch and a frame stride), stream s starting at image + s * frame_stride.  Results are those of
+ * GRAY8 frames holding the luma.  The same rules as ea_frameset_preprocess_image_*, and the same state rule as
+ * ea_tracker_set_image_format (EA_ERR_STATE after the first step until ea_tracker_reset).  BGR8 with a pitch is accepted for
+ * ea_tracker_step_host, whose copy packs it dense; ea_tracker_step_device then returns EA_ERR_INVALID_ARG. */
+int ea_tracker_set_image_layout(ea_tracker* tr, const ea_image_layout* layout);
 /* By default the device buffers passed to ea_tracker_step_device are ordered by the context stream (work enqueued there
  * before the call produces them).  ready != 0 declares instead that they are COMPLETE in memory when the call is made; the
  * tracker then preprocesses frame t+1 on its own stream while frame t is still being aligned (its kernels take over the

@@ -54,9 +54,7 @@ class Frame {
     if (rgb.rows != params_.height || rgb.cols != params_.width) throw std::runtime_error("Frame::set: image size differs from ea_frame_params");
     const int type = rgb.type();
     if (type != ea::U8C3 && type != ea::U8C1) throw std::runtime_error("Frame::set: the image must be 8UC3 (BGR) or 8UC1 (gray)");
-    const size_t W = size_t(params_.width), H = size_t(params_.height), C = (type == ea::U8C3) ? 3 : 1;
-    bgr_.resize(W * H * C);
-    for (size_t y = 0; y < H; ++y) std::copy(rgb.data + y * size_t(rgb.step), rgb.data + y * size_t(rgb.step) + W * C, bgr_.begin() + y * W * C);
+    const size_t W = size_t(params_.width), H = size_t(params_.height);
     const void* dptr = nullptr;
     if (depth && depth->data) {
       const bool want_f32 = params_.depth_type == EA_DEPTH_F32, have_f32 = depth->type() == ea::F32C1;
@@ -78,8 +76,10 @@ class Frame {
       dptr = depth_.data();
     }
     const int32_t slot = 0;
-    if (C == 3) ea::check(ea_frameset_preprocess_host(fs_, 1, &slot, bgr_.data(), dptr, roles), "ea_frameset_preprocess_host");
-    else ea::check(ea_frameset_preprocess_gray_host(fs_, 1, &slot, bgr_.data(), dptr, nullptr, nullptr, roles), "ea_frameset_preprocess_gray_host");
+    // the rows are read where they lie: the upload skips the padding between them
+    const ea_image_layout layout{type == ea::U8C3 ? EA_IMAGE_BGR8 : EA_IMAGE_GRAY8, 0, int64_t(size_t(rgb.step)), 0};
+    ea::check(ea_frameset_preprocess_image_host(fs_, 1, &slot, &layout, rgb.data, dptr, nullptr, nullptr, roles),
+              "ea_frameset_preprocess_image_host");
     ea::check(ea_sync(ctx_), "ea_sync");
   }
 
@@ -104,6 +104,5 @@ class Frame {
   ea_context* ctx_ = nullptr;
   ea_frameset* fs_ = nullptr;
   ea_frame_params params_{};
-  std::vector<uint8_t> bgr_;            // the image as uploaded: BGR or gray rows without padding
   std::vector<unsigned char> depth_;
 };
